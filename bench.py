@@ -8,7 +8,12 @@ A "step" is one full particle-filter log-likelihood evaluation (estimate_likelih
 steps.  `value` is measured with theta and the result resident in HBM (dpomp_pf_loglik_device); `e2e` is the same metric
 through the public API closure get_particle_filter_lpdf(model, y)(theta) with HOST buffers.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
+
+--dump-outputs DIR writes what the last timed step of each C2 loop returned, as DIR/<name>.npy: `loglik` (device-resident
+path) with `population` (the filter's particles after that call, n x C, exact in float32), `loglik_e2e` (public API
+closure) and `loglik_f64_loop`.  Seeds, theta and data are fixed, so the same arguments give the same inputs on every run
+and two builds can be compared output for output.
 """
 from __future__ import annotations
 
@@ -353,7 +358,10 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-smc2", action="store_true", help="skip the SMC^2 (config C4) secondary measurement")
     ap.add_argument("--no-outer", action="store_true", help="skip the pMCMC (C3) and MBP-IBIS (C5) secondary measurements")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step of each C2 loop to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         return run_reference(args)
@@ -412,6 +420,10 @@ def main():
         events += pf.last_event_count()
     barrier()
     ll_last = float(out_dev.item())
+    dumps = {}
+    if args.dump_outputs:
+        dumps["loglik"] = np.array([ll_last])
+        dumps["population"] = pf.get_pop(1).astype(np.float32)
 
     # ---- timed region 2: end to end through the public API closure, host theta -> host float -------------------
     f = dp.get_particle_filter_lpdf(model, y, np=N_PARTICLES, seed=2000 + rank, device=local_rank)
@@ -428,12 +440,14 @@ def main():
         wall_e2e += time.perf_counter() - t0
     barrier()
     clocks = sampler.stop()
+    if args.dump_outputs:
+        dumps["loglik_e2e"] = np.array([ll_e2e])
 
     # ---- roofline pass: CUDA events around every kernel launch of the same step --------------------------------
     pf.set_kernel_timing(True)
     k_ms = np.zeros(2)
     k_n = np.zeros(2, dtype=np.int64)
-    roof_steps = min(args.steps, 20)
+    roof_steps = args.steps
     for _ in range(roof_steps):
         flush.zero_()
         torch.cuda.synchronize()
@@ -448,7 +462,7 @@ def main():
     pf64 = dp.ParticleFilter(dm, N_PARTICLES, 1, 1, seed=3000 + rank, device=local_rank, sim_precision=dp._capi.SIM_F64)
     for _ in range(2):
         pf64.loglik_device(theta_dev.data_ptr(), 1, out_dev.data_ptr())
-    f64_steps = max(3, min(args.steps, 10))
+    f64_steps = args.steps
     barrier()
     wall_f64 = 0.0
     for _ in range(f64_steps):
@@ -460,6 +474,12 @@ def main():
     barrier()
     ll_f64 = float(out_dev.item())
     del pf64
+    if args.dump_outputs:
+        dumps["loglik_f64_loop"] = np.array([ll_f64])
+        if rank == 0:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, arr in dumps.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), arr)
 
     smc2 = pmcmc = mbpi = None
     if not args.no_smc2:
