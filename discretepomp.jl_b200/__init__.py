@@ -13,8 +13,9 @@ Exported names are those of the reference's public API that lie on the path (src
 """
 from .structs import (DPOMPModel, Event, HiddenMarkovModel, ImportanceSample, MCMCSample, Observation, Particle,
                       RejectionSample, SimResults)
-from .examples import (GaussianObsModel, UniformProduct, dmy_obs_fn, generate_custom_model, generate_model,
-                       generate_trans_fn, generate_weak_prior, partial_gaussian_obs_model)
+from .examples import (CountObsModel, GaussianObsModel, UniformProduct, dmy_obs_fn, generate_custom_model, generate_model,
+                       generate_trans_fn, generate_weak_prior, partial_binomial_obs_model, partial_gaussian_obs_model,
+                       partial_negbin_obs_model, partial_poisson_obs_model)
 from .rate_table import ModelCompileError, compile_obs_table, compile_rate_table
 from .utils import get_observations
 from .particle_filter import (C_DF_ESS_CRIT, C_DF_PF_P, DeviceModel, ParticleFilter, compile_model, compute_ess,

@@ -19,6 +19,7 @@ MAX_OBS_VALS = 8
 RS_SYSTEMATIC, RS_STRATIFIED, RS_MULTINOMIAL = 1, 2, 3
 SIM_F32, SIM_F64 = 0, 1
 SCATTER_REFERENCE, SCATTER_INTERLEAVED = 0, 1
+OBS_GAUSSIAN, OBS_POISSON, OBS_BINOMIAL, OBS_NEGBIN = 0, 1, 2, 3
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 # DPOMP_LIB_PATH selects another build of the same library (kernel A/B measurements); there is still no fallback
@@ -69,6 +70,7 @@ _SIGS = {
     "dpomp_device_count": (C.c_int, [C.POINTER(C.c_int)]),
     "dpomp_model_create": (C.c_int, [C.POINTER(ModelDesc), C.POINTER(_P)]),
     "dpomp_model_destroy": (C.c_int, [_P]),
+    "dpomp_model_set_obs_model": (C.c_int, [_P, C.c_int32, _P, _P]),
     "dpomp_pf_create": (C.c_int, [_P, C.c_int64, C.c_int32, C.c_int32, C.c_uint64, C.c_int32, C.POINTER(_P)]),
     "dpomp_pf_destroy": (C.c_int, [_P]),
     "dpomp_pf_set_sim_precision": (C.c_int, [_P, C.c_int32]),

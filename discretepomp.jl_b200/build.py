@@ -13,7 +13,8 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIBDIR = os.path.join(HERE, "lib")
 OBJDIR = os.path.join(LIBDIR, "obj")
-SOURCES = ["capi.cu", "pf_kernels.cu", "pf_sim_f32.cu", "pf_sim_f64.cu", "mbp.cu", "comm.cu"]
+SOURCES = ["capi.cu", "pf_kernels.cu", "pf_sim_f32.cu", "pf_sim_f64.cu", "pf_sim_count_f32.cu", "pf_sim_count_f64.cu", "mbp.cu",
+           "comm.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
     "-Xcompiler", "-fPIC", "-Xptxas", "-v", "--expt-relaxed-constexpr", "-ftz=true",

@@ -40,7 +40,7 @@ static uint64_t call_key(const dpomp_pf* pf) {
 extern "C" {
 
 const char* dpomp_last_error(void) { return g_err.c_str(); }
-int dpomp_version(void) { return 100; }
+int dpomp_version(void) { return 101; }
 
 int dpomp_device_count(int* out_count) {
     if (!out_count) return fail(DPOMP_ERR_ARG, "out_count is null");
@@ -89,6 +89,56 @@ int dpomp_model_create(const dpomp_model_desc* d, dpomp_model** out_model) {
     return DPOMP_OK;
 }
 
+// lgamma(Y+1) and, for a fixed negative-binomial size k, lgamma(Y+k) - lgamma(k) of every observation (glibc, as the oracle)
+static void count_obs_constants(ModelHost& h) {
+    h.obs_lgy.assign(h.obs_ysum.size(), 0.0);
+    h.obs_lgk.assign(h.obs_ysum.size(), 0.0);
+    const bool fixed_k = h.obs_family == DPOMP_OBS_NEGBIN && h.obs_par_index[1] < 0;
+    for (size_t t = 0; t < h.obs_ysum.size(); ++t) {
+        const double y = h.obs_ysum[t];
+        if (!(y >= 0.0)) continue;  // Y < 0: log g = -Inf, the constants are not read
+        h.obs_lgy[t] = lgamma(y + 1.0);
+        if (fixed_k) h.obs_lgk[t] = lgamma(y + h.obs_par_value[1]) - lgamma(h.obs_par_value[1]);
+    }
+}
+
+int dpomp_model_set_obs_model(dpomp_model* model, int32_t family, const int32_t* par_index, const double* par_value) {
+    if (!model || !par_index || !par_value) return fail(DPOMP_ERR_ARG, "null argument");
+    if (family < DPOMP_OBS_GAUSSIAN || family > DPOMP_OBS_NEGBIN) return fail(DPOMP_ERR_ARG, "unknown observation family");
+    if (model->frozen.load()) return fail(DPOMP_ERR_STATE, "the model already has a filter or MBP handle; it is frozen");
+    ModelHost& h = model->h;
+    const dpomp_model_desc& d = h.desc;
+    if (family != DPOMP_OBS_GAUSSIAN) {
+        const int n_par = family == DPOMP_OBS_NEGBIN ? 2 : 1;
+        for (int i = 0; i < n_par; ++i) {
+            if (par_index[i] >= d.n_params || par_index[i] < -1)
+                return fail(DPOMP_ERR_MODEL, "observation parameter index out of range");
+            if (par_index[i] >= 0) continue;
+            const double v = par_value[i];
+            const bool ok = family == DPOMP_OBS_BINOMIAL ? (v >= 0.0 && v <= 1.0) : (v > 0.0 && v < INFINITY);
+            if (!ok) return fail(DPOMP_ERR_MODEL, family == DPOMP_OBS_BINOMIAL ? "binomial p outside [0, 1]"
+                                                                               : "rate / size must be positive and finite");
+        }
+        for (int c = 0; c < d.n_compartments; ++c)
+            if (d.obs_xmask[c] != 0 && d.obs_xmask[c] != 1) return fail(DPOMP_ERR_MODEL, "count families need a 0/1 obs_xmask");
+        for (int v = 0; v < d.n_obs_vals; ++v)
+            if (d.obs_ymask[v] != 0 && d.obs_ymask[v] != 1) return fail(DPOMP_ERR_MODEL, "count families need a 0/1 obs_ymask");
+    }
+    h.obs_family = family;
+    for (int i = 0; i < 2; ++i) {
+        const bool used = family != DPOMP_OBS_GAUSSIAN && (i == 0 || family == DPOMP_OBS_NEGBIN);
+        h.obs_par_index[i] = used ? par_index[i] : -1;
+        h.obs_par_value[i] = used && par_index[i] < 0 ? par_value[i] : 0.0;
+    }
+    if (family == DPOMP_OBS_GAUSSIAN) {
+        h.obs_lgy.clear();
+        h.obs_lgk.clear();
+    } else {
+        count_obs_constants(h);
+    }
+    return DPOMP_OK;
+}
+
 int dpomp_model_destroy(dpomp_model* model) {
     delete model;
     return DPOMP_OK;
@@ -103,6 +153,7 @@ static void pf_free(dpomp_pf* pf) {
     cudaFree(pf->filt_m); cudaFree(pf->filt_s); cudaFree(pf->ll_acc); cudaFree(pf->tile_counter); cudaFree(pf->counters);
     cudaFree(pf->obs_time_dev); cudaFree(pf->obs_ysum_dev); cudaFree(pf->slots_dev); cudaFree(pf->filter_ids_dev); cudaFree(pf->work_counter); cudaFree(pf->filt_gen);
     cudaFree(pf->rows_done); cudaFree(pf->gen_flags); cudaFree(pf->obs_haslik_dev);
+    cudaFree(pf->obs_lgy_dev); cudaFree(pf->obs_lgk_dev);
     cudaFreeHost(pf->h_theta); cudaFreeHost(pf->h_ll); cudaFreeHost(pf->h_slots); cudaFreeHost(pf->h_cnt);
     for (cudaEvent_t e : pf->kev) cudaEventDestroy(e);
     if (pf->ev0) cudaEventDestroy(pf->ev0);
@@ -185,6 +236,11 @@ int dpomp_pf_create(const dpomp_model* model, int64_t n_particles, int32_t n_bat
     ALLOC(pf->filter_ids_dev, B * sizeof(uint32_t));
     ALLOC(pf->work_counter, sizeof(unsigned long long));
     ALLOC(pf->filt_gen, B * sizeof(unsigned int));
+    const bool count_obs = model->h.obs_family != DPOMP_OBS_GAUSSIAN;
+    if (count_obs) {
+        ALLOC(pf->obs_lgy_dev, (size_t)d.n_obs * sizeof(double));
+        ALLOC(pf->obs_lgk_dev, (size_t)d.n_obs * sizeof(double));
+    }
 #undef ALLOC
     bool ok = cudaMallocHost((void**)&pf->h_theta, B * pf->n_params * sizeof(double)) == cudaSuccess &&
               cudaMallocHost((void**)&pf->h_ll, B * sizeof(double)) == cudaSuccess &&
@@ -203,12 +259,18 @@ int dpomp_pf_create(const dpomp_model* model, int64_t n_particles, int32_t n_bat
                               cudaMemcpyHostToDevice, pf->stream) == cudaSuccess &&
               cudaMemcpyAsync(pf->obs_ysum_dev, model->h.obs_ysum.data(), (size_t)d.n_obs * sizeof(double),
                               cudaMemcpyHostToDevice, pf->stream) == cudaSuccess &&
+              (!count_obs ||
+               (cudaMemcpyAsync(pf->obs_lgy_dev, model->h.obs_lgy.data(), (size_t)d.n_obs * sizeof(double),
+                                cudaMemcpyHostToDevice, pf->stream) == cudaSuccess &&
+                cudaMemcpyAsync(pf->obs_lgk_dev, model->h.obs_lgk.data(), (size_t)d.n_obs * sizeof(double),
+                                cudaMemcpyHostToDevice, pf->stream) == cudaSuccess)) &&
               cudaStreamSynchronize(pf->stream) == cudaSuccess;
     if (!ok) {
         std::string msg = std::string("pf setup: ") + cudaGetErrorString(cudaGetLastError());
         pf_free(pf);
         return fail(DPOMP_ERR_CUDA, msg);
     }
+    model->frozen.store(true);
     *out_pf = pf;
     return DPOMP_OK;
 }
@@ -421,6 +483,7 @@ int dpomp_run_partial_enqueue(dpomp_pf* pf, const double* theta, bool theta_on_d
         a.t = t; a.fresh = (oi == 1); a.has_lik = has_lik;
         a.key = key; a.filter0 = (uint32_t)pf->batch_offset; a.max_events = pf->max_events;
         a.filter_ids = pf->use_filter_ids ? pf->filter_ids_dev : nullptr;
+        a.cobs = count_obs_of(mh, pf->obs_lgy_dev, pf->obs_lgk_dev);
         // one fused launch (simulate + resample) when every tile of a filter can be resident at once
         const bool fused = do_rs && fused_ok;
         bool fused_tickets = false;

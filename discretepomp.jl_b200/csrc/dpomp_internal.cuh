@@ -3,11 +3,13 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <atomic>
 #include <string>
 #include <vector>
 
 #include "../../include/dpomp.h"
 #include "dpomp_dev.cuh"
+#include "obs_count.cuh"
 
 namespace dpomp {
 
@@ -88,6 +90,7 @@ struct SimLaunch {
     uint32_t filter0;        // global id of local filter 0
     const uint32_t* filter_ids;  // optional explicit global ids [n_filters] (overrides filter0 + b)
     long long max_events;
+    CountObs cobs;           // count observation family (read only by the kModelCountObs instantiations, pf_sim_count_*.cu)
 };
 
 struct ResampleLaunch {
@@ -128,6 +131,12 @@ struct ModelHost {
     std::vector<int32_t> obs_id;
     std::vector<int64_t> obs_val;
     std::vector<double> obs_ysum;
+    // observation family (dpomp_model_set_obs_model); obs_lgy / obs_lgk are the host constants lgamma(Y+1) and, for a fixed k,
+    // lgamma(Y+k) - lgamma(k), empty for the Gaussian
+    int obs_family = DPOMP_OBS_GAUSSIAN;
+    int obs_par_index[2] = {-1, -1};
+    double obs_par_value[2] = {0.0, 0.0};
+    std::vector<double> obs_lgy, obs_lgk;
 };
 
 }  // namespace dpomp
@@ -135,6 +144,7 @@ struct ModelHost {
 // ---- the opaque handles of include/dpomp.h (host-side state; shared by capi.cu and comm.cu) -------------------------
 struct dpomp_model {
     dpomp::ModelHost h;
+    mutable std::atomic<bool> frozen{false};  // set when a filter or MBP handle is created from the model
 };
 
 struct dpomp_pf {
@@ -166,6 +176,7 @@ struct dpomp_pf {
     unsigned int* tile_counter = nullptr;
     unsigned long long* counters = nullptr;  // [0] events of the last call, [1] sticky overflow count
     double *obs_time_dev = nullptr, *obs_ysum_dev = nullptr;
+    double *obs_lgy_dev = nullptr, *obs_lgk_dev = nullptr;  // count observation constants [T] (count families only)
     int64_t* slots_dev = nullptr;            // 2 * n_batch
     unsigned long long* work_counter = nullptr;  // fused step kernel: arrival-order CTA tickets (monotone)
     unsigned long long work_base = 0;
@@ -249,5 +260,7 @@ cudaError_t launch_pack_filters(int32_t* dst_packed, const int32_t* pop, const i
 cudaError_t launch_search_hook(int rs_type, const double* cw_dev, long long n, const double* u_dev, long long n_out,
                                int64_t* out_dev, cudaStream_t stream);
 int sim_kernel_supported(int n_comp, int n_events);
+// count observation law of a model with its device arrays (obs_lgy / obs_lgk uploaded by the caller)
+CountObs count_obs_of(const ModelHost& m, const double* lgy_dev, const double* lgk_dev);
 
 }  // namespace dpomp

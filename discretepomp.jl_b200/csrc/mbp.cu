@@ -24,6 +24,7 @@
 #include "dpomp_dev.cuh"
 #include "dpomp_internal.cuh"
 #include "dpomp_models.cuh"
+#include "obs_count.cuh"
 
 namespace dpomp {
 
@@ -150,6 +151,18 @@ __device__ __forceinline__ double mbp_obs_ll(const MbpModel& m, double ysum, con
     const double d = ysum - (double)xs;
     return m.obs_tmp1 - __ddiv_rn(__dmul_rn(d, d), m.obs_tmp2);
 }
+// COUNT: the model's count observation family (obs_count.cuh) with its theta-indexed parameters taken from th (the walk's theta)
+template <class R, bool COUNT>
+__device__ __forceinline__ double mbp_obs_ll(const MbpModel& m, const CountObs& co, const double* th, int t, double ysum,
+                                             const int (&x)[R::CMAX]) {
+    if constexpr (!COUNT) {
+        return mbp_obs_ll<R>(m, ysum, x);
+    } else {
+        long long xs = 0;
+        for (int c = 0; c < m.n_comp; ++c) xs += (long long)m.xmask[c] * x[c];
+        return count_obs_logpmf(count_obs_const(co, th, t, ysum), ysum, (double)xs);
+    }
+}
 
 // ---- event-list access policies -------------------------------------------------------------------------------------
 // The walks below are written once against an IO policy, so the thread-per-trajectory and the warp-per-trajectory kernels
@@ -238,10 +251,11 @@ struct WarpShared {  // per warp
 };
 
 // iterate_particle! (src/hmm_sim.jl:6-25) of particle p; `writer`: this thread stores the particle's scalars
-template <class IO, class R>
+template <class IO, class R, bool COUNT = false>
 __device__ __forceinline__ void mbp_iterate_body(const MbpModel& m, MbpStore& st, IO& io, int p, bool writer, const double* theta,
                                                  const double* obs_time, const double* obs_ysum, int cap, int t, int fresh, int has_lik,
-                                                 uint64_t key, uint32_t id0, double* out_logg, const MbpGrow& g) {
+                                                 uint64_t key, uint32_t id0, double* out_logg, const MbpGrow& g,
+                                                 const CountObs& co = CountObs{}) {
     const int nc = mbp_nc<R>(m), ne = mbp_ne<R>(m);
     const double* thp = theta + (size_t)p * m.n_params;
     double th[R::PMAX];
@@ -270,7 +284,7 @@ __device__ __forceinline__ void mbp_iterate_body(const MbpModel& m, MbpStore& st
         ++len;
     }
     io.finish(len);
-    const double out = overflow ? -INFINITY : mbp_obs_ll<R>(m, obs_ysum[t], x);
+    const double out = overflow ? -INFINITY : mbp_obs_ll<R, COUNT>(m, co, th, t, obs_ysum[t], x);
     if (!writer) return;
     if (overflow && cap < g.cap_max) {  // the stride, not MAX_TRAJ: nothing is committed, the host grows the store and re-launches
         *g.need_grow = 1;
@@ -312,11 +326,11 @@ __global__ void __launch_bounds__(32 * kMbpWarpsPerCta) mbp_iterate_warp_kernel(
 }
 
 // partial_model_based_proposal (src/hmm_mbp.jl:83-108): xi = current store (through io), xf = proposal store
-template <class IO, class R>
+template <class IO, class R, bool COUNT = false>
 __device__ __forceinline__ void mbp_propose_body(const MbpModel& m, MbpStore& xf, IO& io, int p, bool writer, bool is_valid,
                                                  const double* theta_i, const double* theta_f, const double* obs_time,
                                                  const double* obs_ysum, const int* obs_haslik, int cap, int ymax, uint64_t key,
-                                                 uint32_t id0, double* out_ll, const MbpGrow& g) {
+                                                 uint32_t id0, double* out_ll, const MbpGrow& g, const CountObs& co = CountObs{}) {
     const int nc = mbp_nc<R>(m), ne = mbp_ne<R>(m);
     double ll0 = 0.0, ll1 = 0.0;
     int flen = 0;
@@ -407,7 +421,7 @@ __device__ __forceinline__ void mbp_propose_body(const MbpModel& m, MbpStore& xf
             }
             if (overflow) break;
             time = t_obs;
-            ll1 = mbp_obs_ll<R>(m, obs_ysum[oi], xfc);
+            ll1 = mbp_obs_ll<R, COUNT>(m, co, thf, oi, obs_ysum[oi], xfc);
             if (obs_haslik[oi]) ll0 += ll1;
         }
         if (overflow) ll0 = -INFINITY;
@@ -458,6 +472,59 @@ __global__ void __launch_bounds__(32 * kMbpWarpsPerCta) mbp_propose_warp_kernel(
     if (is_valid) io.load(0);
     mbp_propose_body<WarpIO, MbpRates<MODEL>>(m, xf, io, p, (threadIdx.x & 31) == 0, is_valid, theta_i, theta_f, obs_time, obs_ysum,
                                               obs_haslik, cap, ymax, key, id0, out_ll, g);
+}
+
+// count observation families (generic rate table only): the same walks with the count log pmf
+__global__ void __launch_bounds__(128) mbp_iterate_count_kernel(const __grid_constant__ MbpModel m, MbpStore st, const double* theta,
+                                                                 const double* obs_time, const double* obs_ysum, int n, int cap, int t,
+                                                                 int fresh, int has_lik, uint64_t key, uint32_t id0, double* out_logg,
+                                                                 MbpGrow g, const __grid_constant__ CountObs co) {
+    const int p = blockIdx.x * blockDim.x + threadIdx.x;
+    if (p >= n || g.done[p] == g.call_id) return;
+    ThreadIO io{nullptr, nullptr, 0, st.ev_time + (size_t)p * cap, st.ev_type + (size_t)p * cap};
+    mbp_iterate_body<ThreadIO, MbpRates<kModelGeneric>, true>(m, st, io, p, true, theta, obs_time, obs_ysum, cap, t, fresh, has_lik, key,
+                                                              id0, out_logg, g, co);
+}
+__global__ void __launch_bounds__(32 * kMbpWarpsPerCta) mbp_iterate_warp_count_kernel(const __grid_constant__ MbpModel m, MbpStore st,
+                                                           const double* theta, const double* obs_time, const double* obs_ysum, int n,
+                                                           int cap, int t, int fresh, int has_lik, uint64_t key, uint32_t id0,
+                                                           double* out_logg, MbpGrow g, const __grid_constant__ CountObs co) {
+    __shared__ WarpShared sh[kMbpWarpsPerCta];
+    const int warp = threadIdx.x >> 5, p = blockIdx.x * kMbpWarpsPerCta + warp;
+    if (p >= n || g.done[p] == g.call_id) return;
+    WarpShared& w = sh[warp];
+    const int len0 = st.len[p];
+    WarpIO io{nullptr, nullptr, 0, st.ev_time + (size_t)p * cap, st.ev_type + (size_t)p * cap, w.it, w.iy, w.ft, w.fy, 0, len0, cap};
+    mbp_iterate_body<WarpIO, MbpRates<kModelGeneric>, true>(m, st, io, p, (threadIdx.x & 31) == 0, theta, obs_time, obs_ysum, cap, t,
+                                                            fresh, has_lik, key, id0, out_logg, g, co);
+}
+__global__ void __launch_bounds__(128) mbp_propose_count_kernel(const __grid_constant__ MbpModel m, MbpStore xi, MbpStore xf,
+                                                                 const double* theta_i, const double* theta_f, const unsigned char* valid,
+                                                                 const double* obs_time, const double* obs_ysum, const int* obs_haslik,
+                                                                 int n, int cap, int ymax, uint64_t key, uint32_t id0, double* out_ll,
+                                                                 MbpGrow g, const __grid_constant__ CountObs co) {
+    const int p = blockIdx.x * blockDim.x + threadIdx.x;
+    if (p >= n || g.done[p] == g.call_id) return;
+    ThreadIO io{xi.ev_time + (size_t)p * cap, xi.ev_type + (size_t)p * cap, xi.len[p], xf.ev_time + (size_t)p * cap,
+                xf.ev_type + (size_t)p * cap};
+    mbp_propose_body<ThreadIO, MbpRates<kModelGeneric>, true>(m, xf, io, p, true, valid[p] != 0, theta_i, theta_f, obs_time, obs_ysum,
+                                                              obs_haslik, cap, ymax, key, id0, out_ll, g, co);
+}
+__global__ void __launch_bounds__(32 * kMbpWarpsPerCta) mbp_propose_warp_count_kernel(const __grid_constant__ MbpModel m, MbpStore xi,
+                                                           MbpStore xf, const double* theta_i, const double* theta_f,
+                                                           const unsigned char* valid, const double* obs_time, const double* obs_ysum,
+                                                           const int* obs_haslik, int n, int cap, int ymax, uint64_t key, uint32_t id0,
+                                                           double* out_ll, MbpGrow g, const __grid_constant__ CountObs co) {
+    __shared__ WarpShared sh[kMbpWarpsPerCta];
+    const int warp = threadIdx.x >> 5, p = blockIdx.x * kMbpWarpsPerCta + warp;
+    if (p >= n || g.done[p] == g.call_id) return;
+    WarpShared& w = sh[warp];
+    WarpIO io{xi.ev_time + (size_t)p * cap, xi.ev_type + (size_t)p * cap, xi.len[p], xf.ev_time + (size_t)p * cap,
+              xf.ev_type + (size_t)p * cap, w.it, w.iy, w.ft, w.fy, 0, 0, cap};
+    const bool is_valid = valid[p] != 0;
+    if (is_valid) io.load(0);
+    mbp_propose_body<WarpIO, MbpRates<kModelGeneric>, true>(m, xf, io, p, (threadIdx.x & 31) == 0, is_valid, theta_i, theta_f, obs_time,
+                                                            obs_ysum, obs_haslik, cap, ymax, key, id0, out_ll, g, co);
 }
 
 // dst[dst_slot[k]] <- src[src_slot[k]] : one CTA per particle, only the live part of the trajectory moves
@@ -778,6 +845,8 @@ struct dpomp_mbp {
     long long batch_offset = 0;
     double *theta_i = nullptr, *theta_f = nullptr, *out = nullptr, *obs_time = nullptr, *obs_ysum = nullptr;
     int* obs_haslik = nullptr;
+    double *obs_lgy = nullptr, *obs_lgk = nullptr;  // count observation constants [T] (count families only)
+    CountObs cobs{};                                // family != DPOMP_OBS_GAUSSIAN: the count kernels run
     unsigned char* valid = nullptr;
     int64_t* slots = nullptr;  // 2 * n
 };
@@ -817,7 +886,7 @@ static void mbp_free(dpomp_mbp* h) {
         cudaFree(h->store[s].fc); cudaFree(h->store[s].ll);
     }
     cudaFree(h->theta_i); cudaFree(h->theta_f); cudaFree(h->out); cudaFree(h->obs_time); cudaFree(h->obs_ysum);
-    cudaFree(h->obs_haslik); cudaFree(h->valid); cudaFree(h->slots); cudaFree(h->done); cudaFree(h->need_grow);
+    cudaFree(h->obs_haslik); cudaFree(h->obs_lgy); cudaFree(h->obs_lgk); cudaFree(h->valid); cudaFree(h->slots); cudaFree(h->done); cudaFree(h->need_grow);
     cudaFreeHost(h->h_need_grow);
     if (h->stream) cudaStreamDestroy(h->stream);
     delete h;
@@ -906,6 +975,14 @@ int dpomp_mbp_create(const dpomp_model* model, int32_t n_particles, int32_t max_
          cudaMemcpy(h->obs_time, model->h.obs_time.data(), d.n_obs * sizeof(double), cudaMemcpyHostToDevice) == cudaSuccess &&
          cudaMemcpy(h->obs_ysum, model->h.obs_ysum.data(), d.n_obs * sizeof(double), cudaMemcpyHostToDevice) == cudaSuccess &&
          cudaMemcpy(h->obs_haslik, haslik.data(), d.n_obs * sizeof(int), cudaMemcpyHostToDevice) == cudaSuccess;
+    if (ok && model->h.obs_family != DPOMP_OBS_GAUSSIAN) {
+        ok = cudaMalloc((void**)&h->obs_lgy, d.n_obs * sizeof(double)) == cudaSuccess &&
+             cudaMalloc((void**)&h->obs_lgk, d.n_obs * sizeof(double)) == cudaSuccess &&
+             cudaMemcpy(h->obs_lgy, model->h.obs_lgy.data(), d.n_obs * sizeof(double), cudaMemcpyHostToDevice) == cudaSuccess &&
+             cudaMemcpy(h->obs_lgk, model->h.obs_lgk.data(), d.n_obs * sizeof(double), cudaMemcpyHostToDevice) == cudaSuccess;
+        h->cobs = count_obs_of(model->h, h->obs_lgy, h->obs_lgk);
+        h->model_id = kModelGeneric;  // the predefined-model walks evaluate the Gaussian only
+    }
     if (!ok) {
         std::string msg = std::string("dpomp_mbp_create: ") + cudaGetErrorString(cudaGetLastError());
         mbp_free(h);
@@ -914,6 +991,7 @@ int dpomp_mbp_create(const dpomp_model* model, int32_t n_particles, int32_t max_
     mbp_reset_kernel<<<(n_particles + 127) / 128, 128, 0, h->stream>>>(h->dm, h->store[0], n_particles);
     MCK(cudaGetLastError());
     MCK(cudaStreamSynchronize(h->stream));
+    model->frozen.store(true);
     *out = h;
     return DPOMP_OK;
 }
@@ -963,7 +1041,18 @@ static int mbp_launch_iterate(dpomp_mbp* h, const double* theta_dev, int n, int 
     }
     for (;;) {
         MCK(cudaMemsetAsync(h->need_grow, 0, sizeof(int), h->stream));
-        DPOMP_MBP_MODELS(DPOMP_MBP_ITERATE)
+        if (h->cobs.family != DPOMP_OBS_GAUSSIAN) {
+            if (warps)
+                mbp_iterate_warp_count_kernel<<<(n + kMbpWarpsPerCta - 1) / kMbpWarpsPerCta, 32 * kMbpWarpsPerCta, 0, h->stream>>>(
+                    h->dm, h->store[h->cur], theta_dev, h->obs_time, h->obs_ysum, n, h->cap, obs_i - 1, fresh ? 1 : 0, has_lik, key,
+                    (uint32_t)h->batch_offset, h->out, g, h->cobs);
+            else
+                mbp_iterate_count_kernel<<<(n + 127) / 128, 128, 0, h->stream>>>(h->dm, h->store[h->cur], theta_dev, h->obs_time,
+                                                                                 h->obs_ysum, n, h->cap, obs_i - 1, fresh ? 1 : 0, has_lik,
+                                                                                 key, (uint32_t)h->batch_offset, h->out, g, h->cobs);
+        } else {
+            DPOMP_MBP_MODELS(DPOMP_MBP_ITERATE)
+        }
         MCK(cudaGetLastError());
         MCK(cudaMemcpyAsync(h->h_need_grow, h->need_grow, sizeof(int), cudaMemcpyDeviceToHost, h->stream));
         MCK(cudaStreamSynchronize(h->stream));
@@ -994,7 +1083,19 @@ static int mbp_launch_propose(dpomp_mbp* h, const double* theta_i_dev, const dou
     }
     for (;;) {
         MCK(cudaMemsetAsync(h->need_grow, 0, sizeof(int), h->stream));
-        DPOMP_MBP_MODELS(DPOMP_MBP_PROPOSE)
+        if (h->cobs.family != DPOMP_OBS_GAUSSIAN) {
+            if (warps)
+                mbp_propose_warp_count_kernel<<<(n + kMbpWarpsPerCta - 1) / kMbpWarpsPerCta, 32 * kMbpWarpsPerCta, 0, h->stream>>>(
+                    h->dm, h->store[h->cur], h->store[2], theta_i_dev, theta_f_dev, valid_dev, h->obs_time, h->obs_ysum, h->obs_haslik,
+                    n, h->cap, ymax, key, (uint32_t)h->batch_offset, h->out, g, h->cobs);
+            else
+                mbp_propose_count_kernel<<<(n + 127) / 128, 128, 0, h->stream>>>(h->dm, h->store[h->cur], h->store[2], theta_i_dev,
+                                                                                 theta_f_dev, valid_dev, h->obs_time, h->obs_ysum,
+                                                                                 h->obs_haslik, n, h->cap, ymax, key,
+                                                                                 (uint32_t)h->batch_offset, h->out, g, h->cobs);
+        } else {
+            DPOMP_MBP_MODELS(DPOMP_MBP_PROPOSE)
+        }
         MCK(cudaGetLastError());
         MCK(cudaMemcpyAsync(h->h_need_grow, h->need_grow, sizeof(int), cudaMemcpyDeviceToHost, h->stream));
         MCK(cudaStreamSynchronize(h->stream));

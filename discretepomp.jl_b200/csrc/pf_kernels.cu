@@ -13,19 +13,40 @@ namespace dpomp {
 
 int sim_f32(const ModelHost& m, int items, const SimLaunch& a, cudaStream_t stream, int mode);
 int sim_f64(const ModelHost& m, int items, const SimLaunch& a, cudaStream_t stream, int mode);
+// count observation families: generic-table kernels only (pf_sim_count_f32.cu / pf_sim_count_f64.cu)
+int sim_count_f32(const ModelHost& m, int items, const SimLaunch& a, cudaStream_t stream, int mode);
+int sim_count_f64(const ModelHost& m, int items, const SimLaunch& a, cudaStream_t stream, int mode);
+
+static int sim_dispatch(const ModelHost& m, int sim_precision, int items, const SimLaunch& a, cudaStream_t stream, int mode) {
+    if (m.obs_family != DPOMP_OBS_GAUSSIAN)
+        return sim_precision == DPOMP_SIM_F64 ? sim_count_f64(m, items, a, stream, mode) : sim_count_f32(m, items, a, stream, mode);
+    return sim_precision == DPOMP_SIM_F64 ? sim_f64(m, items, a, stream, mode) : sim_f32(m, items, a, stream, mode);
+}
 
 cudaError_t launch_sim_weight(const ModelHost& m, int sim_precision, int items, int fused, const SimLaunch& a, cudaStream_t stream) {
     const int mode = fused;  // 0 plain, 1 fused step, 3 persistent
-    return (cudaError_t)(sim_precision == DPOMP_SIM_F64 ? sim_f64(m, items, a, stream, mode) : sim_f32(m, items, a, stream, mode));
+    return (cudaError_t)sim_dispatch(m, sim_precision, items, a, stream, mode);
 }
 int sim_fused_capacity(const ModelHost& m, int sim_precision, int items) {
     SimLaunch dummy{};
-    return sim_precision == DPOMP_SIM_F64 ? sim_f64(m, items, dummy, nullptr, 2) : sim_f32(m, items, dummy, nullptr, 2);
+    return sim_dispatch(m, sim_precision, items, dummy, nullptr, 2);
 }
 
 int sim_persist_capacity(const ModelHost& m, int sim_precision, int items) {
     SimLaunch dummy{};
-    return sim_precision == DPOMP_SIM_F64 ? 0 : sim_f32(m, items, dummy, nullptr, 4);
+    return sim_precision == DPOMP_SIM_F64 ? 0 : sim_dispatch(m, sim_precision, items, dummy, nullptr, 4);
+}
+
+CountObs count_obs_of(const ModelHost& m, const double* lgy_dev, const double* lgk_dev) {
+    CountObs c{};
+    c.family = m.obs_family;
+    for (int i = 0; i < 2; ++i) {
+        c.par_index[i] = m.obs_par_index[i];
+        c.par_value[i] = m.obs_par_value[i];
+    }
+    c.lgy = lgy_dev;
+    c.lgk = lgk_dev;
+    return c;
 }
 
 // does the rate table equal one of the hand-specialised predefined models (pf_sim.cuh Builtin<>)?

@@ -19,6 +19,7 @@
 #include "dpomp_dev.cuh"
 #include "dpomp_internal.cuh"
 #include "dpomp_models.cuh"
+#include "obs_count.cuh"
 #include "pf_resample.cuh"
 
 namespace dpomp {
@@ -132,9 +133,13 @@ __device__ __forceinline__ unsigned int ld_acquire_u32(const unsigned int* p) {
     asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
     return v;
 }
+// MODEL = kModelCountObs: the generic rate table with a count observation family (obs_count.cuh, a.cobs) in the weight pass
+constexpr int kModelCountObs = -1;
 template <typename Real, int C, int E, int ITEMS, int MODEL = kModelGeneric, int MODE = kModePlain, int ILP = DPOMP_SIM_ILP>
 __global__ void __launch_bounds__(kBlockThreads, sim_min_blocks<Real, C, E>())
 pf_sim_weight_kernel(const __grid_constant__ DevModel<Real, C, E> m, const __grid_constant__ SimLaunch a) {
+    constexpr bool COUNT = MODEL == kModelCountObs;
+    constexpr int RMODEL = COUNT ? kModelGeneric : MODEL;  // rate table of the event loop
     constexpr int TILE = kBlockThreads * ITEMS;
     constexpr int CHUNK = 32 * ITEMS;  // particles owned by one warp
     constexpr bool kF32 = sizeof(Real) == 4;
@@ -223,7 +228,7 @@ pf_sim_weight_kernel(const __grid_constant__ DevModel<Real, C, E> m, const __gri
         *reinterpret_cast<Vec*>(ovf_s + tid * ITEMS) = z;
     }
     // compartments present: a compile-time constant for the predefined models
-    const int n_comp = (MODEL != kModelGeneric) ? C : a.n_comp;
+    const int n_comp = (RMODEL != kModelGeneric) ? C : a.n_comp;
     if (PERSIST && staged) {
         // no resampling at the previous observation: the tile's states are still in shared memory
     } else if (!fresh) {
@@ -313,7 +318,7 @@ pf_sim_weight_kernel(const __grid_constant__ DevModel<Real, C, E> m, const __gri
                 // One attempt for every lane, branch free: an absorbed state (`cum_rates[end] == 0.0 && break`, :22) makes
                 // the waiting time -inf / NaN, so `tmn >= 0` is false; the event cap is folded into the same predicate.
                 Real cum[E];
-                cum_rates<Real, C, E, MODEL>(m, par, x[s], cum);
+                cum_rates<Real, C, E, RMODEL>(m, par, x[s], cum);
                 const Real rtot = cum[E - 1];
                 uint2 w;
                 if constexpr (PIPE) {
@@ -327,7 +332,7 @@ pf_sim_weight_kernel(const __grid_constant__ DevModel<Real, C, E> m, const __gri
                 const bool capped = k[s] >= max_ev;  // event cap: documented divergence, the reference loop is unbounded
                 const bool go = (rtot > (Real)0) && !capped && (tmn >= (Real)0);  // `time > tmax && break` (:24)
                 Real dx[C];
-                chosen_transition<Real, C, E, MODEL>(m, cum, u32_event_f32(w.y) * rtot, dx);  // choose_event + fn_transition (:25-26)
+                chosen_transition<Real, C, E, RMODEL>(m, cum, u32_event_f32(w.y) * rtot, dx);  // choose_event + fn_transition (:25-26)
                 if (go) {
 #pragma unroll
                     for (int c = 0; c < C; ++c) x[s][c] += dx[c];
@@ -339,7 +344,7 @@ pf_sim_weight_kernel(const __grid_constant__ DevModel<Real, C, E> m, const __gri
             } else {
                 if (active[s]) {
                     Real cum[E];
-                    cum_rates<Real, C, E, MODEL>(m, par, x[s], cum);
+                    cum_rates<Real, C, E, RMODEL>(m, par, x[s], cum);
                     const Real rtot = cum[E - 1];
                     fin[s] = !(rtot > (Real)0);  // `cum_rates[end] == 0.0 && break` (:22)
                     if (!fin[s]) {
@@ -352,7 +357,7 @@ pf_sim_weight_kernel(const __grid_constant__ DevModel<Real, C, E> m, const __gri
                             fin[s] = tm[s] > t_obs;                           // `time > tmax && break` (:24)
                             if (!fin[s]) {
                                 Real dx[C];
-                                chosen_transition<Real, C, E, MODEL>(m, cum, __dmul_rn(u32_open_f64(w.y), rtot), dx);
+                                chosen_transition<Real, C, E, RMODEL>(m, cum, __dmul_rn(u32_open_f64(w.y), rtot), dx);
 #pragma unroll
                                 for (int c = 0; c < C; ++c) x[s][c] += dx[c];
                                 ++k[s];
@@ -452,7 +457,26 @@ pf_sim_weight_kernel(const __grid_constant__ DevModel<Real, C, E> m, const __gri
         if (lane == 1 && ev_local) atomicAdd(a.grp_ev + (size_t)b * a.ngroups + tile / kGroupTiles, ev_local);
         if (lane == 1 && ovf_local) atomicAdd(a.ovf_count, ovf_local);
 
-        if (int_obs) {
+        if constexpr (COUNT) {
+            // Count families: the log pmf is not monotone in |Y - X|, so there is no integer min-reduction or exp table; every
+            // particle takes the direct path.  The (filter, observation) constants are CTA-uniform and formed once.
+            const CountObsConst cc = count_obs_const(a.cobs, th, t, ysum);
+            double it[ITEMS], mloc = -INFINITY;
+#pragma unroll
+            for (int kk = 0; kk < ITEMS; ++kk) {
+                it[kk] = excluded[kk] ? -INFINITY : count_obs_logpmf(cc, ysum, (double)xs[kk]);
+                mloc = fmax(mloc, it[kk]);
+            }
+            if (a.record_logw) {
+                double* lw_b = a.logw + (size_t)b * a.n_pad + base_n + (size_t)tid * ITEMS;
+#pragma unroll
+                for (int kk = 0; kk < ITEMS; ++kk) lw_b[kk] = it[kk];
+            }
+            m_b = block_max(mloc, warp_scratch);
+            const double ref = (m_b == -INFINITY) ? 0.0 : m_b;
+#pragma unroll
+            for (int kk = 0; kk < ITEMS; ++kk) av[kk] = (it[kk] == -INFINITY) ? 0.0 : exp(it[kk] - ref);
+        } else if (int_obs) {
             const int ys = (int)ysum;
             unsigned du[ITEMS], dloc = kExcluded;
 #pragma unroll
@@ -616,7 +640,7 @@ pf_sim_weight_kernel(const __grid_constant__ DevModel<Real, C, E> m, const __gri
         const RsArgs ra{a.tile_f, a.tile_off, a.grp_f, a.grp_off, a.filt_s, nullptr, nullptr, nullptr, a.pop_dst, a.anc, a.n, a.n_pad,
                         a.ntiles, a.ngroups, a.n_comp, t, a.rs_type, a.key, a.perm};
         // ovf_s (TILE ints) is free after the weight pass: it becomes the per-warp offspring windows
-        resample_tile<ITEMS, SState, true, 0, true, (MODEL != kModelGeneric ? C : 0)>(ra, b, tile, gfilter, incl, st_s, TILE, ovf_s,
+        resample_tile<ITEMS, SState, true, 0, true, (RMODEL != kModelGeneric ? C : 0)>(ra, b, tile, gfilter, incl, st_s, TILE, ovf_s,
                                                                                       warp_max_s, lohi_s);
         DPOMP_STAMP(1, 4);
     }
@@ -718,7 +742,7 @@ static int sim_inst(const ModelHost& mh, const SimLaunch& a, cudaStream_t stream
         cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
         return per_sm * sms;
     }
-    if constexpr (sizeof(Real) == 4 && MODEL != kModelGeneric) {
+    if constexpr (sizeof(Real) == 4 && MODEL > kModelGeneric) {
         // the persistent kernel is instantiated for the f32 loop of the predefined models
         auto kern_p = pf_sim_weight_kernel<Real, C, E, ITEMS, MODEL, kModePersist, ILP>;
         static bool configured_p = false;
@@ -811,6 +835,21 @@ static int sim_typed(const ModelHost& mh, int items, const SimLaunch& a, cudaStr
     DPOMP_SIM_SHAPES(X)
 #undef X
     return (mode == 2 || mode == 4) ? 0 : (int)cudaErrorInvalidValue;
+}
+
+// count observation families: the generic (C, E) shapes only -- never the predefined-model, persistent or two-per-lane kernels
+template <typename Real>
+static int sim_count_typed(const ModelHost& mh, int items, const SimLaunch& a, cudaStream_t stream, int mode) {
+    if (mode == 3 || mode == 4) return mode == 4 ? 0 : (int)cudaErrorInvalidValue;
+    const int c = mh.desc.n_compartments, e = mh.desc.n_events;
+#define X(CC, EE)                                                                                                \
+    if (c <= CC && e <= EE) {                                                                                    \
+        return items == kItemsSmall ? sim_inst<Real, CC, EE, kItemsSmall, kModelCountObs>(mh, a, stream, mode) \
+                                    : sim_inst<Real, CC, EE, kItemsLarge, kModelCountObs>(mh, a, stream, mode); \
+    }
+    DPOMP_SIM_SHAPES(X)
+#undef X
+    return mode == 2 ? 0 : (int)cudaErrorInvalidValue;
 }
 
 }  // namespace dpomp

@@ -10,7 +10,8 @@ from typing import Callable, Optional, Sequence
 
 import numpy as np
 
-from .rate_table import ObsTable
+from . import _capi
+from .rate_table import ObsTable, count_logpmf
 from .structs import DPOMPModel, Observation
 
 
@@ -95,6 +96,60 @@ class GaussianObsModel:
 def partial_gaussian_obs_model(sigma: float = 2.0, seq=(2,), y_seq=None) -> GaussianObsModel:
     """partial_gaussian_obs_model(σ = 2.0; seq = 2:2, y_seq = seq) (src/hmm_examples.jl:59-67)"""
     return GaussianObsModel(sigma, seq, y_seq)
+
+
+class CountObsModel:
+    """Count observation model: Y = sum(y.val[y_seq]) given X = sum(population[seq]) (1-based index lists, like
+    GaussianObsModel) follows a Poisson, binomial or negative-binomial law (include/dpomp.h DPOMP_OBS_*).  A parameter is a
+    fixed value or, with its *_index (0-based), the theta component of each filter / trajectory, so that pMCMC, SMC^2 and ARQ
+    infer it.  Calls return the log pmf, like the reference's obs_model closures; `obs_table` is what the device evaluates."""
+
+    def __init__(self, family: int, values, indices, seq=(2,), y_seq=None):
+        self.family = int(family)
+        self.par_value = tuple(float(v) for v in values)
+        self.par_index = tuple(-1 if i is None else int(i) for i in indices)
+        self.seq = tuple(int(s) for s in (seq if np.iterable(seq) else (seq,)))
+        ys = self.seq if y_seq is None else y_seq
+        self.y_seq = tuple(int(s) for s in (ys if np.iterable(ys) else (ys,)))
+        if any(i < -1 for i in self.par_index):
+            raise ValueError("parameter indices are 0-based theta components")
+        ok = {_capi.OBS_POISSON: lambda a, k: a > 0.0, _capi.OBS_BINOMIAL: lambda a, k: 0.0 <= a <= 1.0,
+              _capi.OBS_NEGBIN: lambda a, k: a > 0.0 and k > 0.0}[self.family]
+        a, k = (v if i < 0 else 0.5 for v, i in zip(self.par_value, self.par_index))
+        if not ok(a, k) or not all(np.isfinite(self.par_value)):
+            raise ValueError(f"fixed observation parameters {self.par_value} outside their range")
+
+    def __call__(self, y: Observation, population: np.ndarray, theta: np.ndarray) -> float:
+        ys = int(sum(int(y.val[i - 1]) for i in self.y_seq))
+        xs = int(sum(int(population[i - 1]) for i in self.seq))
+        a, k = self.obs_table(len(population), len(y.val)).count_params(theta)
+        return count_logpmf(self.family, ys, xs, a, k)
+
+    def obs_table(self, n_compartments: int, n_obs_vals: int) -> ObsTable:
+        xm = np.zeros(n_compartments, dtype=np.int64)
+        ym = np.zeros(n_obs_vals, dtype=np.int64)
+        for i in self.seq:
+            xm[i - 1] = 1
+        for i in self.y_seq:
+            ym[i - 1] = 1
+        return ObsTable(1.0, xm, ym, self.family, self.par_index, self.par_value)
+
+
+def partial_poisson_obs_model(rho: float = 1.0, rho_index: Optional[int] = None, seq=(2,), y_seq=None) -> CountObsModel:
+    """Cases reported at rate rho: Y ~ Poisson(rho * X), e.g. `logpdf(Poisson(theta[3] * pop[2]), y.val[2])` with
+    rho_index = 2 (0-based)."""
+    return CountObsModel(_capi.OBS_POISSON, (rho, 0.0), (rho_index, None), seq, y_seq)
+
+
+def partial_binomial_obs_model(p: float = 1.0, p_index: Optional[int] = None, seq=(2,), y_seq=None) -> CountObsModel:
+    """Each counted individual detected with probability p: Y ~ Binomial(X, p)."""
+    return CountObsModel(_capi.OBS_BINOMIAL, (p, 0.0), (p_index, None), seq, y_seq)
+
+
+def partial_negbin_obs_model(rho: float = 1.0, k: float = 1.0, rho_index: Optional[int] = None, k_index: Optional[int] = None,
+                             seq=(2,), y_seq=None) -> CountObsModel:
+    """Over-dispersed reporting: Y negative binomial with mean rho * X and size k (variance mu + mu^2 / k)."""
+    return CountObsModel(_capi.OBS_NEGBIN, (rho, k), (rho_index, k_index), seq, y_seq)
 
 
 def generate_model(model_name: str, initial_condition: Sequence[int], freq_dep: bool = False,

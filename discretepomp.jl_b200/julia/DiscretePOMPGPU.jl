@@ -23,6 +23,7 @@ import Random
 const LIBDPOMP = get(ENV, "LIBDPOMP", "libdpomp")
 const DPOMP_RS_SYSTEMATIC, DPOMP_RS_STRATIFIED, DPOMP_RS_MULTINOMIAL = Int32(1), Int32(2), Int32(3)
 const DPOMP_UNIQUE_ID_BYTES = 128
+const DPOMP_OBS_GAUSSIAN, DPOMP_OBS_POISSON, DPOMP_OBS_BINOMIAL, DPOMP_OBS_NEGBIN = Int32(0), Int32(1), Int32(2), Int32(3)
 
 # struct dpomp_model_desc (include/dpomp.h); NTuple-of-64 fields are the row-major [8][8] C arrays
 struct DpompModelDesc
@@ -59,6 +60,7 @@ rows(m::AbstractMatrix, T) = ntuple(k -> (e = (k - 1) ÷ 8 + 1; c = (k - 1) % 8 
 # Model closures -> device rate table.  Closures cannot run on the device: the host PROBES rate_function / obs_model and
 # fits    rate[e] = theta[p_e] * (k1 + f1.x) * (k2 + f2.x) / (kd + dn.x)      (small integer forms)
 #         log g   = log(1/(sqrt(2 pi) sigma)) - (ymask.y - xmask.x)^2 / (2 sigma^2)
+#                   or a Poisson / binomial / negative-binomial log pmf of Y = ymask.y given X = xmask.x (0/1 masks)
 # which covers every predefined model (src/hmm_examples.jl:103-168 incl. freq_dep and ROSSMAC) and the custom model of
 # test/runtests.jl:74-100; the fit is verified on random states and anything else throws ModelCompileError (there is no
 # CPU fallback).  Same algorithm as discretepomp.jl_b200/rate_table.py (compile_rate_table / compile_obs_table), which
@@ -74,7 +76,58 @@ struct ObsTable
     sigma::Float64
     xmask::Vector{Int}
     ymask::Vector{Int}
+    family::Int32                 # DPOMP_OBS_*; count families: parameter i = theta[par_index[i] + 1] or, for -1, par_value[i]
+    par_index::NTuple{2,Int32}    # 0-based (the C ABI's convention)
+    par_value::NTuple{2,Float64}
 end
+ObsTable(sigma, xmask, ymask) = ObsTable(sigma, xmask, ymask, DPOMP_OBS_GAUSSIAN, (Int32(-1), Int32(-1)), (0.0, 0.0))
+
+## log pmf of the count families with the boundary cases of include/dpomp.h (same association as rate_table.count_logpmf)
+function count_logpmf(family, y::Integer, x::Integer, a::Float64, k::Float64 = 0.0)
+    y < 0 && return -Inf
+    yf, xf = Float64(y), Float64(x)
+    if family == DPOMP_OBS_POISSON
+        0.0 < a < Inf || return -Inf
+        x == 0 && return y == 0 ? 0.0 : -Inf
+        ylog = y == 0 ? 0.0 : yf * (log(a) + log(xf))
+        return (ylog - a * xf) - lgamma_f64(yf + 1.0)
+    elseif family == DPOMP_OBS_BINOMIAL
+        (0.0 <= a <= 1.0 && y <= x) || return -Inf
+        a == 0.0 && return y == 0 ? 0.0 : -Inf
+        a == 1.0 && return y == x ? 0.0 : -Inf
+        nx = xf - yf
+        r = (lgamma_f64(xf + 1.0) - lgamma_f64(yf + 1.0)) - lgamma_f64(nx + 1.0)
+        return (r + yf * log(a)) + nx * log1p(-a)
+    else
+        (0.0 < a < Inf && 0.0 < k < Inf) || return -Inf
+        x == 0 && return y == 0 ? 0.0 : -Inf
+        mu = a * xf; km = k + mu
+        r = ((lgamma_f64(yf + k) - lgamma_f64(k)) - lgamma_f64(yf + 1.0)) + k * log(k / km)
+        return y == 0 ? r : r + yf * log(mu / km)
+    end
+end
+lgamma_f64(v::Float64) = Distributions.SpecialFunctions.logabsgamma(v)[1]
+
+## count observation models with the reference's closure signature obs_model(y, population, theta); seq / y_seq are 1-based
+## compartment / value indices, *_index a 1-based theta component (nothing = the fixed value)
+struct CountObsModel <: Function
+    family::Int32
+    par_index::NTuple{2,Int32}
+    par_value::NTuple{2,Float64}
+    seq::Vector{Int}
+    y_seq::Vector{Int}
+end
+function (m::CountObsModel)(y, population, theta)
+    a, k = ntuple(i -> m.par_index[i] >= 0 ? Float64(theta[m.par_index[i] + 1]) : m.par_value[i], 2)
+    return count_logpmf(m.family, sum(y.val[m.y_seq]), sum(population[m.seq]), a, k)
+end
+_idx(i) = i === nothing ? Int32(-1) : Int32(i - 1)
+partial_poisson_obs_model(rho = 1.0; rho_index = nothing, seq = 2:2, y_seq = seq) =
+    CountObsModel(DPOMP_OBS_POISSON, (_idx(rho_index), Int32(-1)), (Float64(rho), 0.0), collect(seq), collect(y_seq))
+partial_binomial_obs_model(p = 1.0; p_index = nothing, seq = 2:2, y_seq = seq) =
+    CountObsModel(DPOMP_OBS_BINOMIAL, (_idx(p_index), Int32(-1)), (Float64(p), 0.0), collect(seq), collect(y_seq))
+partial_negbin_obs_model(rho = 1.0, k = 1.0; rho_index = nothing, k_index = nothing, seq = 2:2, y_seq = seq) =
+    CountObsModel(DPOMP_OBS_NEGBIN, (_idx(rho_index), _idx(k_index)), (Float64(rho), Float64(k)), collect(seq), collect(y_seq))
 
 function call_rates(rate_function::Function, E::Int, theta::Vector{Float64}, x::Vector{Int64})
     out = zeros(Float64, E)
@@ -248,6 +301,24 @@ function combinations_of(n::Int, k::Int)
 end
 
 function fit_obs_table(obs_model::Function, C::Int, V::Int, n_params::Int)
+    if obs_model isa CountObsModel
+        xm, ym = zeros(Int, C), zeros(Int, V)
+        xm[obs_model.seq] .= 1; ym[obs_model.y_seq] .= 1
+        return ObsTable(1.0, xm, ym, obs_model.family, obs_model.par_index, obs_model.par_value)
+    end
+    tab = try
+        fit_gaussian_obs(obs_model, C, V, n_params)
+    catch e
+        e isa Union{DomainError, InexactError, OverflowError} || rethrow()
+        nothing
+    end
+    tab === nothing && (tab = fit_count_obs(obs_model, C, V, n_params))
+    tab === nothing && throw(ModelCompileError("obs_model is not a Gaussian in integer masks of (y, x), nor a Poisson, binomial or " *
+                                               "negative-binomial law of 0/1 masks; no device table"))
+    return tab
+end
+
+function fit_gaussian_obs(obs_model::Function, C::Int, V::Int, n_params::Int)
     theta = ones(n_params)
     g(yv, xv) = Float64(obs_model(Observation(0.0, 1, 1.0, Int64.(yv)), Int64.(xv), theta))
     zy, zx = zeros(Int64, V), zeros(Int64, C)
@@ -277,10 +348,64 @@ function fit_obs_table(obs_model::Function, C::Int, V::Int, n_params::Int)
     for _ in 1:64
         y = Int64.(rand(rng, 0:49, V)); x = Int64.(rand(rng, 0:49, C))
         d = sum(ym .* y) - sum(xm .* x)
-        isapprox(tmp1 - d * d / tmp2, g(y, x); rtol = 1e-10, atol = 1e-12) ||
-            throw(ModelCompileError("obs_model is not a Gaussian in integer masks of (y, x); no device table"))
+        isapprox(tmp1 - d * d / tmp2, g(y, x); rtol = 1e-10, atol = 1e-12) || return nothing
     end
     return ObsTable(sigma, xm, ym)
+end
+
+snap(v) = (s = round(v; sigdigits = 12); abs(s - v) <= 1e-12 * abs(v) ? s : v)
+
+## count-law probe, as rate_table._fit_count_obs: 0/1 masks from the components that move the value, parameters from probe
+## points (g(0, X) = -rho X; g(1, 1) = log p; g(1, X) - g(0, X) = log(k mu / (k + mu)) at X = 1, 2), theta-indexing by
+## perturbing each theta component, then 64 random verification points
+function fit_count_obs(obs_model::Function, C::Int, V::Int, n_params::Int)
+    rng = Random.MersenneTwister(11)
+    theta0 = 0.2 .+ 0.6 .* rand(rng, n_params)
+    g(yv, xv, th) = Float64(obs_model(Observation(0.0, 1, 1.0, Int64.(yv)), Int64.(xv), th))
+    try
+        x0, y0 = fill(Int64(50), C), ones(Int64, V)
+        base = g(y0, x0, theta0)
+        isfinite(base) || return nothing
+        xm = [Int(g(y0, (x = copy(x0); x[i] += 1; x), theta0) != base) for i in 1:C]
+        ym = [Int(g((y = copy(y0); y[j] += 1; y), x0, theta0) != base) for j in 1:V]
+        (any(xm .== 1) && any(ym .== 1)) || return nothing
+        ix, iy = findfirst(==(1), xm), findfirst(==(1), ym)
+        G(yy, xx, th) = g((y = zeros(Int64, V); y[iy] = yy; y), (x = zeros(Int64, C); x[ix] = xx; x), th)
+        function fit(family, th)
+            family == DPOMP_OBS_POISSON && return (-G(0, 1, th), 0.0)
+            family == DPOMP_OBS_BINOMIAL && return (exp(G(1, 1, th)), 0.0)
+            e1 = exp(-(G(1, 1, th) - G(0, 1, th))); e2 = exp(-(G(1, 2, th) - G(0, 2, th)))
+            return (1.0 / (2.0 * (e1 - e2)), 1.0 / (2.0 * e2 - e1))
+        end
+        for family in (DPOMP_OBS_POISSON, DPOMP_OBS_BINOMIAL, DPOMP_OBS_NEGBIN)
+            n_par = family == DPOMP_OBS_NEGBIN ? 2 : 1
+            vals = fit(family, theta0)
+            all(isfinite, vals[1:n_par]) || continue
+            idx, fixed = [Int32(-1), Int32(-1)], [0.0, 0.0]
+            for i in 1:n_par
+                for j in 1:n_params
+                    isapprox(vals[i], theta0[j]; rtol = 1e-9) || continue
+                    th = copy(theta0); th[j] *= 0.9
+                    if isapprox(fit(family, th)[i], th[j]; rtol = 1e-9)
+                        idx[i] = Int32(j - 1); break
+                    end
+                end
+                idx[i] < 0 && (fixed[i] = snap(vals[i]))
+            end
+            tab = ObsTable(1.0, xm, ym, family, (idx[1], idx[2]), (fixed[1], fixed[2]))
+            vrng = Random.MersenneTwister(7)
+            ok = all(1:64) do _
+                y = Int64.(rand(vrng, 0:19, V)); x = Int64.(rand(vrng, 0:59, C)); th = 0.2 .+ 0.6 .* rand(vrng, n_params)
+                a, k = ntuple(i -> tab.par_index[i] >= 0 ? th[tab.par_index[i] + 1] : tab.par_value[i], 2)
+                got, want = count_logpmf(family, sum(ym .* y), sum(xm .* x), a, k), g(y, x, th)
+                got == want || isapprox(got, want; rtol = 1e-9, atol = 1e-9)
+            end
+            ok && return tab
+        end
+    catch e
+        e isa Union{DomainError, InexactError, OverflowError, ArgumentError, BoundsError} || rethrow()
+    end
+    return nothing
 end
 
 # --------------------------------------------------------------------------------------------------------------------
@@ -311,6 +436,13 @@ function dpomp_model(model::HiddenMarkovModel)
             ot.sigma, pad(ot.xmask, 8, Int32), V, pad(ot.ymask, 8, Int32),
             length(times), pointer(times), pointer(ids), pointer(vals))
         dpomp_check(ccall((:dpomp_model_create, LIBDPOMP), Cint, (Ref{DpompModelDesc}, Ref{Ptr{Cvoid}}), desc, handle))
+    end
+    if ot.family != DPOMP_OBS_GAUSSIAN
+        pidx, pval = Int32[ot.par_index...], Float64[ot.par_value...]
+        rc = GC.@preserve pidx pval ccall((:dpomp_model_set_obs_model, LIBDPOMP), Cint, (Ptr{Cvoid}, Int32, Ptr{Int32}, Ptr{Float64}),
+                                          handle[], ot.family, pidx, pval)
+        rc == 0 || ccall((:dpomp_model_destroy, LIBDPOMP), Cint, (Ptr{Cvoid},), handle[])
+        dpomp_check(rc)
     end
     m = DpompModel(handle[], n_params)      # the library copied the observations
     finalizer(x -> ccall((:dpomp_model_destroy, LIBDPOMP), Cint, (Ptr{Cvoid},), x.handle), m)

@@ -35,6 +35,11 @@ class DeviceModel:
         self.compiled = compiled
         self._h = C.c_void_p()
         _capi.check(_capi.lib().dpomp_model_create(C.byref(compiled.desc), C.byref(self._h)))
+        obs = compiled.obs
+        if obs is not None and obs.family != _capi.OBS_GAUSSIAN:
+            idx = np.ascontiguousarray(obs.par_index, dtype=np.int32)
+            val = np.ascontiguousarray(obs.par_value, dtype=np.float64)
+            _capi.check(_capi.lib().dpomp_model_set_obs_model(self._h, int(obs.family), _capi.ptr(idx), _capi.ptr(val)))
 
     @property
     def handle(self) -> C.c_void_p:

@@ -6,6 +6,7 @@ PROBES them and fits the table
 
     rate[e] = theta[p_e] * (k1 + f1.x) * (k2 + f2.x) / (kd + dn.x)          (integer forms)
     log g   = log(1/(sqrt(2 pi) sigma)) - (ymask.y - xmask.x)^2 / (2 sigma^2)
+          or  a Poisson / binomial / negative-binomial log pmf of Y = ymask.y given X = xmask.x (0/1 masks)
 
 which covers every predefined model (src/hmm_examples.jl:103-168, incl. freq_dep and ROSSMAC) and the custom models of
 the reference's tests (test/runtests.jl:74-100).  The fit is verified on random states; a closure that does not fit
@@ -18,6 +19,8 @@ from dataclasses import dataclass, field
 from typing import Callable, List, Optional, Sequence
 
 import numpy as np
+
+import math
 
 from . import _capi
 from .structs import Observation
@@ -61,6 +64,52 @@ class ObsTable:
     sigma: float
     xmask: np.ndarray  # (C,)
     ymask: np.ndarray  # (V,)
+    # observation family (include/dpomp.h DPOMP_OBS_*); count families: parameter i is theta[par_index[i]] (0-based) or,
+    # for par_index[i] = -1, the fixed par_value[i]; Poisson (rho, -), binomial (p, -), negative binomial (rho, k)
+    family: int = _capi.OBS_GAUSSIAN
+    par_index: tuple = (-1, -1)
+    par_value: tuple = (0.0, 0.0)
+
+    def count_params(self, theta) -> tuple:
+        """(a, k) of a count family at theta: a = rho or p, k = negative-binomial size."""
+        return tuple(float(theta[i]) if i >= 0 else float(v) for i, v in zip(self.par_index, self.par_value))
+
+
+def count_logpmf(family: int, y: int, x: int, a: float, k: float = 0.0) -> float:
+    """log g(Y = y | X = x) of a count family with the boundary cases of include/dpomp.h: 0 log 0 = 0, a zero mean gives 0 for
+    y = 0 and -inf otherwise, y > x in the binomial gives -inf, p = 0 / 1 are exact, a parameter out of range gives -inf.  Same
+    association as the device code and the oracle."""
+    y, x = int(y), int(x)
+    if y < 0:
+        return -math.inf
+    yf, xf = float(y), float(x)
+    if family == _capi.OBS_POISSON:
+        if not (0.0 < a < math.inf):
+            return -math.inf
+        if x == 0:
+            return 0.0 if y == 0 else -math.inf
+        ylog = 0.0 if y == 0 else yf * (math.log(a) + math.log(xf))
+        return (ylog - a * xf) - math.lgamma(yf + 1.0)
+    if family == _capi.OBS_BINOMIAL:
+        if not (0.0 <= a <= 1.0) or y > x:
+            return -math.inf
+        if a == 0.0:
+            return 0.0 if y == 0 else -math.inf
+        if a == 1.0:
+            return 0.0 if y == x else -math.inf
+        nx = xf - yf
+        r = (math.lgamma(xf + 1.0) - math.lgamma(yf + 1.0)) - math.lgamma(nx + 1.0)
+        return (r + yf * math.log(a)) + nx * math.log1p(-a)
+    if family == _capi.OBS_NEGBIN:
+        if not (0.0 < a < math.inf) or not (0.0 < k < math.inf):
+            return -math.inf
+        if x == 0:
+            return 0.0 if y == 0 else -math.inf
+        mu = a * xf
+        km = k + mu
+        r = ((math.lgamma(yf + k) - math.lgamma(k)) - math.lgamma(yf + 1.0)) + k * math.log(k / km)
+        return r if y == 0 else r + yf * math.log(mu / km)
+    raise ValueError(f"unknown count family {family}")
 
 
 def _call_rates(fn: Callable, n_events: int, theta: np.ndarray, x: np.ndarray) -> np.ndarray:
@@ -204,10 +253,24 @@ def compile_rate_table(rate_function: Callable, n_events: int, n_params: int, n_
 
 
 def compile_obs_table(obs_model: Callable, n_compartments: int, n_obs_vals: int, n_params: int) -> ObsTable:
-    """Fit the Gaussian observation table; objects produced by partial_gaussian_obs_model carry it directly."""
+    """Fit the observation table: the Gaussian first, then the count families.  Objects produced by
+    partial_gaussian_obs_model and the partial_*_obs_model count constructors carry it directly."""
     direct = getattr(obs_model, "obs_table", None)
     if direct is not None:
         return direct(n_compartments, n_obs_vals)
+    try:
+        tab = _fit_gaussian_obs(obs_model, n_compartments, n_obs_vals, n_params)
+    except (ArithmeticError, ValueError):  # a count law: -inf / degenerate values at the Gaussian probe points
+        tab = None
+    if tab is None:
+        tab = _fit_count_obs(obs_model, n_compartments, n_obs_vals, n_params)
+    if tab is None:
+        raise ModelCompileError("obs_model is not a Gaussian in integer masks of (y, x), nor a Poisson, binomial or negative-binomial "
+                                "law of 0/1 masks; no device table")
+    return tab
+
+
+def _fit_gaussian_obs(obs_model: Callable, n_compartments: int, n_obs_vals: int, n_params: int) -> Optional[ObsTable]:
     c, v = n_compartments, n_obs_vals
     theta = np.ones(n_params)
 
@@ -243,8 +306,104 @@ def compile_obs_table(obs_model: Callable, n_compartments: int, n_obs_vals: int,
         want = g(y, x)
         d = int(ym @ y) - int(xm @ x)
         if not np.isclose(tmp1 - d * d / tmp2, want, rtol=1e-10, atol=1e-12):
-            raise ModelCompileError("obs_model is not a Gaussian in integer masks of (y, x); no device table")
+            return None
     return tab
+
+
+def _snap(v: float) -> float:
+    """a probed parameter read back through exp / log: the nearby 12-digit decimal when it is that value up to rounding"""
+    s = float(f"{v:.12g}")
+    return s if abs(s - v) <= 1e-12 * abs(v) else v
+
+
+def _fit_count_obs(obs_model: Callable, n_compartments: int, n_obs_vals: int, n_params: int) -> Optional[ObsTable]:
+    """Probe a closure for a count law: 0/1 masks from the components that move its value, the parameters from a few probe
+    points (g(0, X) = -rho X for the Poisson, g(1, 1) = log p for the binomial, g(1, X) - g(0, X) = log(k mu / (k + mu)) at
+    X = 1, 2 for the negative binomial), theta-indexing by perturbing each theta component, then 64 random verification points."""
+    c, v = n_compartments, n_obs_vals
+    rng = np.random.default_rng(11)
+    theta0 = rng.uniform(0.2, 0.8, size=n_params)
+
+    def g(yv, xv, th):
+        with np.errstate(all="ignore"):
+            return float(obs_model(Observation(0.0, 1, 1.0, np.asarray(yv, dtype=np.int64)), np.asarray(xv, dtype=np.int64),
+                                   np.asarray(th, dtype=np.float64)))
+
+    try:
+        # 1. masks: components whose unit change moves the value at an interior point (Y well below X)
+        x0, y0 = np.full(c, 50, dtype=np.int64), np.ones(v, dtype=np.int64)
+        base = g(y0, x0, theta0)
+        if not math.isfinite(base):
+            return None
+        xm = np.zeros(c, dtype=np.int64)
+        ym = np.zeros(v, dtype=np.int64)
+        for i in range(c):
+            x = x0.copy(); x[i] += 1
+            xm[i] = int(g(y0, x, theta0) != base)
+        for j in range(v):
+            y = y0.copy(); y[j] += 1
+            ym[j] = int(g(y, x0, theta0) != base)
+        if not xm.any() or not ym.any():
+            return None
+        ix, iy = int(np.argmax(xm)), int(np.argmax(ym))
+
+        def G(yy, xx, th):  # Y in the first y component of the mask, X in the first x component, the rest zero
+            y = np.zeros(v, dtype=np.int64); y[iy] = yy
+            x = np.zeros(c, dtype=np.int64); x[ix] = xx
+            return g(y, x, th)
+
+        # 2. parameters of each family at theta, None if the probe values are not those of the family
+        def fit(family, th):
+            if family == _capi.OBS_POISSON:
+                return (-G(0, 1, th), 0.0)
+            if family == _capi.OBS_BINOMIAL:
+                return (math.exp(G(1, 1, th)), 0.0)
+            e1 = math.exp(-(G(1, 1, th) - G(0, 1, th)))
+            e2 = math.exp(-(G(1, 2, th) - G(0, 2, th)))
+            inv_rho, inv_k = 2.0 * (e1 - e2), 2.0 * e2 - e1
+            return (1.0 / inv_rho, 1.0 / inv_k)
+
+        for family in (_capi.OBS_POISSON, _capi.OBS_BINOMIAL, _capi.OBS_NEGBIN):
+            n_par = 2 if family == _capi.OBS_NEGBIN else 1
+            try:
+                vals = fit(family, theta0)
+            except (ArithmeticError, ValueError):
+                continue
+            if not all(math.isfinite(vals[i]) for i in range(n_par)):
+                continue
+            # 3. theta-indexing: a parameter equal to theta[j] that follows a perturbation of theta[j]
+            idx, fixed = [-1, -1], [0.0, 0.0]
+            for i in range(n_par):
+                for jth in range(n_params):
+                    if not math.isclose(vals[i], theta0[jth], rel_tol=1e-9):
+                        continue
+                    th = theta0.copy(); th[jth] *= 0.9
+                    try:
+                        moved = fit(family, th)[i]
+                    except (ArithmeticError, ValueError):
+                        continue
+                    if math.isclose(moved, th[jth], rel_tol=1e-9):
+                        idx[i] = jth
+                        break
+                if idx[i] < 0:
+                    fixed[i] = _snap(vals[i])
+            tab = ObsTable(1.0, xm, ym, family, tuple(idx), tuple(fixed))
+            # 4. verification on random points (scipy / lgamma closures agree with the table to rounding)
+            ok = True
+            vrng = np.random.default_rng(7)
+            for _ in range(64):
+                y = vrng.integers(0, 20, size=v); x = vrng.integers(0, 60, size=c)
+                th = vrng.uniform(0.2, 0.8, size=n_params)
+                want = g(y, x, th)
+                got = count_logpmf(family, int(ym @ y), int(xm @ x), *tab.count_params(th))
+                if not (got == want or np.isclose(got, want, rtol=1e-9, atol=1e-9)):
+                    ok = False
+                    break
+            if ok:
+                return tab
+    except (ArithmeticError, ValueError, TypeError, IndexError):
+        return None
+    return None
 
 
 @dataclass
@@ -283,6 +442,9 @@ def build_model_desc(rate: RateTable, obs: ObsTable, m_transition: np.ndarray, i
         d.initial_condition[k] = int(initial_condition[k])
         d.obs_xmask[k] = int(obs.xmask[k])
     d.obs_sigma = float(obs.sigma)
+    # the count-family oracle (oracle/count_oracle.py) reads the observation family from here; the device model gets it through
+    # dpomp_model_set_obs_model (particle_filter.DeviceModel)
+    d.obs_spec = (int(obs.family), tuple(int(i) for i in obs.par_index), tuple(float(p) for p in obs.par_value))
     n_t = len(obs_data)
     v = len(obs_data[0].val) if n_t else 1
     if not (1 <= v <= _capi.MAX_OBS_VALS):

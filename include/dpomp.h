@@ -64,6 +64,7 @@ typedef enum dpomp_status {
  *
  *   observation model (Gaussian, partial_gaussian_obs_model src/hmm_examples.jl:59-67):
  *       log g = log(1/(sqrt(2 pi) sigma)) - (sum_v obs_ymask[v]*y.val[v] - sum_c obs_xmask[c]*x[c])^2 / (2 sigma^2)
+ *   or one of the count families selected by dpomp_model_set_obs_model (below), on the same masks.
  */
 typedef struct dpomp_model_desc {
     int32_t n_compartments;                                   /* C, 1..DPOMP_MAX_COMPARTMENTS */
@@ -103,6 +104,37 @@ int dpomp_device_count(int* out_count);
 /* replaces get_private_model (src/DiscretePOMP.jl:96-99): validates the descriptor, copies observations */
 int dpomp_model_create(const dpomp_model_desc* desc, dpomp_model** out_model);
 int dpomp_model_destroy(dpomp_model* model);
+
+/*
+ * Observation family of a model (the reference's arbitrary obs_model closure restricted to the laws epidemic counts are
+ * modelled with).  Write Y = sum_v obs_ymask[v] * y.val[v] and X = sum_c obs_xmask[c] * x[c]; for the count families both
+ * masks must have 0/1 entries.  Every log g is evaluated in f64 on the device, by both event loops.
+ *
+ *   DPOMP_OBS_GAUSSIAN  the desc's obs_sigma and masks (the law above the descriptor): the default of dpomp_model_create
+ *   DPOMP_OBS_POISSON   Y ~ Poisson(rho X):          log g = Y log(rho X) - rho X - lgamma(Y+1)                         rho > 0
+ *   DPOMP_OBS_BINOMIAL  Y ~ Binomial(X, p):          log g = lgamma(X+1) - lgamma(Y+1) - lgamma(X-Y+1)
+ *                                                            + Y log p + (X-Y) log1p(-p)                            0 <= p <= 1
+ *   DPOMP_OBS_NEGBIN    mean mu = rho X, size k:     log g = lgamma(Y+k) - lgamma(k) - lgamma(Y+1)
+ *                                                            + k log(k/(k+mu)) + Y log(mu/(k+mu))                rho > 0, k > 0
+ * Parameters: Poisson (rho, unused), binomial (p, unused), negative binomial (rho, k).  par_index[i] >= 0 takes parameter i
+ * from theta[par_index[i]] (0-based) of each filter / trajectory, so pMCMC, SMC^2 and ARQ can infer it; par_index[i] = -1
+ * takes the fixed par_value[i].
+ * Boundary cases: 0 log 0 = 0; rho X = 0 (or mu = 0) gives log g = 0 when Y = 0 and -Inf otherwise; Y > X in the binomial
+ * gives -Inf; p = 0 and p = 1 are exact (log g = 0 for Y = 0, resp. Y = X, else -Inf); Y < 0 gives -Inf.  A theta-indexed
+ * value outside its range (p outside [0, 1], rho or k not positive and finite) gives -Inf for every particle: the filter
+ * then returns what it returns when every weight is zero, and an MH step rejects the proposal.
+ * obs_sigma keeps its validation in dpomp_model_create and is ignored by the count families.  The per-observation constants
+ * lgamma(Y+1) and, for a fixed k, lgamma(Y+k) - lgamma(k) are computed on the host.
+ * Returns DPOMP_ERR_ARG for an unknown family or a null pointer, DPOMP_ERR_MODEL for an index >= n_params, a fixed value out of
+ * range or a mask entry other than 0 / 1, and DPOMP_ERR_STATE once a filter or MBP handle has been created from the model
+ * (handles read the model when they launch, so it is frozen from then on).
+ */
+#define DPOMP_OBS_GAUSSIAN 0 /* the desc's sigma / masks: the default */
+#define DPOMP_OBS_POISSON 1
+#define DPOMP_OBS_BINOMIAL 2
+#define DPOMP_OBS_NEGBIN 3
+int dpomp_model_set_obs_model(dpomp_model* model, int32_t family, const int32_t* par_index /*[2], -1 = fixed*/,
+                              const double* par_value /*[2]*/);
 
 /*
  * A batch of n_batch independent bootstrap filters of n_particles each on one device
