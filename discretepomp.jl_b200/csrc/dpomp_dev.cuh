@@ -236,6 +236,22 @@ __device__ __forceinline__ double u32_open_f64(uint32_t w) { return ((double)w +
 //                 rate and choose_event can never fall through to a zero-rate last event
 __device__ __forceinline__ float u32_wait_f32(uint32_t w) { return fmaf(__uint2float_rn(w), 0x1.0p-32f, 0x1.0p-33f); }
 __device__ __forceinline__ float u32_event_f32(uint32_t w) { return __uint2float_rz(w) * 0x1.0p-32f; }
+// The two XU operations of the f32 waiting time, pinned to their flush-to-zero forms whatever -ftz the translation unit is
+// built with (the non-ftz forms add a denormal scaling and, for the quotient, a range fix-up around the MUFU):
+//   lg2_ftz: the argument is u32_wait_f32(w) >= 2^-33, never subnormal, so the ftz form returns the same value;
+//   rcp_ftz: for every normal total rate the same value as the non-ftz reciprocal.  A subnormal rate (flushed to 0) gives
+//            +inf instead of ~1e38, so the new remaining time is -inf or NaN rather than a huge negative number: the attempt
+//            fails `t_new >= 0` either way.
+__device__ __forceinline__ float lg2_ftz(float x) {
+    float y;
+    asm("lg2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
+    return y;
+}
+__device__ __forceinline__ float rcp_ftz(float x) {
+    float y;
+    asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
+    return y;
+}
 // [0,1) with 53-bit resolution (Julia's rand() range) for the resampling draws
 __device__ __forceinline__ double u53(uint32_t hi, uint32_t lo) {
     return (double)(((uint64_t)hi << 21) | (uint64_t)(lo >> 11)) * 0x1.0p-53;

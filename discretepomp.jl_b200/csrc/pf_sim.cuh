@@ -149,7 +149,7 @@ pf_sim_weight_kernel(const __grid_constant__ DevModel<Real, C, E> m, const __gri
     // staged compartment counts: f32 loop keeps them as floats (no conversions in the divergent refill path; exact
     // below 2^24), the f64 parity loop as int32
     using SState = typename std::conditional<kF32, float, int>::type;
-    int* ovf_s = reinterpret_cast<int*>(smem_raw);        // [TILE] 1 = the particle hit the event cap
+    int* ovf_s = reinterpret_cast<int*>(smem_raw);        // [TILE] parked particle: events | (hit the event cap) << 31
     SState* st_s = reinterpret_cast<SState*>(ovf_s + TILE);  // [C][TILE]
     __shared__ double warp_scratch[kBlockThreads / 32];
     __shared__ unsigned warp_min_s[kBlockThreads / 32];
@@ -277,10 +277,13 @@ pf_sim_weight_kernel(const __grid_constant__ DevModel<Real, C, E> m, const __gri
     const long long left = a.n - (base_n + chunk0);
     const int chunk_valid = left < CHUNK ? (left > 0 ? (int)left : 0) : CHUNK;
     const unsigned lt_mask = (1u << lane) - 1u;
-    int next = 32 * S;  // warp-uniform: next unassigned slot of the chunk
-    int parked = 0;     // warp-uniform: particles of the chunk that are done
+    // Warp-uniform queue head: tile index of the next unassigned slot of the chunk.  Every slot handed out after the first
+    // 32 * S replaces a parked particle, so head - chunk0 - 32 * S particles are done.  A lane's particle is its tile index q;
+    // slots at or past chunk_valid are idle, so `q < qend` is the lane's active flag.
+    int head = chunk0 + 32 * S;
+    const int qend = chunk0 + chunk_valid;
+    const uint32_t g_tile = (uint32_t)base_n;  // global index of the tile's first particle (mod 2^32)
     int q[S];
-    bool active[S];
     Real x[S][C];
     Real tm[S];
     const Real tm0 = kF32 ? (Real)(t_obs - t_prev) : (Real)t_prev;  // f32: remaining time; f64: absolute time
@@ -294,21 +297,21 @@ pf_sim_weight_kernel(const __grid_constant__ DevModel<Real, C, E> m, const __gri
     // and the loop is issue bound there.
     constexpr bool PIPE = DPOMP_SIM_PIPE && kF32 && S == 2;
     uint2 wn[S];
-    unsigned long long ev_local = 0, ovf_local = 0;
 #pragma unroll
     for (int s = 0; s < S; ++s) {
         const int slot = lane + 32 * s;
-        active[s] = slot < chunk_valid;
-        q[s] = chunk0 + (slot < CHUNK ? slot : lane);
+        const int q0 = chunk0 + (slot < CHUNK ? slot : lane);
+        q[s] = chunk0 + slot;
         tm[s] = tm0;
         k[s] = 0;
-        pc[s] = (uint32_t)(base_n + q[s]) ^ ss.a;
+        pc[s] = (uint32_t)(base_n + q0) ^ ss.a;
         if constexpr (PIPE) wn[s] = philox2x32_10(pc[s], 0u ^ ss.b, ss.k);
 #pragma unroll
-        for (int c = 0; c < C; ++c) x[s][c] = (c < n_comp) ? (Real)st_s[c * TILE + q[s]] : (Real)0;  // idle lanes: harmless values
+        for (int c = 0; c < C; ++c) x[s][c] = (c < n_comp) ? (Real)st_s[c * TILE + q0] : (Real)0;  // idle lanes: harmless values
     }
 
-    while (parked < chunk_valid) {
+    const int head_end = qend + 32 * S;  // head once every particle of the chunk is parked
+    while (head < head_end) {
         bool fin[S], ovf[S];
 #pragma unroll
         for (int s = 0; s < S; ++s) {
@@ -328,7 +331,7 @@ pf_sim_weight_kernel(const __grid_constant__ DevModel<Real, C, E> m, const __gri
                     w = philox2x32_10(pc[s], k[s] ^ ss.b, ss.k);
                 }
                 // time -= log(rand()) / R  (:23) as remaining time; lg2.approx + rcp.approx on the XU pipe
-                const Real tmn = fmaf(__log2f(u32_wait_f32(w.x)), __fdividef(0.693147180559945f, rtot), tm[s]);
+                const Real tmn = fmaf(lg2_ftz(u32_wait_f32(w.x)), rcp_ftz(rtot) * 0.693147180559945f, tm[s]);
                 const bool capped = k[s] >= max_ev;  // event cap: documented divergence, the reference loop is unbounded
                 const bool go = (rtot > (Real)0) && !capped && (tmn >= (Real)0);  // `time > tmax && break` (:24)
                 Real dx[C];
@@ -337,12 +340,12 @@ pf_sim_weight_kernel(const __grid_constant__ DevModel<Real, C, E> m, const __gri
 #pragma unroll
                     for (int c = 0; c < C; ++c) x[s][c] += dx[c];
                     ++k[s];
-                    tm[s] = tmn;
                 }
-                fin[s] = active[s] && !go;
+                tm[s] = tmn;  // a failed attempt ends the particle, whose remaining time is never read again
+                fin[s] = q[s] < qend && !go;
                 ovf[s] = capped && (rtot > (Real)0);
             } else {
-                if (active[s]) {
+                if (q[s] < qend) {
                     Real cum[E];
                     cum_rates<Real, C, E, RMODEL>(m, par, x[s], cum);
                     const Real rtot = cum[E - 1];
@@ -371,34 +374,32 @@ pf_sim_weight_kernel(const __grid_constant__ DevModel<Real, C, E> m, const __gri
         for (int s = 0; s < S; ++s) {
             const unsigned fmask = __ballot_sync(FULL, fin[s]);
             if (fmask) {  // warp-uniform: finished lanes park their particle and pull the next slot of the chunk
+                // Park (finished lanes) and refill (finished lanes that get a slot of the chunk) as flat predicated blocks: no
+                // divergent region to reconverge.  Park stores the particle's event count and cap flag as k | ovf << 31
+                // (k <= max_ev < 2^31), summed in the weight pass; the flag needs no `fin` guard, since an active lane with
+                // ovf always parks and an idle lane's k is never stored.
+                if (ovf[s]) k[s] |= 0x80000000u;
                 if (fin[s]) {
                     DPOMP_CHECK_IDX(q[s], TILE);
 #pragma unroll
                     for (int c = 0; c < C; ++c)
                         if (c < n_comp) st_s[c * TILE + q[s]] = (SState)x[s][c];
-                    if (ovf[s]) {
-                        ovf_s[q[s]] = 1;
-                        ++ovf_local;
-                    }
-                    ev_local += k[s];
-                    const int slot = next + __popc(fmask & lt_mask);
-                    active[s] = slot < chunk_valid;
-                    if (active[s]) {
-                        q[s] = chunk0 + slot;
-                        DPOMP_CHECK_IDX(q[s], TILE);
-                        DPOMP_CHECK_IDX(slot, CHUNK);
-                        DPOMP_CHECK_IDX(base_n + q[s], a.n);
-                        pc[s] = (uint32_t)(base_n + q[s]) ^ ss.a;
-#pragma unroll
-                        for (int c = 0; c < C; ++c) x[s][c] = (c < n_comp) ? (Real)st_s[c * TILE + q[s]] : (Real)0;
-                        tm[s] = tm0;
-                        k[s] = 0;
-                        if constexpr (PIPE) wn[s] = philox2x32_10(pc[s], 0u ^ ss.b, ss.k);
-                    }
+                    ovf_s[q[s]] = (int)k[s];
                 }
-                const int nf = __popc(fmask);
-                next += nf;
-                parked += nf;
+                const int qn = head + __popc(fmask & lt_mask);
+                if (fin[s]) q[s] = qn;
+                if (fin[s] && qn < qend) {
+                    DPOMP_CHECK_IDX(qn, TILE);
+                    DPOMP_CHECK_IDX(qn - chunk0, CHUNK);
+                    DPOMP_CHECK_IDX(base_n + qn, a.n);
+                    pc[s] = (g_tile + (uint32_t)qn) ^ ss.a;
+#pragma unroll
+                    for (int c = 0; c < C; ++c) x[s][c] = (c < n_comp) ? (Real)st_s[c * TILE + qn] : (Real)0;
+                    tm[s] = tm0;
+                    k[s] = 0;
+                    if constexpr (PIPE) wn[s] = philox2x32_10(pc[s], 0u ^ ss.b, ss.k);
+                }
+                head += __popc(fmask);
             }
         }
     }
@@ -441,21 +442,26 @@ pf_sim_weight_kernel(const __grid_constant__ DevModel<Real, C, E> m, const __gri
         const Vec of = *reinterpret_cast<const Vec*>(ovf_s + tid * ITEMS);
         bool excluded[ITEMS];
 #pragma unroll
-        for (int kk = 0; kk < ITEMS; ++kk) excluded[kk] = !(base_n + tid * ITEMS + kk < a.n) || of.v[kk] != 0;
+        for (int kk = 0; kk < ITEMS; ++kk) excluded[kk] = !(base_n + tid * ITEMS + kk < a.n) || of.v[kk] < 0;
 
-        // event statistics: one RED per warp, issued by lane 1 -- thread 0 takes the tickets below, and its __threadfence
-        // would wait for its own RED, queued behind those of every other warp on the same address
+        // event statistics (padding slots are never parked and stay 0): one RED per warp, spread over one counter per
+        // (filter, group of tiles) -- round 1 put all 4096 REDs of a C2 launch on ONE address (0.8 us per observation),
+        // summing along the combine tree instead lengthened the serial tail by more than that; the counters are summed by a
+        // tiny kernel at the end of the call (capi.cu).  Issued by lane 1: thread 0 takes the tickets below, and its
+        // __threadfence would wait for its own RED
+        unsigned long long ev_w = 0, ovf_w = 0;
+#pragma unroll
+        for (int kk = 0; kk < ITEMS; ++kk) {
+            ev_w += (uint32_t)of.v[kk] & 0x7fffffffu;
+            ovf_w += of.v[kk] < 0;
+        }
 #pragma unroll
         for (int d = 16; d > 0; d >>= 1) {
-            ev_local += __shfl_xor_sync(0xffffffffu, ev_local, d);
-            ovf_local += __shfl_xor_sync(0xffffffffu, ovf_local, d);
+            ev_w += __shfl_xor_sync(0xffffffffu, ev_w, d);
+            ovf_w += __shfl_xor_sync(0xffffffffu, ovf_w, d);
         }
-        // event statistics: one RED per warp, spread over one counter per (filter, group of tiles) -- round 1 put all 4096 REDs
-        // of a C2 launch on ONE address (0.8 us per observation), summing along the combine tree instead lengthened the serial
-        // tail by more than that; the counters are summed by a tiny kernel at the end of the call (capi.cu).  Issued by lane 1:
-        // thread 0 takes the tickets below, and its __threadfence would wait for its own RED
-        if (lane == 1 && ev_local) atomicAdd(a.grp_ev + (size_t)b * a.ngroups + tile / kGroupTiles, ev_local);
-        if (lane == 1 && ovf_local) atomicAdd(a.ovf_count, ovf_local);
+        if (lane == 1 && ev_w) atomicAdd(a.grp_ev + (size_t)b * a.ngroups + tile / kGroupTiles, ev_w);
+        if (lane == 1 && ovf_w) atomicAdd(a.ovf_count, ovf_w);
 
         if constexpr (COUNT) {
             // Count families: the log pmf is not monotone in |Y - X|, so there is no integer min-reduction or exp table; every
