@@ -27,6 +27,7 @@ from .ibis import (compute_is_mu_covar, get_mv_param, get_prop_density, run_ibis
 from .mcmc import gelman_diagnostic_sre, handle_rej_samples, run_pmcmc, run_pmcmc_analysis
 from .mbp_ibis import MbpParticles, run_mbp_ibis
 from .mbp_mcmc import generate_x0, run_mbp_mcmc, run_mcmc_analysis
+from .da_mcmc import run_std_mcmc
 from .sim import generate_observations, gillespie_sim, save_to_file
 from .arq import (ARQMCMCSample, ARQModel, GridPoint, GridRequest, LikelihoodModel, adapt_jw, get_grid_points, get_theta_f,
                   run_arq_mcmc_analysis)

@@ -124,6 +124,8 @@ _SIGS = {
     "dpomp_mbp_reserve": (C.c_int, [_P, C.c_int32]),
     "dpomp_mbp_get_states": (C.c_int, [_P, C.c_int32, _P]),
     "dpomp_mbp_get_particle": (C.c_int, [_P, C.c_int32, C.c_int32, _P, _P, _P, _P, C.c_int64, _P]),
+    "dpomp_da_loglike": (C.c_int, [_P, _P, C.c_int32, _P]),
+    "dpomp_da_step": (C.c_int, [_P, _P, _P, _P, C.c_int32, C.c_int32, C.c_int32, _P, _P]),
     "dpomp_comm_unique_id": (C.c_int, [_P, C.c_int32]),
     "dpomp_comm_create": (C.c_int, [_P, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.POINTER(_P)]),
     "dpomp_comm_destroy": (C.c_int, [_P]),

@@ -25,144 +25,9 @@
 #include "dpomp_internal.cuh"
 #include "dpomp_models.cuh"
 #include "obs_count.cuh"
+#include "mbp_walk.cuh"
 
 namespace dpomp {
-
-constexpr uint32_t kTagMbp = 2u;
-
-struct MbpModel {  // integer rate table + f64 observation constants, runtime C / E
-    int n_comp, n_events, n_params, t0_index;
-    int par[DPOMP_MAX_EVENTS];
-    int f1[DPOMP_MAX_EVENTS][DPOMP_MAX_COMPARTMENTS], k1[DPOMP_MAX_EVENTS];
-    int f2[DPOMP_MAX_EVENTS][DPOMP_MAX_COMPARTMENTS], k2[DPOMP_MAX_EVENTS];
-    int dn[DPOMP_MAX_EVENTS][DPOMP_MAX_COMPARTMENTS], kd[DPOMP_MAX_EVENTS], has_den[DPOMP_MAX_EVENTS];
-    int trans[DPOMP_MAX_EVENTS][DPOMP_MAX_COMPARTMENTS];
-    int xmask[DPOMP_MAX_COMPARTMENTS], ic[DPOMP_MAX_COMPARTMENTS];
-    double obs_tmp1, obs_tmp2;
-};
-
-struct MbpStore {
-    double* ev_time;      // [n][cap]
-    unsigned char* ev_type;  // [n][cap]
-    int* len;             // [n]
-    int* fc;              // [n][C]
-    double* ll;           // [n][2]
-};
-
-struct MbpStream {
-    uint32_t k, a, b, id, j;
-};
-__device__ __forceinline__ MbpStream mbp_stream_init(uint64_t key, uint32_t id, uint32_t obs, uint32_t which) {
-    const Philox4 p = stream_draw(key, 0u, id, obs, kTagMbp, which);
-    return MbpStream{p.w0, p.w1, p.w2, id, 0u};
-}
-__device__ __forceinline__ uint2 mbp_draw(MbpStream& s) {
-    const uint2 w = philox2x32_10(s.id ^ s.a, s.j ^ s.b, s.k);
-    s.j += 1;
-    return w;
-}
-
-// ---- rate policies ----------------------------------------------------------------------------------------------------
-// MbpRates<kModelGeneric>: the integer rate table with run-time C / E (any model the table compiler accepts).
-// MbpRates<ID>: a predefined model with compile-time structure -- loops unroll, states and rates stay in registers, and
-// rate[e] = (theta[e] * x_a) * x_b is the same f64 expression the table evaluates (l1 = x_a, l2 = x_b or 1 exactly), so both
-// give bit-identical walks; a walk is one dependent instruction chain, so its length is what the kernels' time is made of.
-template <int MODEL>
-struct MbpRates {
-    using BM = Builtin<MODEL>;
-    static constexpr int C = BM::C, E = BM::E, CMAX = BM::C, EMAX = BM::E, PMAX = BM::E;  // parameter e drives event e
-    static __device__ __forceinline__ void load_params(const MbpModel&, const double* src, double (&th)[PMAX]) {
-#pragma unroll
-        for (int i = 0; i < PMAX; ++i) th[i] = src[i];
-    }
-    static __device__ __forceinline__ void rates(const MbpModel&, const double (&th)[PMAX], const int (&x)[CMAX], double (&out)[EMAX]) {
-#pragma unroll
-        for (int e = 0; e < E; ++e) {
-            double r = __dmul_rn(th[e], (double)x[BM::A(e)]);
-            r = __dmul_rn(r, BM::B(e) >= 0 ? (double)x[BM::B(e) >= 0 ? BM::B(e) : 0] : 1.0);
-            out[e] = r;
-        }
-    }
-    static __device__ __forceinline__ void apply(const MbpModel&, int e, int (&x)[CMAX]) {
-#pragma unroll
-        for (int i = 0; i < E; ++i)
-#pragma unroll
-            for (int c = 0; c < C; ++c) x[c] += (e == i) ? BM::T(i, c) : 0;
-    }
-    static __device__ __forceinline__ double pick(const double (&v)[EMAX], int e) {
-        double r = v[0];
-#pragma unroll
-        for (int i = 1; i < E; ++i) r = (e == i) ? v[i] : r;
-        return r;
-    }
-};
-template <>
-struct MbpRates<kModelGeneric> {
-    static constexpr int C = 0, E = 0, CMAX = DPOMP_MAX_COMPARTMENTS, EMAX = DPOMP_MAX_EVENTS, PMAX = DPOMP_MAX_PARAMS;
-    static __device__ __forceinline__ void load_params(const MbpModel& m, const double* src, double (&th)[PMAX]) {
-        for (int i = 0; i < m.n_params; ++i) th[i] = src[i];
-    }
-    static __device__ __forceinline__ void rates(const MbpModel& m, const double (&th)[PMAX], const int (&x)[CMAX], double (&out)[EMAX]) {
-        for (int e = 0; e < m.n_events; ++e) {
-            long long l1 = m.k1[e], l2 = m.k2[e], dn = m.kd[e];
-            for (int c = 0; c < m.n_comp; ++c) {
-                l1 += (long long)m.f1[e][c] * x[c];
-                l2 += (long long)m.f2[e][c] * x[c];
-                dn += (long long)m.dn[e][c] * x[c];
-            }
-            const double p = m.par[e] >= 0 ? th[m.par[e]] : 1.0;
-            double r = __dmul_rn(__dmul_rn(p, (double)l1), (double)l2);
-            if (m.has_den[e]) r = (dn == 0) ? 0.0 : __ddiv_rn(r, (double)dn);
-            out[e] = r;
-        }
-    }
-    static __device__ __forceinline__ void apply(const MbpModel& m, int e, int (&x)[CMAX]) {
-        for (int c = 0; c < m.n_comp; ++c) x[c] += m.trans[e][c];
-    }
-    static __device__ __forceinline__ double pick(const double (&v)[EMAX], int e) { return v[e]; }
-};
-template <class R> __device__ __forceinline__ int mbp_nc(const MbpModel& m) { if constexpr (R::C > 0) return R::C; else return m.n_comp; }
-template <class R> __device__ __forceinline__ int mbp_ne(const MbpModel& m) { if constexpr (R::E > 0) return R::E; else return m.n_events; }
-
-template <class R>
-__device__ __forceinline__ void mbp_cumsum(const MbpModel& m, double (&v)[R::EMAX]) {
-    const int n = mbp_ne<R>(m);
-#pragma unroll
-    for (int i = 1; i < n; ++i) v[i] = __dadd_rn(v[i - 1], v[i]);
-}
-// choose_event (src/hmm_cmn.jl:4-10): first i < E - 1 with cum[i] > etc, else the last event (0-based)
-template <class R>
-__device__ __forceinline__ int mbp_choose(const MbpModel& m, const double (&cum)[R::EMAX], double u) {
-    const int n = mbp_ne<R>(m);
-    const double etc = __dmul_rn(u, R::pick(cum, n - 1));
-    int e = n - 1;
-#pragma unroll
-    for (int i = R::EMAX - 2; i >= 0; --i)
-        if (i < n - 1 && cum[i] > etc) e = i;
-    return e;
-}
-template <class R>
-__device__ __forceinline__ double mbp_obs_ll(const MbpModel& m, double ysum, const int (&x)[R::CMAX]) {
-    const int nc = mbp_nc<R>(m);
-    long long xs = 0;
-#pragma unroll
-    for (int c = 0; c < R::CMAX; ++c)
-        if (c < nc) xs += (long long)m.xmask[c] * x[c];
-    const double d = ysum - (double)xs;
-    return m.obs_tmp1 - __ddiv_rn(__dmul_rn(d, d), m.obs_tmp2);
-}
-// COUNT: the model's count observation family (obs_count.cuh) with its theta-indexed parameters taken from th (the walk's theta)
-template <class R, bool COUNT>
-__device__ __forceinline__ double mbp_obs_ll(const MbpModel& m, const CountObs& co, const double* th, int t, double ysum,
-                                             const int (&x)[R::CMAX]) {
-    if constexpr (!COUNT) {
-        return mbp_obs_ll<R>(m, ysum, x);
-    } else {
-        long long xs = 0;
-        for (int c = 0; c < m.n_comp; ++c) xs += (long long)m.xmask[c] * x[c];
-        return count_obs_logpmf(count_obs_const(co, th, t, ysum), ysum, (double)xs);
-    }
-}
 
 // ---- event-list access policies -------------------------------------------------------------------------------------
 // The walks below are written once against an IO policy, so the thread-per-trajectory and the warp-per-trajectory kernels
@@ -824,32 +689,6 @@ struct MbpOuter {
     uint64_t sweep = 0;
 };
 
-struct dpomp_mbp {
-    MbpOuter* outer = nullptr;
-    const dpomp_model* model = nullptr;
-    int device = 0, n = 0;
-    int cap = 0;       // current stride of the stores (events reserved per trajectory); grows on demand up to cap_max
-    int cap_max = 0;   // MAX_TRAJ (src/DiscretePOMP.jl:40): the reference's hard limit, beyond which log-likelihood = -Inf
-    int call_id = 0;   // id of the current iterate / propose call (MbpGrow)
-    int* done = nullptr;       // [n]
-    int* need_grow = nullptr;  // [1] device
-    int* h_need_grow = nullptr;  // pinned
-    cudaStream_t stream = nullptr;
-    MbpModel dm{};
-    MbpStore store[3]{};   // [cur], [cur ^ 1] (resample workspace), [2] proposal
-    int cur = 0;
-    int mode = 0;          // 0 automatic, 1 one thread per trajectory, 2 one warp per trajectory
-    int model_id = 0;      // predefined model with compile-time structure (dpomp_models.cuh), 0 = generic rate table
-    uint64_t seed = 0, call_index = 0, forced_key = 0;
-    bool key_forced = false;
-    long long batch_offset = 0;
-    double *theta_i = nullptr, *theta_f = nullptr, *out = nullptr, *obs_time = nullptr, *obs_ysum = nullptr;
-    int* obs_haslik = nullptr;
-    double *obs_lgy = nullptr, *obs_lgk = nullptr;  // count observation constants [T] (count families only)
-    CountObs cobs{};                                // family != DPOMP_OBS_GAUSSIAN: the count kernels run
-    unsigned char* valid = nullptr;
-    int64_t* slots = nullptr;  // 2 * n
-};
 
 static uint64_t mbp_splitmix64(uint64_t x) {
     x += 0x9E3779B97F4A7C15ull;
@@ -857,7 +696,7 @@ static uint64_t mbp_splitmix64(uint64_t x) {
     x = (x ^ (x >> 27)) * 0x94D049BB133111EBull;
     return x ^ (x >> 31);
 }
-static uint64_t mbp_next_key(dpomp_mbp* h) {
+uint64_t mbp_next_key(dpomp_mbp* h) {
     const uint64_t k = h->key_forced ? h->forced_key : mbp_splitmix64(h->seed ^ mbp_splitmix64(0x4D4250ull + h->call_index));
     h->key_forced = false;
     h->call_index += 1;
@@ -886,14 +725,14 @@ static void mbp_free(dpomp_mbp* h) {
         cudaFree(h->store[s].fc); cudaFree(h->store[s].ll);
     }
     cudaFree(h->theta_i); cudaFree(h->theta_f); cudaFree(h->out); cudaFree(h->obs_time); cudaFree(h->obs_ysum);
-    cudaFree(h->obs_haslik); cudaFree(h->obs_lgy); cudaFree(h->obs_lgk); cudaFree(h->valid); cudaFree(h->slots); cudaFree(h->done); cudaFree(h->need_grow);
+    cudaFree(h->obs_haslik); cudaFree(h->obs_lgy); cudaFree(h->obs_lgk); cudaFree(h->valid); cudaFree(h->slots); cudaFree(h->done); cudaFree(h->need_grow); cudaFree(h->da_work);
     cudaFreeHost(h->h_need_grow);
     if (h->stream) cudaStreamDestroy(h->stream);
     delete h;
 }
 
 // widen the stride of all three stores to new_cap (<= cap_max); the live prefixes are copied on the store's stream
-static int mbp_grow(dpomp_mbp* h, int new_cap) {
+int mbp_grow(dpomp_mbp* h, int new_cap) {
     if (new_cap > h->cap_max) new_cap = h->cap_max;
     if (new_cap <= h->cap) return DPOMP_OK;
     const size_t N = (size_t)h->n;

@@ -13,6 +13,8 @@
 #     run_pibis               src/hmm_ibis.jl:12-135     (its three partial_log_likelihood! call sites, batched)
 #     run_mbp_ibis            src/hmm_ibis.jl:140-244    (iterate_particle!, deepcopy, partial_model_based_proposal loops)
 #     rs_systematic           src/hmm_resample.jl:44-62
+#     run_std_mcmc            src/hmm_mcmc.jl            (run_mcmc_analysis(...; mbp = false) dispatches to it: the data-augmented
+#                                                        sampler runs on the device)
 # plus DpompComm for sharding theta-particles over several GPUs (one Julia process per GPU).
 
 import LinearAlgebra
@@ -767,5 +769,75 @@ function run_mbp_ibis(model::HiddenMarkovModel, theta::Array{Float64, 2}, ess_rs
     compute_is_mu_covar!(mu, cv, theta, w)
     output = ImportanceSample(mu, cv, theta, w, time_ns() - start_time, -bme)
     comm.rank == 0 && println("- finished in ", print_runtime(output.run_time), " (AR := ", round(100.0 * k_log[2] / k_log[1]; sigdigits = 3), "%)")
+    return output
+end
+
+# --------------------------------------------------------------------------------------------------------------------
+# run_std_mcmc (src/hmm_mcmc.jl; gibbs_mh_alg! :138, compute_full_log_like! :78, the proposals of src/hmm_std.jl): the
+# data-augmented sampler of run_mcmc_analysis(...; mbp = false).  All chains in lock step on one dpomp_mbp store, one
+# dpomp_da_step per MCMC step: chains drawing a theta proposal (probability ppp) are evaluated under theta_f and decided here,
+# the others run traj_props insert / delete / move proposals that are drawn, decided and applied on the device.
+# --------------------------------------------------------------------------------------------------------------------
+function da_loglike(s::DpompMBP, theta::Array{Float64,2})
+    out = Array{Float64,2}(undef, 2, size(theta, 2))                                        # column p = {full, observation}
+    GC.@preserve theta out dpomp_check(ccall((:dpomp_da_loglike, LIBDPOMP), Cint,
+        (Ptr{Cvoid}, Ptr{Float64}, Int32, Ptr{Float64}), s.handle, theta, size(theta, 2), out))
+    return out
+end
+function da_step!(s::DpompMBP, theta::Array{Float64,2}, theta_f::Array{Float64,2}, kind::Vector{UInt8}, traj_props::Int, mvp::Int)
+    out = Array{Float64,2}(undef, 2, size(theta, 2))
+    acc = Array{Int32,2}(undef, 3, size(theta, 2))                                           # accepted inserts, deletes, moves
+    GC.@preserve theta theta_f kind out acc dpomp_check(ccall((:dpomp_da_step, LIBDPOMP), Cint,
+        (Ptr{Cvoid}, Ptr{Float64}, Ptr{Float64}, Ptr{UInt8}, Int32, Int32, Int32, Ptr{Float64}, Ptr{Int32}),
+        s.handle, theta, theta_f, kind, size(theta, 2), traj_props, mvp, out, acc))
+    return out, acc
+end
+
+function run_std_mcmc(model::HiddenMarkovModel, theta_init::Array{Float64, 2}, steps::Int64, adapt_period::Int64, fin_adapt::Bool,
+                      ppp::Float64, mvp::Int64; traj_props::Int64 = 1)
+    start_time = time_ns()
+    d, n_chains = size(theta_init)
+    println("Running: ", n_chains, "-chain ", steps, "-sample data-augmented MCMC analysis (model: ", model.model_name, ")")
+    store = DpompMBP(dpomp_model(model), n_chains)
+    theta = copy(theta_init)
+    for obs_i in eachindex(model.obs_data)                                                   # generate_x0 (src/hmm_sim.jl:160-168)
+        mbp_iterate!(store, theta, obs_i, obs_i == 1)
+    end
+    log_like = da_loglike(store, theta)[1, :]
+    prior = [Distributions.logpdf(model.prior, theta[:, k]) for k in 1:n_chains]
+    samples = zeros(d, steps, n_chains)
+    samples[:, 1, :] .= theta
+    propd = [Distributions.MvNormal(LinearAlgebra.Diagonal([theta[i, k] == 0.0 ? 1.0 : theta[i, k]^2 for i in 1:d])) for k in 1:n_chains]
+    c = fill(C_INITIAL, n_chains)
+    adapt_interval = adapt_period / C_MCMC_ADAPT_INTERVALS
+    for i in 2:steps
+        on_theta = rand(n_chains) .< ppp
+        theta_f = hcat([get_mv_param(propd[k], c[k], theta[:, k]) for k in 1:n_chains]...)
+        prior_f = [Distributions.logpdf(model.prior, theta_f[:, k]) for k in 1:n_chains]
+        kind = UInt8[on_theta[k] ? (prior_f[k] == -Inf ? 2 : 0) : 1 for k in 1:n_chains]
+        ll, _ = da_step!(store, theta, theta_f, kind, traj_props, mvp)
+        for k in 1:n_chains
+            if kind[k] == 1
+                log_like[k] = ll[1, k]
+            elseif on_theta[k]
+                accepted = kind[k] == 0 && exp(prior_f[k] - prior[k]) * exp(ll[1, k] - log_like[k]) > rand()
+                if accepted
+                    theta[:, k] = theta_f[:, k]; prior[k] = prior_f[k]; log_like[k] = ll[1, k]
+                end
+                if !fin_adapt || i < adapt_period
+                    c[k] *= accepted ? 1.002 : 0.999
+                end
+            end
+        end
+        samples[:, i, :] .= theta
+        if (!fin_adapt || i < adapt_period) && i % adapt_interval == 0
+            for k in 1:n_chains
+                propd[k] = get_prop_density(Statistics.cov(transpose(samples[:, 1:i, k])), propd[k])
+            end
+        end
+    end
+    rejs = handle_rej_samples(samples, adapt_period)
+    output = MCMCSample(rejs, adapt_period, gelman_diagnostic(samples, adapt_period).psrf, time_ns() - start_time)
+    println("- finished in ", print_runtime(output.run_time), ". E(x) := ", output.samples.mu)
     return output
 end

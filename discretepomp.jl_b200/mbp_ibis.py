@@ -93,6 +93,24 @@ class MbpParticles:
                                                   _capi.ptr(out)))
         return out
 
+    def da_loglike(self, theta) -> np.ndarray:
+        """dpomp_da_loglike: full log-likelihood {full, observation} (n, 2) of trajectories 1..n under theta (n_theta, n)."""
+        th = self._cols(theta)
+        out = np.empty((th.shape[0], 2))
+        _capi.check(_capi.lib().dpomp_da_loglike(self._h, _capi.ptr(th), th.shape[0], _capi.ptr(out)))
+        return out
+
+    def da_step(self, theta_cur, theta_f, kind, traj_props: int, mvp: int):
+        """dpomp_da_step: one data-augmented Gibbs step of chains 1..n (kind 0 theta, 1 trajectory, 2 nothing).  Returns
+        ({full, observation} log-likelihoods (n, 2), accepted inserts / deletes / moves (n, 3))."""
+        tc, tf = self._cols(theta_cur), self._cols(theta_f)
+        k = np.ascontiguousarray(kind, dtype=np.uint8)
+        out = np.empty((tc.shape[0], 2))
+        acc = np.empty((tc.shape[0], 3), dtype=np.int32)
+        _capi.check(_capi.lib().dpomp_da_step(self._h, _capi.ptr(tc), _capi.ptr(tf), _capi.ptr(k), tc.shape[0], int(traj_props),
+                                              int(mvp), _capi.ptr(out), _capi.ptr(acc)))
+        return out, acc.astype(np.int64)
+
     def accept(self, slots) -> None:
         s = _capi.as_i64(slots)
         if len(s):

@@ -37,7 +37,9 @@ def generate_x0(model: HiddenMarkovModel, ptcls: MbpParticles, theta: np.ndarray
     `theta` is (n_theta, n)."""
     n = theta.shape[1]
     ll = np.full(n, -np.inf)
-    for _ in range(ntries):
+    for attempt in range(ntries):
+        if attempt and hasattr(ptcls, "reset"):  # the device store keeps its events across calls: retries start afresh
+            ptcls.reset()
         ll = np.zeros(n)
         for obs_i in range(1, len(model.obs_data) + 1):
             ptcls.set_stream_key(next_key())
@@ -50,6 +52,56 @@ def generate_x0(model: HiddenMarkovModel, ptcls: MbpParticles, theta: np.ndarray
             return ll
     print("WARNING: having an issue generating a valid trajectory")
     return ll
+
+
+class AdaptiveRandomWalk:
+    """The adaptive random walk on theta of the reference's MCMC samplers, for every chain of this rank: @initialise_mcmc
+    (src/hmm_mcmc.jl:10-25), get_mv_param (src/hmm_cmn.jl:13-18), @met_hastings_adapt (:44-52) and @mcmc_adapt_period
+    (:28-41).  theta is (n_theta, n_chains)."""
+
+    def __init__(self, theta: np.ndarray, adapt_period: int):
+        d, n = theta.shape
+        # @initialise_mcmc: covar[i,i] = theta[i] == 0 ? 1 : theta[i]^2; propd = MvNormal(covar); c = C_INITIAL
+        self.chol = np.zeros((n, d, d))  # Cholesky factor of every chain's proposal covariance
+        self.chol[:, np.arange(d), np.arange(d)] = np.where(theta.T == 0.0, 1.0, np.abs(theta.T))
+        self.c = np.full(n, C_INITIAL)
+        self.sum_x = theta.T.copy()                                   # running sums of the samples of every chain: the
+        self.sum_xx = np.einsum("ki,kj->kij", theta.T, theta.T)       # covariance of @mcmc_adapt_period without a pass over them
+        self.adapt_interval = adapt_period / C_MCMC_ADAPT_INTERVALS  # Float64, like the reference
+
+    def propose(self, theta: np.ndarray, z: np.ndarray) -> np.ndarray:
+        """theta + c L z for standard normal z (n_chains, n_theta)"""
+        return theta + (self.c[:, None] * np.einsum("kij,kj->ki", self.chol, z)).T
+
+    def record(self, theta: np.ndarray) -> None:
+        """the samples of the current step enter the running sums"""
+        self.sum_x += theta.T
+        self.sum_xx += np.einsum("ki,kj->kij", theta.T, theta.T)
+
+    def scale(self, accepted: np.ndarray, on: Optional[np.ndarray] = None) -> None:
+        """c *= 1.002 after an accepted, 0.999 after a rejected proposal; `on` restricts the update to those chains"""
+        f = np.where(accepted, 1.002, 0.999)
+        if on is None:
+            self.c *= f
+        else:
+            self.c[on] *= f[on]
+
+    def adapt_period(self, i: int) -> None:
+        """@mcmc_adapt_period at step i (1-based): every adapt_period / 10 steps the proposal covariance becomes that of the
+        samples 1..i"""
+        if self.adapt_interval > 0 and math.fmod(i, self.adapt_interval) == 0:
+            # covar = cov(transpose(theta[:, 1:i, mc])); propd = get_prop_density(covar, propd): kept when the
+            # covariance is not positive definite (src/hmm_cmn.jl:33-42)
+            mean = self.sum_x / i
+            covar = (self.sum_xx - i * np.einsum("ki,kj->kij", mean, mean)) / (i - 1)
+            sym = np.triu(covar) + np.transpose(np.triu(covar, 1), (0, 2, 1))  # Hermitian(): the upper triangle
+            ok = np.linalg.eigvalsh(sym).min(axis=1) > 0
+            if ok.any():
+                try:
+                    self.chol[ok] = np.linalg.cholesky(sym[ok])
+                except np.linalg.LinAlgError:  # borderline matrices: decide chain by chain
+                    for k in np.nonzero(ok)[0]:
+                        self.chol[k] = get_prop_density(sym[k], ProposalDensity(self.chol[k])).chol
 
 
 def run_mbp_mcmc(model: HiddenMarkovModel, theta_init: np.ndarray, steps: int, adapt_period: int, fin_adapt: bool = False,
@@ -82,15 +134,9 @@ def run_mbp_mcmc(model: HiddenMarkovModel, theta_init: np.ndarray, steps: int, a
     if n_loc:
         log_like = generate_x0(model, ptcls, theta, next_key)  # x0.log_like[1]
         prior = prior_logpdf_columns(model.prior, theta)       # x0.prior
-        # @initialise_mcmc: covar[i,i] = theta[i] == 0 ? 1 : theta[i]^2; propd = MvNormal(covar); c = C_INITIAL
-        chol = np.zeros((n_loc, d, d))  # Cholesky factor of every chain's proposal covariance
-        chol[:, np.arange(d), np.arange(d)] = np.where(theta.T == 0.0, 1.0, np.abs(theta.T))
-        c = np.full(n_loc, C_INITIAL)
+        rw = AdaptiveRandomWalk(theta, adapt_period)
         chains[:, 0, :] = theta.T
         a_cnt[:, 0] = 1
-        sum_x = theta.T.copy()                                   # running sums of the samples of every chain: the
-        sum_xx = np.einsum("ki,kj->kij", theta.T, theta.T)       # covariance of @mcmc_adapt_period without a pass over them
-        adapt_interval = adapt_period / C_MCMC_ADAPT_INTERVALS  # Float64, like the reference
         n_obs = len(model.obs_data)
         for i in range(2, steps + 1):  # Julia's 1-based step index
             # host draws of step i for ALL chains from one stream keyed by (seed, i); a rank uses the rows of its chains, so
@@ -98,7 +144,7 @@ def run_mbp_mcmc(model: HiddenMarkovModel, theta_init: np.ndarray, steps: int, a
             g = np.random.default_rng([seed & 0xFFFFFFFF, 0x4D43, i])
             z = g.standard_normal((n_chains, d))[lo:hi]
             u = g.random(n_chains)[lo:hi]
-            theta_f = theta + (c[:, None] * np.einsum("kij,kj->ki", chol, z)).T  # get_mv_param(propd, c, theta[:, i-1, mc]) (:126)
+            theta_f = rw.propose(theta, z)  # get_mv_param(propd, c, theta[:, i-1, mc]) (:126)
             prior_f = prior_logpdf_columns(model.prior, theta_f)
             valid = prior_f != -np.inf
             ptcls.set_stream_key(next_key())
@@ -112,23 +158,10 @@ def run_mbp_mcmc(model: HiddenMarkovModel, theta_init: np.ndarray, steps: int, a
             log_like[accepted] = ll_f[accepted]
             a_cnt[accepted, 1 if i > adapt_period else 0] += 1
             chains[:, i - 1, :] = theta.T
-            sum_x += theta.T
-            sum_xx += np.einsum("ki,kj->kij", theta.T, theta.T)
+            rw.record(theta)
             if (not fin_adapt) or i < adapt_period:  # @met_hastings_adapt
-                c *= np.where(accepted, 1.002, 0.999)
-                if adapt_interval > 0 and math.fmod(i, adapt_interval) == 0:  # @mcmc_adapt_period
-                    # covar = cov(transpose(theta[:, 1:i, mc])); propd = get_prop_density(covar, propd): kept when the
-                    # covariance is not positive definite (src/hmm_cmn.jl:33-42)
-                    mean = sum_x / i
-                    covar = (sum_xx - i * np.einsum("ki,kj->kij", mean, mean)) / (i - 1)
-                    sym = np.triu(covar) + np.transpose(np.triu(covar, 1), (0, 2, 1))  # Hermitian(): the upper triangle
-                    ok = np.linalg.eigvalsh(sym).min(axis=1) > 0
-                    if ok.any():
-                        try:
-                            chol[ok] = np.linalg.cholesky(sym[ok])
-                        except np.linalg.LinAlgError:  # borderline matrices: decide chain by chain
-                            for k in np.nonzero(ok)[0]:
-                                chol[k] = get_prop_density(sym[k], ProposalDensity(chol[k])).chol
+                rw.scale(accepted)
+                rw.adapt_period(i)
     flat = comm.allgather_f64(chains.reshape(n_loc, steps * d), n_chains)
     samples = np.ascontiguousarray(flat.reshape(n_chains, steps, d).transpose(2, 1, 0))
     rejs = handle_rej_samples(samples, adapt_period)
@@ -149,7 +182,8 @@ def run_mcmc_analysis(model: DPOMPModel, obs_data, n_chains: int = 3, initial_pa
     adapt_period, fin_adapt = false, mbp = true, ppp, mvp) (src/DiscretePOMP.jl:185-193).  Only the MBP-MCMC default is on
     the accelerated path; `mbp = false` (the standard data-augmented Gibbs sampler, run_std_mcmc) is out of scope."""
     if not mbp:
-        raise NotImplementedError("run_std_mcmc (mbp = false) is outside the accelerated path; use mbp = True")
+        raise NotImplementedError("run_mcmc_analysis(mbp = false) is not provided; call run_std_mcmc for the data-augmented "
+                                  "sampler, or use mbp = True")
     mdl = get_private_model(model, obs_data)
     if adapt_period is None:
         adapt_period = int(math.floor(steps * C_DF_MCMC_ADAPT))

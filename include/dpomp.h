@@ -311,6 +311,36 @@ int dpomp_mbp_get_particle(dpomp_mbp* mbp, int32_t p, int32_t which, int64_t* fc
                            int32_t* types, int64_t cap_out, double* loglike2);
 
 /*
+ * Data-augmented MCMC (run_std_mcmc, src/hmm_mcmc.jl; the sampler of run_mcmc_analysis(...; mbp = false)) over the
+ * trajectory store of an MBP handle: chain p is trajectory p, theta is n_params x n column-major.
+ *
+ * Full log-likelihood (compute_full_log_like!, src/hmm_mcmc.jl:78), f64.  From t = t0 (0 or theta[t0_index]) and the initial
+ * condition, events and observations are walked in time order (an event at an observation time belongs to the interval that
+ * ends there): an event (t_k, e_k) adds log rate[e_k] - (sum of rates) (t_k - t), then its transition applies; an observation
+ * subtracts (sum of rates) (t_obs - t) and, if obs_id > 0, adds log g(y | x, theta).  -Inf for a zero-rate event, a negative
+ * compartment, an event at or before t0, or an event after the last observation.  out_ll2[p] = {full, observation part}.
+ */
+int dpomp_da_loglike(dpomp_mbp* mbp, const double* theta, int32_t n, double* out_ll2);  /* writes nothing to the store */
+/*
+ * One Gibbs step (gibbs_mh_alg!, src/hmm_mcmc.jl:138) for chains 1..n in one launch; kind[p] selects what chain p does:
+ *   0  evaluates its trajectory under theta_f (a theta proposal; the host takes the decision): out_ll2[p], store unchanged
+ *   1  runs traj_props proposals (src/hmm_std.jl) one after another under theta_cur: kind k uniform on 1..mvp,
+ *        1 insert  a type uniform on 1..E at a time uniform on (t0, T]     ratio E (T - t0) / (n + 1)
+ *        2 delete  an event uniform on 1..n                                ratio n / (E (T - t0))
+ *       >2 move    an event uniform on 1..n to a time uniform on (t0, T]   ratio 1
+ *      accepted with probability min(1, ratio exp(l_f - l)); a delete or move of an empty trajectory and an insert into a
+ *      trajectory of max_traj events are rejected.  l is the full log-likelihood of the current trajectory under theta_cur.
+ *      Accepted edits are written to the store (events, length, final state, log_like = out_ll2[p] under theta_cur);
+ *      out_acc[p][3] = accepted inserts, deletes, moves
+ *   2  nothing (a theta proposal outside the prior): out_ll2[p] = -Inf
+ * T is the last observation time.  The stride grows before the launch to hold traj_props more events than the longest
+ * trajectory.  Draws are Philox streams keyed by the call key and the GLOBAL chain id (dpomp_mbp_set_batch_offset), so results
+ * do not depend on the number of ranks; the mapping of the words is documented in da.cu.
+ */
+int dpomp_da_step(dpomp_mbp* mbp, const double* theta_cur, const double* theta_f, const uint8_t* kind, int32_t n,
+                  int32_t traj_props, int32_t mvp, double* out_ll2, int32_t* out_acc);
+
+/*
  * Bit-exactness hook for the resampling searches (host buffers).
  *   on_cumulative = 1: `w` is already cumulative  -> rsp_* semantics (src/hmm_pf_resample.jl:24-42, and the
  *                      intended semantics of the broken rsp_stratified/rsp_multinomial :46-63, :5-20)
