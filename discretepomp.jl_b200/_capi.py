@@ -71,6 +71,7 @@ _SIGS = {
     "dpomp_model_create": (C.c_int, [C.POINTER(ModelDesc), C.POINTER(_P)]),
     "dpomp_model_destroy": (C.c_int, [_P]),
     "dpomp_model_set_obs_model": (C.c_int, [_P, C.c_int32, _P, _P]),
+    "dpomp_model_builtin_id": (C.c_int, [_P, C.POINTER(C.c_int32)]),
     "dpomp_pf_create": (C.c_int, [_P, C.c_int64, C.c_int32, C.c_int32, C.c_uint64, C.c_int32, C.POINTER(_P)]),
     "dpomp_pf_destroy": (C.c_int, [_P]),
     "dpomp_pf_set_sim_precision": (C.c_int, [_P, C.c_int32]),

@@ -40,7 +40,7 @@ static uint64_t call_key(const dpomp_pf* pf) {
 extern "C" {
 
 const char* dpomp_last_error(void) { return g_err.c_str(); }
-int dpomp_version(void) { return 101; }
+int dpomp_version(void) { return 102; }
 
 int dpomp_device_count(int* out_count) {
     if (!out_count) return fail(DPOMP_ERR_ARG, "out_count is null");
@@ -136,6 +136,13 @@ int dpomp_model_set_obs_model(dpomp_model* model, int32_t family, const int32_t*
     } else {
         count_obs_constants(h);
     }
+    return DPOMP_OK;
+}
+
+int dpomp_model_builtin_id(const dpomp_model* model, int32_t* out_id) {
+    if (!model || !out_id) return fail(DPOMP_ERR_ARG, "null argument");
+    // the count families run the generic rate-table kernels (pf_sim.cuh sim_count_typed, mbp.cu dpomp_mbp_create)
+    *out_id = model->h.obs_family != DPOMP_OBS_GAUSSIAN ? 0 : builtin_model_id(model->h.desc);
     return DPOMP_OK;
 }
 

@@ -137,6 +137,15 @@ int dpomp_model_set_obs_model(dpomp_model* model, int32_t family, const int32_t*
                               const double* par_value /*[2]*/);
 
 /*
+ * Which kernels the model runs on (read-only, no device needed).  *out_id = 1..7 (SI, SIR, SIS, SEI, SEIR, SEIS, LOTKA) when
+ * the rate table is exactly that predefined density-dependent model -- same compartments, events, parameter order, factors
+ * and transition rows -- and the filter, the MBP walks and the DA walks use its compile-time instantiations; 0 for every other
+ * table, which runs the generic rate-table kernels on the smallest instantiated (compartments, events) shape covering it.
+ * A count observation family (dpomp_model_set_obs_model) always gives 0: those kernels evaluate the generic table.
+ */
+int dpomp_model_builtin_id(const dpomp_model* model, int32_t* out_id);
+
+/*
  * A batch of n_batch independent bootstrap filters of n_particles each on one device
  * (the `pop::Array{Int64,2}` workspaces of estimate_likelihood src/hmm_particle_filter.jl:79-84 and of
  * run_pibis src/hmm_ibis.jl:26-35, resident in HBM as int32 SoA [batch][compartment][particle]).

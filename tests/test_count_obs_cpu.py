@@ -140,7 +140,7 @@ def _desc(dp, om=None):
 
 
 def test_set_obs_model_validates_its_arguments(built_lib, dp):
-    assert built_lib.dpomp_version() == 101
+    assert built_lib.dpomp_version() == 102
     cm = _desc(dp)
     h = C.c_void_p()
     assert built_lib.dpomp_model_create(C.byref(cm.desc), C.byref(h)) == 0
