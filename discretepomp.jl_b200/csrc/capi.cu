@@ -141,8 +141,9 @@ int dpomp_model_set_obs_model(dpomp_model* model, int32_t family, const int32_t*
 
 int dpomp_model_builtin_id(const dpomp_model* model, int32_t* out_id) {
     if (!model || !out_id) return fail(DPOMP_ERR_ARG, "null argument");
-    // the count families run the generic rate-table kernels (pf_sim.cuh sim_count_typed, mbp.cu dpomp_mbp_create)
-    *out_id = model->h.obs_family != DPOMP_OBS_GAUSSIAN ? 0 : builtin_model_id(model->h.desc);
+    // the kernels of a count family run the generic rate table, reported as 0
+    const int id = kernel_model_id(model->h);
+    *out_id = id == kModelCountObs ? kModelGeneric : id;
     return DPOMP_OK;
 }
 

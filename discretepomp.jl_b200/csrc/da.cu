@@ -32,11 +32,12 @@ __device__ __forceinline__ int da_uniform_int(uint32_t w, int n) { return (int)(
 // merged after the events at times <= tins (eins < 0: none).  Returns the full log-likelihood; llo = its observation part,
 // x = the final state, q = position of the inserted event in the edited list.  -Inf (both parts): a zero rate for an event,
 // a negative compartment, an event at or before t0, or an event after the last observation.
-template <class R, bool COUNT>
-__device__ __forceinline__ double da_walk(const MbpModel& m, const CountObs& co, const double (&th)[R::PMAX], double t0,
+template <int MODEL>
+__device__ __forceinline__ double da_walk(const MbpModel& m, const CountObs& co, const double (&th)[MbpRates<MODEL>::PMAX], double t0,
                                           const double* et, const unsigned char* ey, int n, int del, double tins, int eins,
                                           const double* obs_time, const double* obs_ysum, const int* obs_haslik, int n_obs,
-                                          int (&x)[R::CMAX], double& llo, int& q) {
+                                          int (&x)[MbpRates<MODEL>::CMAX], double& llo, int& q) {
+    using R = MbpRates<MODEL>;
     const int nc = mbp_nc<R>(m), ne = mbp_ne<R>(m);
 #pragma unroll
     for (int c = 0; c < R::CMAX; ++c) x[c] = (c < nc) ? m.ic[c] : 0;
@@ -80,7 +81,7 @@ __device__ __forceinline__ double da_walk(const MbpModel& m, const CountObs& co,
         ll = __dsub_rn(ll, __dmul_rn(R::pick(lam, ne - 1), __dsub_rn(t_obs, t)));
         t = t_obs;
         if (obs_haslik[oi]) {
-            const double g = mbp_obs_ll<R, COUNT>(m, co, th, oi, obs_ysum[oi], x);
+            const double g = mbp_obs_ll<MODEL>(m, co, th, oi, obs_ysum[oi], x);
             ll = __dadd_rn(ll, g);
             llo = __dadd_rn(llo, g);
         }
@@ -92,7 +93,7 @@ __device__ __forceinline__ double da_walk(const MbpModel& m, const CountObs& co,
 
 // kind == nullptr (dpomp_da_loglike): every chain evaluates its trajectory under theta_f.  Otherwise per chain: 0 evaluates under
 // theta_f, 1 runs traj_props proposals under theta_cur and commits the accepted ones, 2 does nothing.
-template <int MODEL, bool COUNT>
+template <int MODEL>
 __global__ void __launch_bounds__(128) da_step_kernel(const __grid_constant__ MbpModel m, MbpStore st, const double* theta_cur,
                                                        const double* theta_f, const unsigned char* kind, int n, int cap, int cap_max,
                                                        int traj_props, int mvp, const double* obs_time, const double* obs_ysum,
@@ -116,7 +117,7 @@ __global__ void __launch_bounds__(128) da_step_kernel(const __grid_constant__ Mb
     const double t0 = m.t0_index > 0 ? thp[m.t0_index - 1] : 0.0;
     int x[R::CMAX], q;
     double llo;
-    double ll = da_walk<R, COUNT>(m, co, th, t0, et, ey, len, -1, 0.0, -1, obs_time, obs_ysum, obs_haslik, n_obs, x, llo, q);
+    double ll = da_walk<MODEL>(m, co, th, t0, et, ey, len, -1, 0.0, -1, obs_time, obs_ysum, obs_haslik, n_obs, x, llo, q);
     if (kd == 1) {
         const int ne = mbp_ne<R>(m), nc = mbp_nc<R>(m);
         const double span = __dsub_rn(obs_time[n_obs - 1], t0);
@@ -144,8 +145,8 @@ __global__ void __launch_bounds__(128) da_step_kernel(const __grid_constant__ Mb
             }
             int xf[R::CMAX], qf;
             double llof;
-            const double llf = da_walk<R, COUNT>(m, co, th, t0, et, ey, len, del, tnew, eins, obs_time, obs_ysum, obs_haslik, n_obs, xf,
-                                                 llof, qf);
+            const double llf = da_walk<MODEL>(m, co, th, t0, et, ey, len, del, tnew, eins, obs_time, obs_ysum, obs_haslik, n_obs, xf,
+                                              llof, qf);
             const Philox4 a = stream_draw(key, gid, (uint32_t)j, 0u, kTagDa, kDaBlockAccept);
             if (!(__dmul_rn(r, exp(__dsub_rn(llf, ll))) > u53(a.w0, a.w1))) continue;  // NaN compares false
             // apply the edit in place: one slot shift of the range between the removed and the inserted position
@@ -188,14 +189,6 @@ __global__ void da_max_len_kernel(const int* len, int n, int* out) {
 
 using namespace dpomp;
 
-#define DCK(expr)                                                                                         \
-    do {                                                                                                  \
-        cudaError_t _e = (expr);                                                                          \
-        if (_e != cudaSuccess) return dpomp_set_error(DPOMP_ERR_CUDA, std::string(#expr) + ": " + cudaGetErrorString(_e)); \
-    } while (0)
-
-#define DPOMP_DA_MODELS(X) X(kModelGeneric) X(kModelSI) X(kModelSIR) X(kModelSIS) X(kModelSEI) X(kModelSEIR) X(kModelSEIS) X(kModelLOTKA)
-
 // one launch over chains 1..n; theta_cur / theta_f / kind already on the device (h->theta_i, h->theta_f, h->valid)
 static int da_launch(dpomp_mbp* h, const unsigned char* kind_dev, int n, int traj_props, int mvp, double* out_ll_host,
                      int32_t* out_acc_host) {
@@ -203,24 +196,15 @@ static int da_launch(dpomp_mbp* h, const unsigned char* kind_dev, int n, int tra
     const uint64_t key = mbp_next_key(h);
     int* acc = kind_dev ? h->da_work : nullptr;
     const unsigned grid = (unsigned)((n + 127) / 128);
-#define DPOMP_DA_LAUNCH(ID)                                                                                                   \
-    if (h->model_id == ID)                                                                                                    \
-        da_step_kernel<ID, false><<<grid, 128, 0, h->stream>>>(h->dm, h->store[h->cur], h->theta_i, h->theta_f, kind_dev, n, h->cap, \
-                                                               h->cap_max, traj_props, mvp, h->obs_time, h->obs_ysum, h->obs_haslik,  \
-                                                               d.n_obs, key, (uint32_t)h->batch_offset, h->out, acc, h->cobs);
-    if (h->cobs.family != DPOMP_OBS_GAUSSIAN) {
-        da_step_kernel<kModelGeneric, true><<<grid, 128, 0, h->stream>>>(h->dm, h->store[h->cur], h->theta_i, h->theta_f, kind_dev, n,
-                                                                         h->cap, h->cap_max, traj_props, mvp, h->obs_time, h->obs_ysum,
-                                                                         h->obs_haslik, d.n_obs, key, (uint32_t)h->batch_offset, h->out,
-                                                                         acc, h->cobs);
-    } else {
-        DPOMP_DA_MODELS(DPOMP_DA_LAUNCH)
-    }
-#undef DPOMP_DA_LAUNCH
-    DCK(cudaGetLastError());
-    DCK(cudaMemcpyAsync(out_ll_host, h->out, (size_t)n * 2 * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
-    if (out_acc_host) DCK(cudaMemcpyAsync(out_acc_host, acc, (size_t)n * 3 * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
-    DCK(cudaStreamSynchronize(h->stream));
+    with_walk_model(h->model_id, [&](auto model) {
+        da_step_kernel<decltype(model)::value><<<grid, 128, 0, h->stream>>>(
+            h->dm, h->store[h->cur], h->theta_i, h->theta_f, kind_dev, n, h->cap, h->cap_max, traj_props, mvp, h->obs_time, h->obs_ysum,
+            h->obs_haslik, d.n_obs, key, (uint32_t)h->batch_offset, h->out, acc, h->cobs);
+    });
+    MCK(cudaGetLastError());
+    MCK(cudaMemcpyAsync(out_ll_host, h->out, (size_t)n * 2 * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+    if (out_acc_host) MCK(cudaMemcpyAsync(out_acc_host, acc, (size_t)n * 3 * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+    MCK(cudaStreamSynchronize(h->stream));
     return DPOMP_OK;
 }
 
@@ -229,8 +213,8 @@ extern "C" {
 int dpomp_da_loglike(dpomp_mbp* h, const double* theta, int32_t n, double* out_ll2) {
     if (!h || !theta || !out_ll2) return dpomp_set_error(DPOMP_ERR_ARG, "null argument");
     if (n < 1 || n > h->n) return dpomp_set_error(DPOMP_ERR_ARG, "n out of range");
-    DCK(cudaSetDevice(h->device));
-    DCK(cudaMemcpyAsync(h->theta_f, theta, (size_t)n * h->dm.n_params * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+    MCK(cudaSetDevice(h->device));
+    MCK(cudaMemcpyAsync(h->theta_f, theta, (size_t)n * h->dm.n_params * sizeof(double), cudaMemcpyHostToDevice, h->stream));
     return da_launch(h, nullptr, n, 0, 1, out_ll2, nullptr);
 }
 
@@ -242,15 +226,15 @@ int dpomp_da_step(dpomp_mbp* h, const double* theta_cur, const double* theta_f, 
     if (mvp < 1) return dpomp_set_error(DPOMP_ERR_ARG, "mvp must be positive");
     for (int p = 0; p < n; ++p)
         if (kind[p] > 2) return dpomp_set_error(DPOMP_ERR_ARG, "kind must be 0 (theta), 1 (trajectory) or 2 (skip)");
-    DCK(cudaSetDevice(h->device));
-    if (!h->da_work) DCK(cudaMalloc((void**)&h->da_work, (3 * (size_t)h->n + 1) * sizeof(int)));
+    MCK(cudaSetDevice(h->device));
+    if (!h->da_work) MCK(cudaMalloc((void**)&h->da_work, (3 * (size_t)h->n + 1) * sizeof(int)));
     // room for traj_props inserts on the longest trajectory (inserts beyond max_traj are rejected)
     int* d_max = h->da_work + 3 * (size_t)h->n;
-    DCK(cudaMemsetAsync(d_max, 0, sizeof(int), h->stream));
+    MCK(cudaMemsetAsync(d_max, 0, sizeof(int), h->stream));
     da_max_len_kernel<<<(unsigned)((n + 255) / 256), 256, 0, h->stream>>>(h->store[h->cur].len, n, d_max);
-    DCK(cudaGetLastError());
-    DCK(cudaMemcpyAsync(h->h_need_grow, d_max, sizeof(int), cudaMemcpyDeviceToHost, h->stream));
-    DCK(cudaStreamSynchronize(h->stream));
+    MCK(cudaGetLastError());
+    MCK(cudaMemcpyAsync(h->h_need_grow, d_max, sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+    MCK(cudaStreamSynchronize(h->stream));
     const long long need0 = (long long)*h->h_need_grow + traj_props;
     const int need = need0 < h->cap_max ? (int)need0 : h->cap_max;
     if (need > h->cap) {
@@ -258,9 +242,9 @@ int dpomp_da_step(dpomp_mbp* h, const double* theta_cur, const double* theta_f, 
         if (rc) return rc;
     }
     const size_t tb = (size_t)n * h->dm.n_params * sizeof(double);
-    DCK(cudaMemcpyAsync(h->theta_i, theta_cur, tb, cudaMemcpyHostToDevice, h->stream));
-    DCK(cudaMemcpyAsync(h->theta_f, theta_f, tb, cudaMemcpyHostToDevice, h->stream));
-    DCK(cudaMemcpyAsync(h->valid, kind, (size_t)n, cudaMemcpyHostToDevice, h->stream));
+    MCK(cudaMemcpyAsync(h->theta_i, theta_cur, tb, cudaMemcpyHostToDevice, h->stream));
+    MCK(cudaMemcpyAsync(h->theta_f, theta_f, tb, cudaMemcpyHostToDevice, h->stream));
+    MCK(cudaMemcpyAsync(h->valid, kind, (size_t)n, cudaMemcpyHostToDevice, h->stream));
     return da_launch(h, h->valid, n, traj_props, mvp, out_ll2, out_acc);
 }
 

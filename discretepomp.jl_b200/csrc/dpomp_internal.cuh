@@ -9,6 +9,7 @@
 
 #include "../../include/dpomp.h"
 #include "dpomp_dev.cuh"
+#include "dpomp_models.cuh"
 #include "obs_count.cuh"
 
 namespace dpomp {
@@ -250,7 +251,9 @@ cudaError_t launch_sim_weight(const ModelHost& m, int sim_precision, int items, 
 int sim_persist_capacity(const ModelHost& m, int sim_precision, int items);
 // co-resident CTAs of the fused step kernel for this model / geometry on the current device (0 = unavailable)
 int sim_fused_capacity(const ModelHost& m, int sim_precision, int items);
-int builtin_model_id(const dpomp_model_desc& d);  // 0 = generic rate table, > 0 = hand-specialised predefined model
+// the kernel family a model runs on (dpomp_models.cuh): kModelCountObs for a count observation family, else the id of the
+// predefined model its rate table equals, else kModelGeneric
+int kernel_model_id(const ModelHost& m);
 cudaError_t launch_resample(int items, const ResampleLaunch& a, cudaStream_t stream);
 cudaError_t launch_sum_events(const unsigned long long* grp_ev_dev, long long n, unsigned long long* out_dev, cudaStream_t stream);
 cudaError_t launch_gather_filters(int32_t* dst, const int32_t* src, const int64_t* dst_slots_dev,

@@ -1,5 +1,5 @@
 // dpomp_models.cuh -- the predefined density-dependent models of the reference with compile-time rate structure, shared by
-// the particle-filter event loop (pf_sim.cuh) and the trajectory walks of the MBP layer (mbp.cu).
+// the particle-filter event loop (pf_sim.cuh) and the trajectory walks of the MBP and DA layers (mbp.cu, da.cu).
 #pragma once
 
 namespace dpomp {
@@ -26,5 +26,11 @@ DPOMP_BUILTIN(kModelSEIS, 3, 3, DPOMP_L(0, 1, 2), DPOMP_L(2, -1, -1), DPOMP_L({-
 DPOMP_BUILTIN(kModelLOTKA, 2, 3, DPOMP_L(1, 0, 0), DPOMP_L(-1, 1, -1), DPOMP_L({0, 1}, {1, -1}, {-1, 0}))
 #undef DPOMP_L
 #undef DPOMP_BUILTIN
+// the predefined models above: the filter, the MBP walks and the DA walks are instantiated for each of them, and
+// kernel_model_id (pf_kernels.cu) recognises a model's rate table as one of them
+#define DPOMP_BUILTIN_MODELS(X) X(kModelSI) X(kModelSIR) X(kModelSIS) X(kModelSEI) X(kModelSEIR) X(kModelSEIS) X(kModelLOTKA)
+
+// the generic rate table with a count observation family (obs_count.cuh): the kernels of every model with a count family
+constexpr int kModelCountObs = -1;
 
 }  // namespace dpomp

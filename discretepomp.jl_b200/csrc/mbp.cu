@@ -116,11 +116,11 @@ struct WarpShared {  // per warp
 };
 
 // iterate_particle! (src/hmm_sim.jl:6-25) of particle p; `writer`: this thread stores the particle's scalars
-template <class IO, class R, bool COUNT = false>
+template <int MODEL, class IO>
 __device__ __forceinline__ void mbp_iterate_body(const MbpModel& m, MbpStore& st, IO& io, int p, bool writer, const double* theta,
                                                  const double* obs_time, const double* obs_ysum, int cap, int t, int fresh, int has_lik,
-                                                 uint64_t key, uint32_t id0, double* out_logg, const MbpGrow& g,
-                                                 const CountObs& co = CountObs{}) {
+                                                 uint64_t key, uint32_t id0, double* out_logg, const MbpGrow& g, const CountObs& co) {
+    using R = MbpRates<MODEL>;
     const int nc = mbp_nc<R>(m), ne = mbp_ne<R>(m);
     const double* thp = theta + (size_t)p * m.n_params;
     double th[R::PMAX];
@@ -149,7 +149,7 @@ __device__ __forceinline__ void mbp_iterate_body(const MbpModel& m, MbpStore& st
         ++len;
     }
     io.finish(len);
-    const double out = overflow ? -INFINITY : mbp_obs_ll<R, COUNT>(m, co, th, t, obs_ysum[t], x);
+    const double out = overflow ? -INFINITY : mbp_obs_ll<MODEL>(m, co, th, t, obs_ysum[t], x);
     if (!writer) return;
     if (overflow && cap < g.cap_max) {  // the stride, not MAX_TRAJ: nothing is committed, the host grows the store and re-launches
         *g.need_grow = 1;
@@ -165,37 +165,36 @@ __device__ __forceinline__ void mbp_iterate_body(const MbpModel& m, MbpStore& st
     g.done[p] = g.call_id;
 }
 
-template <int MODEL>
-__global__ void __launch_bounds__(128) mbp_iterate_kernel(const __grid_constant__ MbpModel m, MbpStore st, const double* theta,
-                                                           const double* obs_time, const double* obs_ysum, int n, int cap, int t,
-                                                           int fresh, int has_lik, uint64_t key, uint32_t id0, double* out_logg,
-                                                           MbpGrow g) {
-    const int p = blockIdx.x * blockDim.x + threadIdx.x;
-    if (p >= n || g.done[p] == g.call_id) return;
-    ThreadIO io{nullptr, nullptr, 0, st.ev_time + (size_t)p * cap, st.ev_type + (size_t)p * cap};
-    mbp_iterate_body<ThreadIO, MbpRates<MODEL>>(m, st, io, p, true, theta, obs_time, obs_ysum, cap, t, fresh, has_lik, key, id0, out_logg, g);
-}
-template <int MODEL>
-__global__ void __launch_bounds__(32 * kMbpWarpsPerCta) mbp_iterate_warp_kernel(const __grid_constant__ MbpModel m, MbpStore st,
+// WARP: one warp per trajectory (WarpIO), else one thread per trajectory (ThreadIO); 128 threads per CTA either way
+template <int MODEL, bool WARP>
+__global__ void __launch_bounds__(32 * kMbpWarpsPerCta) mbp_iterate_kernel(const __grid_constant__ MbpModel m, MbpStore st,
                                                            const double* theta, const double* obs_time, const double* obs_ysum, int n,
                                                            int cap, int t, int fresh, int has_lik, uint64_t key, uint32_t id0,
-                                                           double* out_logg, MbpGrow g) {
-    __shared__ WarpShared sh[kMbpWarpsPerCta];
-    const int warp = threadIdx.x >> 5, p = blockIdx.x * kMbpWarpsPerCta + warp;
-    if (p >= n || g.done[p] == g.call_id) return;
-    WarpShared& w = sh[warp];
-    const int len0 = st.len[p];
-    WarpIO io{nullptr, nullptr, 0, st.ev_time + (size_t)p * cap, st.ev_type + (size_t)p * cap, w.it, w.iy, w.ft, w.fy, 0, len0, cap};
-    mbp_iterate_body<WarpIO, MbpRates<MODEL>>(m, st, io, p, (threadIdx.x & 31) == 0, theta, obs_time, obs_ysum, cap, t, fresh, has_lik, key,
-                                              id0, out_logg, g);
+                                                           double* out_logg, MbpGrow g, const __grid_constant__ CountObs co) {
+    if constexpr (WARP) {
+        __shared__ WarpShared sh[kMbpWarpsPerCta];
+        const int warp = threadIdx.x >> 5, p = blockIdx.x * kMbpWarpsPerCta + warp;
+        if (p >= n || g.done[p] == g.call_id) return;
+        WarpShared& w = sh[warp];
+        const int len0 = st.len[p];
+        WarpIO io{nullptr, nullptr, 0, st.ev_time + (size_t)p * cap, st.ev_type + (size_t)p * cap, w.it, w.iy, w.ft, w.fy, 0, len0, cap};
+        mbp_iterate_body<MODEL>(m, st, io, p, (threadIdx.x & 31) == 0, theta, obs_time, obs_ysum, cap, t, fresh, has_lik, key, id0,
+                                out_logg, g, co);
+    } else {
+        const int p = blockIdx.x * blockDim.x + threadIdx.x;
+        if (p >= n || g.done[p] == g.call_id) return;
+        ThreadIO io{nullptr, nullptr, 0, st.ev_time + (size_t)p * cap, st.ev_type + (size_t)p * cap};
+        mbp_iterate_body<MODEL>(m, st, io, p, true, theta, obs_time, obs_ysum, cap, t, fresh, has_lik, key, id0, out_logg, g, co);
+    }
 }
 
 // partial_model_based_proposal (src/hmm_mbp.jl:83-108): xi = current store (through io), xf = proposal store
-template <class IO, class R, bool COUNT = false>
+template <int MODEL, class IO>
 __device__ __forceinline__ void mbp_propose_body(const MbpModel& m, MbpStore& xf, IO& io, int p, bool writer, bool is_valid,
                                                  const double* theta_i, const double* theta_f, const double* obs_time,
                                                  const double* obs_ysum, const int* obs_haslik, int cap, int ymax, uint64_t key,
-                                                 uint32_t id0, double* out_ll, const MbpGrow& g, const CountObs& co = CountObs{}) {
+                                                 uint32_t id0, double* out_ll, const MbpGrow& g, const CountObs& co) {
+    using R = MbpRates<MODEL>;
     const int nc = mbp_nc<R>(m), ne = mbp_ne<R>(m);
     double ll0 = 0.0, ll1 = 0.0;
     int flen = 0;
@@ -286,7 +285,7 @@ __device__ __forceinline__ void mbp_propose_body(const MbpModel& m, MbpStore& xf
             }
             if (overflow) break;
             time = t_obs;
-            ll1 = mbp_obs_ll<R, COUNT>(m, co, thf, oi, obs_ysum[oi], xfc);
+            ll1 = mbp_obs_ll<MODEL>(m, co, thf, oi, obs_ysum[oi], xfc);
             if (obs_haslik[oi]) ll0 += ll1;
         }
         if (overflow) ll0 = -INFINITY;
@@ -308,88 +307,31 @@ __device__ __forceinline__ void mbp_propose_body(const MbpModel& m, MbpStore& xf
     g.done[p] = g.call_id;
 }
 
-template <int MODEL>
-__global__ void __launch_bounds__(128) mbp_propose_kernel(const __grid_constant__ MbpModel m, MbpStore xi, MbpStore xf,
-                                                           const double* theta_i, const double* theta_f, const unsigned char* valid,
-                                                           const double* obs_time, const double* obs_ysum, const int* obs_haslik,
-                                                           int n, int cap, int ymax, uint64_t key, uint32_t id0, double* out_ll,
-                                                           MbpGrow g) {
-    const int p = blockIdx.x * blockDim.x + threadIdx.x;
-    if (p >= n || g.done[p] == g.call_id) return;
-    ThreadIO io{xi.ev_time + (size_t)p * cap, xi.ev_type + (size_t)p * cap, xi.len[p], xf.ev_time + (size_t)p * cap,
-                xf.ev_type + (size_t)p * cap};
-    mbp_propose_body<ThreadIO, MbpRates<MODEL>>(m, xf, io, p, true, valid[p] != 0, theta_i, theta_f, obs_time, obs_ysum, obs_haslik, cap,
-                                                ymax, key, id0, out_ll, g);
-}
-template <int MODEL>
-__global__ void __launch_bounds__(32 * kMbpWarpsPerCta) mbp_propose_warp_kernel(const __grid_constant__ MbpModel m, MbpStore xi,
-                                                           MbpStore xf, const double* theta_i, const double* theta_f,
-                                                           const unsigned char* valid, const double* obs_time, const double* obs_ysum,
-                                                           const int* obs_haslik, int n, int cap, int ymax, uint64_t key, uint32_t id0,
-                                                           double* out_ll, MbpGrow g) {
-    __shared__ WarpShared sh[kMbpWarpsPerCta];
-    const int warp = threadIdx.x >> 5, p = blockIdx.x * kMbpWarpsPerCta + warp;
-    if (p >= n || g.done[p] == g.call_id) return;
-    WarpShared& w = sh[warp];
-    WarpIO io{xi.ev_time + (size_t)p * cap, xi.ev_type + (size_t)p * cap, xi.len[p], xf.ev_time + (size_t)p * cap,
-              xf.ev_type + (size_t)p * cap, w.it, w.iy, w.ft, w.fy, 0, 0, cap};
-    const bool is_valid = valid[p] != 0;
-    if (is_valid) io.load(0);
-    mbp_propose_body<WarpIO, MbpRates<MODEL>>(m, xf, io, p, (threadIdx.x & 31) == 0, is_valid, theta_i, theta_f, obs_time, obs_ysum,
-                                              obs_haslik, cap, ymax, key, id0, out_ll, g);
-}
-
-// count observation families (generic rate table only): the same walks with the count log pmf
-__global__ void __launch_bounds__(128) mbp_iterate_count_kernel(const __grid_constant__ MbpModel m, MbpStore st, const double* theta,
-                                                                 const double* obs_time, const double* obs_ysum, int n, int cap, int t,
-                                                                 int fresh, int has_lik, uint64_t key, uint32_t id0, double* out_logg,
-                                                                 MbpGrow g, const __grid_constant__ CountObs co) {
-    const int p = blockIdx.x * blockDim.x + threadIdx.x;
-    if (p >= n || g.done[p] == g.call_id) return;
-    ThreadIO io{nullptr, nullptr, 0, st.ev_time + (size_t)p * cap, st.ev_type + (size_t)p * cap};
-    mbp_iterate_body<ThreadIO, MbpRates<kModelGeneric>, true>(m, st, io, p, true, theta, obs_time, obs_ysum, cap, t, fresh, has_lik, key,
-                                                              id0, out_logg, g, co);
-}
-__global__ void __launch_bounds__(32 * kMbpWarpsPerCta) mbp_iterate_warp_count_kernel(const __grid_constant__ MbpModel m, MbpStore st,
-                                                           const double* theta, const double* obs_time, const double* obs_ysum, int n,
-                                                           int cap, int t, int fresh, int has_lik, uint64_t key, uint32_t id0,
-                                                           double* out_logg, MbpGrow g, const __grid_constant__ CountObs co) {
-    __shared__ WarpShared sh[kMbpWarpsPerCta];
-    const int warp = threadIdx.x >> 5, p = blockIdx.x * kMbpWarpsPerCta + warp;
-    if (p >= n || g.done[p] == g.call_id) return;
-    WarpShared& w = sh[warp];
-    const int len0 = st.len[p];
-    WarpIO io{nullptr, nullptr, 0, st.ev_time + (size_t)p * cap, st.ev_type + (size_t)p * cap, w.it, w.iy, w.ft, w.fy, 0, len0, cap};
-    mbp_iterate_body<WarpIO, MbpRates<kModelGeneric>, true>(m, st, io, p, (threadIdx.x & 31) == 0, theta, obs_time, obs_ysum, cap, t,
-                                                            fresh, has_lik, key, id0, out_logg, g, co);
-}
-__global__ void __launch_bounds__(128) mbp_propose_count_kernel(const __grid_constant__ MbpModel m, MbpStore xi, MbpStore xf,
-                                                                 const double* theta_i, const double* theta_f, const unsigned char* valid,
-                                                                 const double* obs_time, const double* obs_ysum, const int* obs_haslik,
-                                                                 int n, int cap, int ymax, uint64_t key, uint32_t id0, double* out_ll,
-                                                                 MbpGrow g, const __grid_constant__ CountObs co) {
-    const int p = blockIdx.x * blockDim.x + threadIdx.x;
-    if (p >= n || g.done[p] == g.call_id) return;
-    ThreadIO io{xi.ev_time + (size_t)p * cap, xi.ev_type + (size_t)p * cap, xi.len[p], xf.ev_time + (size_t)p * cap,
-                xf.ev_type + (size_t)p * cap};
-    mbp_propose_body<ThreadIO, MbpRates<kModelGeneric>, true>(m, xf, io, p, true, valid[p] != 0, theta_i, theta_f, obs_time, obs_ysum,
-                                                              obs_haslik, cap, ymax, key, id0, out_ll, g, co);
-}
-__global__ void __launch_bounds__(32 * kMbpWarpsPerCta) mbp_propose_warp_count_kernel(const __grid_constant__ MbpModel m, MbpStore xi,
+template <int MODEL, bool WARP>
+__global__ void __launch_bounds__(32 * kMbpWarpsPerCta) mbp_propose_kernel(const __grid_constant__ MbpModel m, MbpStore xi,
                                                            MbpStore xf, const double* theta_i, const double* theta_f,
                                                            const unsigned char* valid, const double* obs_time, const double* obs_ysum,
                                                            const int* obs_haslik, int n, int cap, int ymax, uint64_t key, uint32_t id0,
                                                            double* out_ll, MbpGrow g, const __grid_constant__ CountObs co) {
-    __shared__ WarpShared sh[kMbpWarpsPerCta];
-    const int warp = threadIdx.x >> 5, p = blockIdx.x * kMbpWarpsPerCta + warp;
-    if (p >= n || g.done[p] == g.call_id) return;
-    WarpShared& w = sh[warp];
-    WarpIO io{xi.ev_time + (size_t)p * cap, xi.ev_type + (size_t)p * cap, xi.len[p], xf.ev_time + (size_t)p * cap,
-              xf.ev_type + (size_t)p * cap, w.it, w.iy, w.ft, w.fy, 0, 0, cap};
-    const bool is_valid = valid[p] != 0;
-    if (is_valid) io.load(0);
-    mbp_propose_body<WarpIO, MbpRates<kModelGeneric>, true>(m, xf, io, p, (threadIdx.x & 31) == 0, is_valid, theta_i, theta_f, obs_time,
-                                                            obs_ysum, obs_haslik, cap, ymax, key, id0, out_ll, g, co);
+    if constexpr (WARP) {
+        __shared__ WarpShared sh[kMbpWarpsPerCta];
+        const int warp = threadIdx.x >> 5, p = blockIdx.x * kMbpWarpsPerCta + warp;
+        if (p >= n || g.done[p] == g.call_id) return;
+        WarpShared& w = sh[warp];
+        WarpIO io{xi.ev_time + (size_t)p * cap, xi.ev_type + (size_t)p * cap, xi.len[p], xf.ev_time + (size_t)p * cap,
+                  xf.ev_type + (size_t)p * cap, w.it, w.iy, w.ft, w.fy, 0, 0, cap};
+        const bool is_valid = valid[p] != 0;
+        if (is_valid) io.load(0);
+        mbp_propose_body<MODEL>(m, xf, io, p, (threadIdx.x & 31) == 0, is_valid, theta_i, theta_f, obs_time, obs_ysum, obs_haslik, cap,
+                                ymax, key, id0, out_ll, g, co);
+    } else {
+        const int p = blockIdx.x * blockDim.x + threadIdx.x;
+        if (p >= n || g.done[p] == g.call_id) return;
+        ThreadIO io{xi.ev_time + (size_t)p * cap, xi.ev_type + (size_t)p * cap, xi.len[p], xf.ev_time + (size_t)p * cap,
+                    xf.ev_type + (size_t)p * cap};
+        mbp_propose_body<MODEL>(m, xf, io, p, true, valid[p] != 0, theta_i, theta_f, obs_time, obs_ysum, obs_haslik, cap, ymax, key,
+                                id0, out_ll, g, co);
+    }
 }
 
 // dst[dst_slot[k]] <- src[src_slot[k]] : one CTA per particle, only the live part of the trajectory moves
@@ -662,13 +604,7 @@ __global__ void __launch_bounds__(128) mbp_copy_flagged_kernel(MbpStore dst, Mbp
 // ------------------------------------------------------------------------------------------------------------
 using namespace dpomp;
 
-// struct dpomp_model and dpomp_set_error: dpomp_internal.cuh
-
-#define MCK(expr)                                                                                         \
-    do {                                                                                                  \
-        cudaError_t _e = (expr);                                                                          \
-        if (_e != cudaSuccess) return dpomp_set_error(DPOMP_ERR_CUDA, std::string(#expr) + ": " + cudaGetErrorString(_e)); \
-    } while (0)
+// struct dpomp_model and dpomp_set_error: dpomp_internal.cuh; MCK: mbp_walk.cuh
 
 // replicated device state of the outer layer (all n_total theta-particles; see the kernels above)
 struct MbpOuter {
@@ -702,8 +638,6 @@ uint64_t mbp_next_key(dpomp_mbp* h) {
     h->call_index += 1;
     return k;
 }
-// the kernels are instantiated for the generic rate table and for every predefined model
-#define DPOMP_MBP_MODELS(X) X(kModelGeneric) X(kModelSI) X(kModelSIR) X(kModelSIS) X(kModelSEI) X(kModelSEIR) X(kModelSEIS) X(kModelLOTKA)
 // one warp per trajectory while the warps of a launch fit on the device a few times over, else one thread per trajectory
 static bool mbp_use_warps(const dpomp_mbp* h, int n) { return h->mode == 2 || (h->mode == 0 && n <= kMbpWarpThreshold); }
 static void mbp_outer_free(dpomp_mbp* h) {
@@ -757,6 +691,58 @@ int mbp_grow(dpomp_mbp* h, int new_cap) {
     return DPOMP_OK;
 }
 
+// launch() until every particle has committed: a walk that reaches the stride commits nothing and raises need_grow, the host
+// widens the stride and launches the same kernel again with the same key for the particles left (see MbpGrow); synchronises
+template <class Launch>
+static int mbp_launch_until_committed(dpomp_mbp* h, Launch&& launch) {
+    for (;;) {
+        MCK(cudaMemsetAsync(h->need_grow, 0, sizeof(int), h->stream));
+        launch();
+        MCK(cudaGetLastError());
+        MCK(cudaMemcpyAsync(h->h_need_grow, h->need_grow, sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+        MCK(cudaStreamSynchronize(h->stream));
+        if (!*h->h_need_grow) return DPOMP_OK;
+        const int rc = mbp_grow(h, h->cap > h->cap_max / 2 ? h->cap_max : 2 * h->cap);
+        if (rc) return rc;
+    }
+}
+// CTAs of a walk launch over n trajectories: 128 threads per CTA, one trajectory per thread or per warp
+static unsigned mbp_walk_grid(bool warps, int n) {
+    return warps ? (unsigned)((n + kMbpWarpsPerCta - 1) / kMbpWarpsPerCta) : (unsigned)((n + 127) / 128);
+}
+
+// iterate_particle! for particles 1..n of this store, theta / outputs on the DEVICE (theta_dev [n][d], h->out [n])
+static int mbp_launch_iterate(dpomp_mbp* h, const double* theta_dev, int n, int obs_i, int fresh, uint64_t key) {
+    const bool warps = mbp_use_warps(h, n);
+    const int has_lik = h->model->h.obs_id[obs_i - 1] > 0;
+    const MbpGrow g{h->cap_max, ++h->call_id, h->done, h->need_grow};
+    return mbp_launch_until_committed(h, [&] {
+        with_walk_model(h->model_id, [&](auto model) {
+            constexpr int MODEL = decltype(model)::value;
+            const auto kern = warps ? mbp_iterate_kernel<MODEL, true> : mbp_iterate_kernel<MODEL, false>;
+            kern<<<mbp_walk_grid(warps, n), 32 * kMbpWarpsPerCta, 0, h->stream>>>(
+                h->dm, h->store[h->cur], theta_dev, h->obs_time, h->obs_ysum, n, h->cap, obs_i - 1, fresh ? 1 : 0, has_lik, key,
+                (uint32_t)h->batch_offset, h->out, g, h->cobs);
+        });
+    });
+}
+
+// partial_model_based_proposal for particles 1..n, all arguments on the DEVICE; result in h->out [n][2]
+static int mbp_launch_propose(dpomp_mbp* h, const double* theta_i_dev, const double* theta_f_dev, const unsigned char* valid_dev, int n,
+                              int ymax, uint64_t key) {
+    const bool warps = mbp_use_warps(h, n);
+    const MbpGrow g{h->cap_max, ++h->call_id, h->done, h->need_grow};
+    return mbp_launch_until_committed(h, [&] {
+        with_walk_model(h->model_id, [&](auto model) {
+            constexpr int MODEL = decltype(model)::value;
+            const auto kern = warps ? mbp_propose_kernel<MODEL, true> : mbp_propose_kernel<MODEL, false>;
+            kern<<<mbp_walk_grid(warps, n), 32 * kMbpWarpsPerCta, 0, h->stream>>>(
+                h->dm, h->store[h->cur], h->store[2], theta_i_dev, theta_f_dev, valid_dev, h->obs_time, h->obs_ysum, h->obs_haslik, n,
+                h->cap, ymax, key, (uint32_t)h->batch_offset, h->out, g, h->cobs);
+        });
+    });
+}
+
 extern "C" {
 
 int dpomp_mbp_create(const dpomp_model* model, int32_t n_particles, int32_t max_traj, uint64_t seed, int32_t device,
@@ -778,7 +764,7 @@ int dpomp_mbp_create(const dpomp_model* model, int32_t n_particles, int32_t max_
     h->cap = max_traj < kMbpInitialStride ? max_traj : kMbpInitialStride;
     MbpModel& m = h->dm;
     m.n_comp = d.n_compartments; m.n_events = d.n_events; m.n_params = d.n_params; m.t0_index = d.t0_index;
-    h->model_id = builtin_model_id(d);
+    h->model_id = kernel_model_id(model->h);
     for (int ev = 0; ev < DPOMP_MAX_EVENTS; ++ev) {
         m.par[ev] = d.rate_par[ev]; m.k1[ev] = d.rate_k1[ev]; m.k2[ev] = d.rate_k2[ev]; m.kd[ev] = d.rate_kd[ev];
         m.has_den[ev] = d.rate_has_den[ev];
@@ -820,7 +806,6 @@ int dpomp_mbp_create(const dpomp_model* model, int32_t n_particles, int32_t max_
              cudaMemcpy(h->obs_lgy, model->h.obs_lgy.data(), d.n_obs * sizeof(double), cudaMemcpyHostToDevice) == cudaSuccess &&
              cudaMemcpy(h->obs_lgk, model->h.obs_lgk.data(), d.n_obs * sizeof(double), cudaMemcpyHostToDevice) == cudaSuccess;
         h->cobs = count_obs_of(model->h, h->obs_lgy, h->obs_lgk);
-        h->model_id = kModelGeneric;  // the predefined-model walks evaluate the Gaussian only
     }
     if (!ok) {
         std::string msg = std::string("dpomp_mbp_create: ") + cudaGetErrorString(cudaGetLastError());
@@ -858,91 +843,6 @@ int dpomp_mbp_reset(dpomp_mbp* h) {
     mbp_reset_kernel<<<(h->n + 127) / 128, 128, 0, h->stream>>>(h->dm, h->store[h->cur], h->n);
     MCK(cudaGetLastError());
     MCK(cudaStreamSynchronize(h->stream));
-    return DPOMP_OK;
-}
-
-// iterate_particle! for particles 1..n of this store, theta / outputs on the DEVICE (theta_dev [n][d], h->out [n]); the
-// launch repeats after the stride has grown (same key, uncommitted particles only: see MbpGrow); synchronises the stream
-static int mbp_launch_iterate(dpomp_mbp* h, const double* theta_dev, int n, int obs_i, int fresh, uint64_t key) {
-    const bool warps = mbp_use_warps(h, n);
-    const int has_lik = h->model->h.obs_id[obs_i - 1] > 0;
-    const MbpGrow g{h->cap_max, ++h->call_id, h->done, h->need_grow};
-#define DPOMP_MBP_ITERATE(ID)                                                                                                  \
-    if (h->model_id == ID) {                                                                                                   \
-        if (warps)                                                                                                             \
-            mbp_iterate_warp_kernel<ID><<<(n + kMbpWarpsPerCta - 1) / kMbpWarpsPerCta, 32 * kMbpWarpsPerCta, 0, h->stream>>>(  \
-                h->dm, h->store[h->cur], theta_dev, h->obs_time, h->obs_ysum, n, h->cap, obs_i - 1, fresh ? 1 : 0, has_lik,    \
-                key, (uint32_t)h->batch_offset, h->out, g);                                                                    \
-        else                                                                                                                   \
-            mbp_iterate_kernel<ID><<<(n + 127) / 128, 128, 0, h->stream>>>(h->dm, h->store[h->cur], theta_dev, h->obs_time,    \
-                                                                           h->obs_ysum, n, h->cap, obs_i - 1, fresh ? 1 : 0,   \
-                                                                           has_lik, key, (uint32_t)h->batch_offset, h->out, g); \
-    }
-    for (;;) {
-        MCK(cudaMemsetAsync(h->need_grow, 0, sizeof(int), h->stream));
-        if (h->cobs.family != DPOMP_OBS_GAUSSIAN) {
-            if (warps)
-                mbp_iterate_warp_count_kernel<<<(n + kMbpWarpsPerCta - 1) / kMbpWarpsPerCta, 32 * kMbpWarpsPerCta, 0, h->stream>>>(
-                    h->dm, h->store[h->cur], theta_dev, h->obs_time, h->obs_ysum, n, h->cap, obs_i - 1, fresh ? 1 : 0, has_lik, key,
-                    (uint32_t)h->batch_offset, h->out, g, h->cobs);
-            else
-                mbp_iterate_count_kernel<<<(n + 127) / 128, 128, 0, h->stream>>>(h->dm, h->store[h->cur], theta_dev, h->obs_time,
-                                                                                 h->obs_ysum, n, h->cap, obs_i - 1, fresh ? 1 : 0, has_lik,
-                                                                                 key, (uint32_t)h->batch_offset, h->out, g, h->cobs);
-        } else {
-            DPOMP_MBP_MODELS(DPOMP_MBP_ITERATE)
-        }
-        MCK(cudaGetLastError());
-        MCK(cudaMemcpyAsync(h->h_need_grow, h->need_grow, sizeof(int), cudaMemcpyDeviceToHost, h->stream));
-        MCK(cudaStreamSynchronize(h->stream));
-        if (!*h->h_need_grow) break;
-        const int rc = mbp_grow(h, h->cap > h->cap_max / 2 ? h->cap_max : 2 * h->cap);
-        if (rc) return rc;
-    }
-#undef DPOMP_MBP_ITERATE
-    return DPOMP_OK;
-}
-
-// partial_model_based_proposal for particles 1..n, all arguments on the DEVICE; result in h->out [n][2]
-static int mbp_launch_propose(dpomp_mbp* h, const double* theta_i_dev, const double* theta_f_dev, const unsigned char* valid_dev, int n,
-                              int ymax, uint64_t key) {
-    const bool warps = mbp_use_warps(h, n);
-    const MbpGrow g{h->cap_max, ++h->call_id, h->done, h->need_grow};
-#define DPOMP_MBP_PROPOSE(ID)                                                                                                  \
-    if (h->model_id == ID) {                                                                                                   \
-        if (warps)                                                                                                             \
-            mbp_propose_warp_kernel<ID><<<(n + kMbpWarpsPerCta - 1) / kMbpWarpsPerCta, 32 * kMbpWarpsPerCta, 0, h->stream>>>(  \
-                h->dm, h->store[h->cur], h->store[2], theta_i_dev, theta_f_dev, valid_dev, h->obs_time, h->obs_ysum,           \
-                h->obs_haslik, n, h->cap, ymax, key, (uint32_t)h->batch_offset, h->out, g);                                    \
-        else                                                                                                                   \
-            mbp_propose_kernel<ID><<<(n + 127) / 128, 128, 0, h->stream>>>(h->dm, h->store[h->cur], h->store[2], theta_i_dev,  \
-                                                                           theta_f_dev, valid_dev, h->obs_time, h->obs_ysum,   \
-                                                                           h->obs_haslik, n, h->cap, ymax, key,                \
-                                                                           (uint32_t)h->batch_offset, h->out, g);              \
-    }
-    for (;;) {
-        MCK(cudaMemsetAsync(h->need_grow, 0, sizeof(int), h->stream));
-        if (h->cobs.family != DPOMP_OBS_GAUSSIAN) {
-            if (warps)
-                mbp_propose_warp_count_kernel<<<(n + kMbpWarpsPerCta - 1) / kMbpWarpsPerCta, 32 * kMbpWarpsPerCta, 0, h->stream>>>(
-                    h->dm, h->store[h->cur], h->store[2], theta_i_dev, theta_f_dev, valid_dev, h->obs_time, h->obs_ysum, h->obs_haslik,
-                    n, h->cap, ymax, key, (uint32_t)h->batch_offset, h->out, g, h->cobs);
-            else
-                mbp_propose_count_kernel<<<(n + 127) / 128, 128, 0, h->stream>>>(h->dm, h->store[h->cur], h->store[2], theta_i_dev,
-                                                                                 theta_f_dev, valid_dev, h->obs_time, h->obs_ysum,
-                                                                                 h->obs_haslik, n, h->cap, ymax, key,
-                                                                                 (uint32_t)h->batch_offset, h->out, g, h->cobs);
-        } else {
-            DPOMP_MBP_MODELS(DPOMP_MBP_PROPOSE)
-        }
-        MCK(cudaGetLastError());
-        MCK(cudaMemcpyAsync(h->h_need_grow, h->need_grow, sizeof(int), cudaMemcpyDeviceToHost, h->stream));
-        MCK(cudaStreamSynchronize(h->stream));
-        if (!*h->h_need_grow) break;
-        const int rc = mbp_grow(h, h->cap > h->cap_max / 2 ? h->cap_max : 2 * h->cap);
-        if (rc) return rc;
-    }
-#undef DPOMP_MBP_PROPOSE
     return DPOMP_OK;
 }
 

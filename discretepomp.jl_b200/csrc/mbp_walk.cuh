@@ -1,9 +1,12 @@
 // mbp_walk.cuh -- what the trajectory walks of mbp.cu (MBP-IBIS, MBP-MCMC) and da.cu (data-augmented MCMC) share: the
-// trajectory store, the rate policies MbpRates<MODEL> / MbpRates<kModelGeneric>, the observation log-likelihoods, and the
-// host handle dpomp_mbp with the helpers that key its calls and widen its stride.
+// trajectory store, the rate policies MbpRates<MODEL>, the observation log-likelihood, and the host handle dpomp_mbp with
+// the helpers that key its calls, widen its stride and pick the walk instantiation of its model.
 #pragma once
 #include <math.h>
 #include <stdint.h>
+
+#include <string>
+#include <type_traits>
 
 #include "dpomp_dev.cuh"
 #include "dpomp_internal.cuh"
@@ -47,7 +50,8 @@ __device__ __forceinline__ uint2 mbp_draw(MbpStream& s) {
 }
 
 // ---- rate policies ----------------------------------------------------------------------------------------------------
-// MbpRates<kModelGeneric>: the integer rate table with run-time C / E (any model the table compiler accepts).
+// MbpRates<kModelGeneric>: the integer rate table with run-time C / E (any model the table compiler accepts); also the rate
+// table of MbpRates<kModelCountObs>, whose walks differ only in mbp_obs_ll.
 // MbpRates<ID>: a predefined model with compile-time structure -- loops unroll, states and rates stay in registers, and
 // rate[e] = (theta[e] * x_a) * x_b is the same f64 expression the table evaluates (l1 = x_a, l2 = x_b or 1 exactly), so both
 // give bit-identical walks; a walk is one dependent instruction chain, so its length is what the kernels' time is made of.
@@ -105,6 +109,8 @@ struct MbpRates<kModelGeneric> {
     }
     static __device__ __forceinline__ double pick(const double (&v)[EMAX], int e) { return v[e]; }
 };
+template <>
+struct MbpRates<kModelCountObs> : MbpRates<kModelGeneric> {};
 template <class R> __device__ __forceinline__ int mbp_nc(const MbpModel& m) { if constexpr (R::C > 0) return R::C; else return m.n_comp; }
 template <class R> __device__ __forceinline__ int mbp_ne(const MbpModel& m) { if constexpr (R::E > 0) return R::E; else return m.n_events; }
 
@@ -125,26 +131,23 @@ __device__ __forceinline__ int mbp_choose(const MbpModel& m, const double (&cum)
         if (i < n - 1 && cum[i] > etc) e = i;
     return e;
 }
-template <class R>
-__device__ __forceinline__ double mbp_obs_ll(const MbpModel& m, double ysum, const int (&x)[R::CMAX]) {
-    const int nc = mbp_nc<R>(m);
-    long long xs = 0;
-#pragma unroll
-    for (int c = 0; c < R::CMAX; ++c)
-        if (c < nc) xs += (long long)m.xmask[c] * x[c];
-    const double d = ysum - (double)xs;
-    return m.obs_tmp1 - __ddiv_rn(__dmul_rn(d, d), m.obs_tmp2);
-}
-// COUNT: the model's count observation family (obs_count.cuh) with its theta-indexed parameters taken from th (the walk's theta)
-template <class R, bool COUNT>
+// log g of observation t: the Gaussian, or for kModelCountObs the model's count observation family (obs_count.cuh) with its
+// theta-indexed parameters taken from th (the walk's theta)
+template <int MODEL>
 __device__ __forceinline__ double mbp_obs_ll(const MbpModel& m, const CountObs& co, const double* th, int t, double ysum,
-                                             const int (&x)[R::CMAX]) {
-    if constexpr (!COUNT) {
-        return mbp_obs_ll<R>(m, ysum, x);
-    } else {
-        long long xs = 0;
+                                             const int (&x)[MbpRates<MODEL>::CMAX]) {
+    using R = MbpRates<MODEL>;
+    long long xs = 0;
+    if constexpr (MODEL == kModelCountObs) {
         for (int c = 0; c < m.n_comp; ++c) xs += (long long)m.xmask[c] * x[c];
         return count_obs_logpmf(count_obs_const(co, th, t, ysum), ysum, (double)xs);
+    } else {
+        const int nc = mbp_nc<R>(m);
+#pragma unroll
+        for (int c = 0; c < R::CMAX; ++c)
+            if (c < nc) xs += (long long)m.xmask[c] * x[c];
+        const double d = ysum - (double)xs;
+        return m.obs_tmp1 - __ddiv_rn(__dmul_rn(d, d), m.obs_tmp2);
     }
 }
 
@@ -170,14 +173,14 @@ struct dpomp_mbp {
     MbpStore store[3]{};   // [cur], [cur ^ 1] (resample workspace), [2] proposal
     int cur = 0;
     int mode = 0;          // 0 automatic, 1 one thread per trajectory, 2 one warp per trajectory
-    int model_id = 0;      // predefined model with compile-time structure (dpomp_models.cuh), 0 = generic rate table
+    int model_id = 0;      // kernel_model_id of the model: the walk instantiation its launches run
     uint64_t seed = 0, call_index = 0, forced_key = 0;
     bool key_forced = false;
     long long batch_offset = 0;
     double *theta_i = nullptr, *theta_f = nullptr, *out = nullptr, *obs_time = nullptr, *obs_ysum = nullptr;
     int* obs_haslik = nullptr;
     double *obs_lgy = nullptr, *obs_lgk = nullptr;  // count observation constants [T] (count families only)
-    CountObs cobs{};                                // family != DPOMP_OBS_GAUSSIAN: the count kernels run
+    CountObs cobs{};                                // count observation family (read only by the kModelCountObs walks)
     unsigned char* valid = nullptr;
     int64_t* slots = nullptr;  // 2 * n
     int* da_work = nullptr;    // [3 n + 1] data-augmented MCMC (da.cu): accept counts per chain, longest trajectory
@@ -187,3 +190,27 @@ struct dpomp_mbp {
 uint64_t mbp_next_key(dpomp_mbp* h);
 // widen the stride of all three stores to new_cap (<= cap_max), keeping every trajectory
 int mbp_grow(dpomp_mbp* h, int new_cap);
+
+namespace dpomp {
+
+// launch(std::integral_constant<int, MODEL>{}) with the walk instantiation MODEL of model_id (kernel_model_id): a predefined
+// model, kModelCountObs or kModelGeneric
+template <class Launch>
+void with_walk_model(int model_id, Launch&& launch) {
+    switch (model_id) {
+#define X(ID) case ID: return launch(std::integral_constant<int, ID>{});
+        DPOMP_BUILTIN_MODELS(X)
+#undef X
+        case kModelCountObs: return launch(std::integral_constant<int, kModelCountObs>{});
+        default: return launch(std::integral_constant<int, kModelGeneric>{});
+    }
+}
+
+}  // namespace dpomp
+
+// return the CUDA error of expr from a C-ABI entry point
+#define MCK(expr)                                                                                         \
+    do {                                                                                                  \
+        cudaError_t _e = (expr);                                                                          \
+        if (_e != cudaSuccess) return dpomp_set_error(DPOMP_ERR_CUDA, std::string(#expr) + ": " + cudaGetErrorString(_e)); \
+    } while (0)

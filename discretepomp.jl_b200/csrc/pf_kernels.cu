@@ -11,16 +11,18 @@
 
 namespace dpomp {
 
-int sim_f32(const ModelHost& m, int items, const SimLaunch& a, cudaStream_t stream, int mode);
-int sim_f64(const ModelHost& m, int items, const SimLaunch& a, cudaStream_t stream, int mode);
-// count observation families: generic-table kernels only (pf_sim_count_f32.cu / pf_sim_count_f64.cu)
+// model_id: kernel_model_id of m, a predefined model or kModelGeneric
+int sim_f32(int model_id, const ModelHost& m, int items, const SimLaunch& a, cudaStream_t stream, int mode);
+int sim_f64(int model_id, const ModelHost& m, int items, const SimLaunch& a, cudaStream_t stream, int mode);
+// kModelCountObs (pf_sim_count_f32.cu / pf_sim_count_f64.cu)
 int sim_count_f32(const ModelHost& m, int items, const SimLaunch& a, cudaStream_t stream, int mode);
 int sim_count_f64(const ModelHost& m, int items, const SimLaunch& a, cudaStream_t stream, int mode);
 
 static int sim_dispatch(const ModelHost& m, int sim_precision, int items, const SimLaunch& a, cudaStream_t stream, int mode) {
-    if (m.obs_family != DPOMP_OBS_GAUSSIAN)
+    const int model_id = kernel_model_id(m);
+    if (model_id == kModelCountObs)
         return sim_precision == DPOMP_SIM_F64 ? sim_count_f64(m, items, a, stream, mode) : sim_count_f32(m, items, a, stream, mode);
-    return sim_precision == DPOMP_SIM_F64 ? sim_f64(m, items, a, stream, mode) : sim_f32(m, items, a, stream, mode);
+    return sim_precision == DPOMP_SIM_F64 ? sim_f64(model_id, m, items, a, stream, mode) : sim_f32(model_id, m, items, a, stream, mode);
 }
 
 cudaError_t launch_sim_weight(const ModelHost& m, int sim_precision, int items, int fused, const SimLaunch& a, cudaStream_t stream) {
@@ -49,31 +51,25 @@ CountObs count_obs_of(const ModelHost& m, const double* lgy_dev, const double* l
     return c;
 }
 
-// does the rate table equal one of the hand-specialised predefined models (pf_sim.cuh Builtin<>)?
-namespace {
-struct BuiltinSpec { int id, C, E; int A[3], B[3]; int T[3][4]; };
-const BuiltinSpec kSpecs[] = {
-    {1, 2, 1, {0}, {1}, {{-1, 1}}},
-    {2, 3, 2, {0, 1}, {1, -1}, {{-1, 1, 0}, {0, -1, 1}}},
-    {3, 2, 2, {0, 1}, {1, -1}, {{-1, 1}, {1, -1}}},
-    {4, 3, 2, {0, 1}, {2, -1}, {{-1, 1, 0}, {0, -1, 1}}},
-    {5, 4, 3, {0, 1, 2}, {2, -1, -1}, {{-1, 1, 0, 0}, {0, -1, 1, 0}, {0, 0, -1, 1}}},
-    {6, 3, 3, {0, 1, 2}, {2, -1, -1}, {{-1, 1, 0}, {0, -1, 1}, {1, 0, -1}}},
-    {7, 2, 3, {1, 0, 0}, {-1, 1, -1}, {{0, 1}, {1, -1}, {-1, 0}}},
-};
-}  // namespace
-int builtin_model_id(const dpomp_model_desc& d) {
-    for (const BuiltinSpec& s : kSpecs) {
-        if (d.n_compartments != s.C || d.n_events != s.E) continue;
-        bool ok = true;
-        for (int e = 0; e < s.E && ok; ++e) {
-            ok = d.rate_par[e] == e && d.rate_has_den[e] == 0 && d.rate_k1[e] == 0 && d.rate_k2[e] == (s.B[e] >= 0 ? 0 : 1);
-            for (int c = 0; c < s.C && ok; ++c)
-                ok = d.rate_f1[e][c] == (c == s.A[e] ? 1 : 0) && d.rate_f2[e][c] == (c == s.B[e] ? 1 : 0) && d.trans[e][c] == s.T[e][c];
-        }
-        if (ok) return s.id;
+// does the rate table equal the predefined model Builtin<ID> (dpomp_models.cuh)?
+template <int ID>
+static bool is_builtin_model(const dpomp_model_desc& d) {
+    using BM = Builtin<ID>;
+    if (d.n_compartments != BM::C || d.n_events != BM::E) return false;
+    bool ok = true;
+    for (int e = 0; e < BM::E && ok; ++e) {
+        ok = d.rate_par[e] == e && d.rate_has_den[e] == 0 && d.rate_k1[e] == 0 && d.rate_k2[e] == (BM::B(e) >= 0 ? 0 : 1);
+        for (int c = 0; c < BM::C && ok; ++c)
+            ok = d.rate_f1[e][c] == (c == BM::A(e) ? 1 : 0) && d.rate_f2[e][c] == (c == BM::B(e) ? 1 : 0) && d.trans[e][c] == BM::T(e, c);
     }
-    return 0;
+    return ok;
+}
+int kernel_model_id(const ModelHost& m) {
+    if (m.obs_family != DPOMP_OBS_GAUSSIAN) return kModelCountObs;  // the predefined-model kernels evaluate the Gaussian only
+#define X(ID) if (is_builtin_model<ID>(m.desc)) return ID;
+    DPOMP_BUILTIN_MODELS(X)
+#undef X
+    return kModelGeneric;
 }
 
 int sim_kernel_supported(int n_comp, int n_events) {

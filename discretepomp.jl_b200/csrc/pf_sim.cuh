@@ -134,7 +134,6 @@ __device__ __forceinline__ unsigned int ld_acquire_u32(const unsigned int* p) {
     return v;
 }
 // MODEL = kModelCountObs: the generic rate table with a count observation family (obs_count.cuh, a.cobs) in the weight pass
-constexpr int kModelCountObs = -1;
 template <typename Real, int C, int E, int ITEMS, int MODEL = kModelGeneric, int MODE = kModePlain, int ILP = DPOMP_SIM_ILP>
 __global__ void __launch_bounds__(kBlockThreads, sim_min_blocks<Real, C, E>())
 pf_sim_weight_kernel(const __grid_constant__ DevModel<Real, C, E> m, const __grid_constant__ SimLaunch a) {
@@ -810,12 +809,25 @@ static int sim_plain_two_per_lane(const ModelHost& mh, const SimLaunch& a, cudaS
 constexpr int kLatencyRegimeCtas = 296;  // 2 CTAs per SM
 // the instantiated generic (C, E) shapes; a model runs on the smallest shape that covers it
 #define DPOMP_SIM_SHAPES(X) X(2, 1) X(2, 2) X(2, 3) X(3, 2) X(3, 3) X(4, 3) X(4, 6) X(8, 8)
-#define DPOMP_SIM_BUILTINS(X) X(kModelSI) X(kModelSIR) X(kModelSIS) X(kModelSEI) X(kModelSEIR) X(kModelSEIS) X(kModelLOTKA)
 
-template <typename Real>
-static int sim_typed(const ModelHost& mh, int items, const SimLaunch& a, cudaStream_t stream, int mode) {
+// the rate table on its generic shape: MODEL = kModelGeneric (Gaussian) or kModelCountObs -- never the predefined-model,
+// persistent or two-per-lane kernels
+template <typename Real, int MODEL>
+static int sim_shaped(const ModelHost& mh, int items, const SimLaunch& a, cudaStream_t stream, int mode) {
     const int c = mh.desc.n_compartments, e = mh.desc.n_events;
-    const int model_id = builtin_model_id(mh.desc);
+#define X(CC, EE)                                                                                       \
+    if (c <= CC && e <= EE) {                                                                           \
+        return items == kItemsSmall ? sim_inst<Real, CC, EE, kItemsSmall, MODEL>(mh, a, stream, mode)   \
+                                    : sim_inst<Real, CC, EE, kItemsLarge, MODEL>(mh, a, stream, mode);  \
+    }
+    DPOMP_SIM_SHAPES(X)
+#undef X
+    return (mode == 2 || mode == 4) ? 0 : (int)cudaErrorInvalidValue;
+}
+
+// model_id: kernel_model_id(mh), a predefined model or kModelGeneric
+template <typename Real>
+static int sim_typed(int model_id, const ModelHost& mh, int items, const SimLaunch& a, cudaStream_t stream, int mode) {
     // latency regime: a few small filters (the reference's default 200 particles) leave most of the device idle, and a lane
     // that interleaves its two particles halves the dependent chain of a step
     const bool latency = sizeof(Real) == 4 && items == kItemsSmall && a.n_filters > 0 &&
@@ -831,31 +843,9 @@ static int sim_typed(const ModelHost& mh, int items, const SimLaunch& a, cudaStr
         }                                                                                                                 \
         return sim_inst<Real, Builtin<ID>::C, Builtin<ID>::E, kItemsLarge, ID>(mh, a, stream, mode);                      \
     }
-    DPOMP_SIM_BUILTINS(X)
+    DPOMP_BUILTIN_MODELS(X)
 #undef X
-#define X(CC, EE)                                                                                      \
-    if (c <= CC && e <= EE) {                                                                          \
-        return items == kItemsSmall ? sim_inst<Real, CC, EE, kItemsSmall>(mh, a, stream, mode)         \
-                                    : sim_inst<Real, CC, EE, kItemsLarge>(mh, a, stream, mode);        \
-    }
-    DPOMP_SIM_SHAPES(X)
-#undef X
-    return (mode == 2 || mode == 4) ? 0 : (int)cudaErrorInvalidValue;
-}
-
-// count observation families: the generic (C, E) shapes only -- never the predefined-model, persistent or two-per-lane kernels
-template <typename Real>
-static int sim_count_typed(const ModelHost& mh, int items, const SimLaunch& a, cudaStream_t stream, int mode) {
-    if (mode == 3 || mode == 4) return mode == 4 ? 0 : (int)cudaErrorInvalidValue;
-    const int c = mh.desc.n_compartments, e = mh.desc.n_events;
-#define X(CC, EE)                                                                                                \
-    if (c <= CC && e <= EE) {                                                                                    \
-        return items == kItemsSmall ? sim_inst<Real, CC, EE, kItemsSmall, kModelCountObs>(mh, a, stream, mode) \
-                                    : sim_inst<Real, CC, EE, kItemsLarge, kModelCountObs>(mh, a, stream, mode); \
-    }
-    DPOMP_SIM_SHAPES(X)
-#undef X
-    return mode == 2 ? 0 : (int)cudaErrorInvalidValue;
+    return sim_shaped<Real, kModelGeneric>(mh, items, a, stream, mode);
 }
 
 }  // namespace dpomp

@@ -4,6 +4,6 @@
 #include "pf_sim.cuh"
 namespace dpomp {
 int sim_count_f32(const ModelHost& m, int items, const SimLaunch& a, cudaStream_t stream, int mode) {
-    return sim_count_typed<float>(m, items, a, stream, mode);
+    return sim_shaped<float, kModelCountObs>(m, items, a, stream, mode);
 }
 }  // namespace dpomp

@@ -3,6 +3,6 @@
 #include "pf_sim.cuh"
 namespace dpomp {
 int sim_count_f64(const ModelHost& m, int items, const SimLaunch& a, cudaStream_t stream, int mode) {
-    return sim_count_typed<double>(m, items, a, stream, mode);
+    return sim_shaped<double, kModelCountObs>(m, items, a, stream, mode);
 }
 }  // namespace dpomp

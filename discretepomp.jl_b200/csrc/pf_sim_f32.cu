@@ -1,8 +1,8 @@
 // pf_sim_f32.cu -- f32 event-loop instantiations of the simulate+weight kernel (DPOMP_SIM_F32, the fast default).
 #include "pf_sim.cuh"
 namespace dpomp {
-int sim_f32(const ModelHost& m, int items, const SimLaunch& a, cudaStream_t stream, int mode) {
-    return sim_typed<float>(m, items, a, stream, mode);
+int sim_f32(int model_id, const ModelHost& m, int items, const SimLaunch& a, cudaStream_t stream, int mode) {
+    return sim_typed<float>(model_id, m, items, a, stream, mode);
 }
 }  // namespace dpomp
 

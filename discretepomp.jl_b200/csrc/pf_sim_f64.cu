@@ -2,7 +2,7 @@
 // draw-for-draw parity against the oracle.
 #include "pf_sim.cuh"
 namespace dpomp {
-int sim_f64(const ModelHost& m, int items, const SimLaunch& a, cudaStream_t stream, int mode) {
-    return sim_typed<double>(m, items, a, stream, mode);
+int sim_f64(int model_id, const ModelHost& m, int items, const SimLaunch& a, cudaStream_t stream, int mode) {
+    return sim_typed<double>(model_id, m, items, a, stream, mode);
 }
 }  // namespace dpomp

@@ -1,7 +1,7 @@
 """GPU tests of every compiled model instantiation against the oracle.
 
 The filter's event loop, the MBP walks and the DA walks are compiled once per model structure: the seven predefined
-density-dependent models (dpomp_models.cuh Builtin<ID>, recognised by builtin_model_id in pf_kernels.cu) and the generic
+density-dependent models (dpomp_models.cuh Builtin<ID>, recognised by kernel_model_id in pf_kernels.cu) and the generic
 rate table on each (compartments, events) shape of DPOMP_SIM_SHAPES (pf_sim.cuh).  Each instantiation is a kernel of its own
 that can be wrong on its own, and the oracle only evaluates the run-time table, so every one of them is put next to the oracle
 here on identical Philox draws.

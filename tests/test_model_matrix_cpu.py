@@ -28,7 +28,7 @@ def sim_shapes():
 
 
 def shape_of(shapes, c, e):
-    """the dispatch rule of sim_typed / sim_count_typed: the first listed shape that covers (c, e)"""
+    """the dispatch rule of sim_shaped: the first listed shape that covers (c, e)"""
     return next(((cc, ee) for cc, ee in shapes if c <= cc and e <= ee), None)
 
 
@@ -107,12 +107,17 @@ def _model_names(entries):
     return out
 
 
+def builtin_models():
+    """DPOMP_BUILTIN_MODELS (dpomp_models.cuh): the filter, the MBP walks and the DA walks are instantiated for each entry"""
+    return _model_names(_xmacro("dpomp_models.cuh", "DPOMP_BUILTIN_MODELS"))
+
+
 def _generic_shape(name):
     return shape_of(sim_shapes(), len(gm.GENERIC[name][2]), len(gm.GENERIC[name][1]))
 
 
-def test_every_predefined_filter_instantiation_has_a_case():
-    names = _model_names(_xmacro("pf_sim.cuh", "DPOMP_SIM_BUILTINS"))
+def test_every_builtin_model_has_a_filter_case():
+    names = builtin_models()
     assert None not in names and sorted(names) == sorted(IDS)
     for nm in names:
         assert nm in gm.CASES and nm in gm.FILTER_VARIANT_MODELS, nm
@@ -128,28 +133,31 @@ def test_every_generic_shape_has_a_gaussian_and_a_count_case():
         assert s in poisson, f"shape {s} of DPOMP_SIM_SHAPES has no Poisson case in test_gpu_model_matrix.py"
 
 
-@pytest.mark.parametrize("fname,macro,cases", [("mbp.cu", "DPOMP_MBP_MODELS", gm.MBP_MODELS), ("da.cu", "DPOMP_DA_MODELS", gm.DA_MODELS)])
-def test_every_walk_instantiation_has_a_case(fname, macro, cases):
-    for nm in _model_names(_xmacro(fname, macro)):
-        if nm is None:  # the generic rate table
-            assert any(c in gm.GENERIC for c in cases), macro
-        else:
-            assert nm in IDS and nm in cases, (macro, nm)
+@pytest.mark.parametrize("walk,cases", [("mbp", gm.MBP_MODELS), ("da", gm.DA_MODELS)], ids=["mbp", "da"])
+def test_every_walk_instantiation_has_a_case(walk, cases):
+    """the walks are instantiated for every predefined model and for the generic rate table (with_walk_model, mbp_walk.cuh)"""
+    for nm in builtin_models():
+        assert nm in IDS and nm in cases, (walk, nm)
+    assert any(c in gm.GENERIC for c in cases), walk
 
 
 def test_guard_fails_for_an_instantiation_without_a_case(tmp_path, monkeypatch):
-    """the guard itself: a shape added to the list, or a model added to a walk list, is reported"""
+    """the guard itself: a shape added to the list is reported, and a predefined model added to the list is reported for the
+    filter and for both walks"""
     src = open(os.path.join(CSRC, "pf_sim.cuh")).read()
     added = re.sub(r"(#define DPOMP_SIM_SHAPES\(X\)[^\n]*)", r"\1 X(6, 4)", src, count=1)
     (tmp_path / "pf_sim.cuh").write_text(added)
-    mbp = open(os.path.join(CSRC, "mbp.cu")).read()
-    (tmp_path / "mbp.cu").write_text(re.sub(r"(#define DPOMP_MBP_MODELS\(X\)[^\n]*)", r"\1 X(kModelSIRS)", mbp, count=1))
+    models = open(os.path.join(CSRC, "dpomp_models.cuh")).read()
+    (tmp_path / "dpomp_models.cuh").write_text(re.sub(r"(#define DPOMP_BUILTIN_MODELS\(X\)[^\n]*)", r"\1 X(kModelSIRS)", models, count=1))
     monkeypatch.setattr(sys.modules[__name__], "CSRC", str(tmp_path))
-    assert (6, 4) in sim_shapes()
+    assert (6, 4) in sim_shapes() and "SIRS" in builtin_models()
     with pytest.raises(AssertionError, match=r"\(6, 4\)"):
         test_every_generic_shape_has_a_gaussian_and_a_count_case()
     with pytest.raises(AssertionError):
-        test_every_walk_instantiation_has_a_case("mbp.cu", "DPOMP_MBP_MODELS", gm.MBP_MODELS)
+        test_every_builtin_model_has_a_filter_case()
+    for walk, cases in (("mbp", gm.MBP_MODELS), ("da", gm.DA_MODELS)):
+        with pytest.raises(AssertionError, match="SIRS"):
+            test_every_walk_instantiation_has_a_case(walk, cases)
 
 
 # ---- the shape each generic case runs on --------------------------------------------------------------------------------------
