@@ -18,9 +18,9 @@ from .examples import (CountObsModel, GaussianObsModel, UniformProduct, dmy_obs_
                        partial_negbin_obs_model, partial_poisson_obs_model)
 from .rate_table import ModelCompileError, compile_obs_table, compile_rate_table
 from .utils import get_observations
-from .particle_filter import (C_DF_ESS_CRIT, C_DF_PF_P, DeviceModel, ParticleFilter, compile_model, compute_ess,
-                              device_model, estimate_likelihood, get_log_pdf_fn, get_particle_filter_lpdf,
-                              get_private_model)
+from .particle_filter import (C_DF_ESS_CRIT, C_DF_PF_P, DeviceModel, FilteredStates, ParticleFilter, compile_model,
+                              compute_ess, device_model, estimate_likelihood, get_filtered_states, get_log_pdf_fn,
+                              get_particle_filter_lpdf, get_private_model)
 from .resample import rs_multinomial, rs_stratified, rs_systematic, rsp_indices
 from .distributed import Comm, migration_plan, partition_bounds, partition_owner
 from .ibis import (compute_is_mu_covar, get_mv_param, get_prop_density, run_ibis_analysis, run_pibis)

@@ -20,6 +20,7 @@ RS_SYSTEMATIC, RS_STRATIFIED, RS_MULTINOMIAL = 1, 2, 3
 SIM_F32, SIM_F64 = 0, 1
 SCATTER_REFERENCE, SCATTER_INTERLEAVED = 0, 1
 OBS_GAUSSIAN, OBS_POISSON, OBS_BINOMIAL, OBS_NEGBIN = 0, 1, 2, 3
+HISTORY_MOMENTS, HISTORY_PATHS = 1, 2
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 # DPOMP_LIB_PATH selects another build of the same library (kernel A/B measurements); there is still no fallback
@@ -93,6 +94,9 @@ _SIGS = {
     "dpomp_pf_get_last_logw": (C.c_int, [_P, C.c_int32, _P]),
     "dpomp_pf_get_last_ancestors": (C.c_int, [_P, C.c_int32, _P]),
     "dpomp_pf_set_record_ancestors": (C.c_int, [_P, C.c_int32]),
+    "dpomp_pf_set_history": (C.c_int, [_P, C.c_int32]),
+    "dpomp_pf_get_filtered_moments": (C.c_int, [_P, C.c_int32, C.c_int32, _P, _P, _P]),
+    "dpomp_pf_sample_paths": (C.c_int, [_P, C.c_int32, C.c_int32, C.c_int32, C.c_uint64, _P]),
     "dpomp_pf_overflow_count": (C.c_int, [_P, C.POINTER(C.c_int64)]),
     "dpomp_pf_last_event_count": (C.c_int, [_P, C.POINTER(C.c_int64)]),
     "dpomp_pf_last_timing": (C.c_int, [_P, C.POINTER(C.c_float), C.POINTER(C.c_int32)]),

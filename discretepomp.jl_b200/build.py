@@ -14,7 +14,7 @@ CSRC = os.path.join(HERE, "csrc")
 LIBDIR = os.path.join(HERE, "lib")
 OBJDIR = os.path.join(LIBDIR, "obj")
 SOURCES = ["capi.cu", "pf_kernels.cu", "pf_sim_f32.cu", "pf_sim_f64.cu", "pf_sim_count_f32.cu", "pf_sim_count_f64.cu", "mbp.cu",
-           "comm.cu", "da.cu"]
+           "comm.cu", "da.cu", "pf_history.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
     "-Xcompiler", "-fPIC", "-Xptxas", "-v", "--expt-relaxed-constexpr", "-ftz=true",

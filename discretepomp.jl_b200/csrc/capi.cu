@@ -162,6 +162,7 @@ static void pf_free(dpomp_pf* pf) {
     cudaFree(pf->obs_time_dev); cudaFree(pf->obs_ysum_dev); cudaFree(pf->slots_dev); cudaFree(pf->filter_ids_dev); cudaFree(pf->work_counter); cudaFree(pf->filt_gen);
     cudaFree(pf->rows_done); cudaFree(pf->gen_flags); cudaFree(pf->obs_haslik_dev);
     cudaFree(pf->obs_lgy_dev); cudaFree(pf->obs_lgk_dev);
+    cudaFree(pf->hist_states); cudaFree(pf->hist_anc); cudaFree(pf->hist_part); cudaFree(pf->hist_mom); cudaFree(pf->hist_haslik);
     cudaFreeHost(pf->h_theta); cudaFreeHost(pf->h_ll); cudaFreeHost(pf->h_slots); cudaFreeHost(pf->h_cnt);
     for (cudaEvent_t e : pf->kev) cudaEventDestroy(e);
     if (pf->ev0) cudaEventDestroy(pf->ev0);
@@ -401,8 +402,17 @@ int dpomp_run_partial_enqueue(dpomp_pf* pf, const double* theta, bool theta_on_d
     CK(cudaMemsetAsync(pf->grp_ev, 0, (size_t)nb * pf->ngroups * sizeof(unsigned long long), st));
     int launches = 0;
     pf->kev_kind.clear();
+    // the history continues only where the previous call of the handle stopped (or restarts with ymin == 1)
+    const bool hist = pf->hist_flags != 0;
+    if (hist && (ymin == 1 || (pf->hist_upto > 0 && ymin == pf->hist_upto + 1))) {
+        pf->hist_nb = ymin == 1 ? nb : (nb < pf->hist_nb ? nb : pf->hist_nb);
+        pf->hist_upto = ymax;
+    } else {
+        pf->hist_upto = 0;
+    }
+    pf->hist_weights_t = hist ? ymax : 0;
     bool fused_ok = false;
-    if (pf->fused_enabled && pf->rs_type != DPOMP_RS_MULTINOMIAL) {
+    if (pf->fused_enabled && pf->rs_type != DPOMP_RS_MULTINOMIAL && !hist) {
         int& cap = pf->fused_capacity[pf->sim_precision == DPOMP_SIM_F64 ? 1 : 0];
         if (cap < 0) cap = sim_fused_capacity(mh, pf->sim_precision, pf->items);
         // measured on B200: with several tiles per filter the CTAs that wait for the combine hold SM slots and the fused
@@ -413,7 +423,7 @@ int dpomp_run_partial_enqueue(dpomp_pf* pf, const double* theta, bool theta_on_d
     // persistent path: ONE cooperative launch for all observations of the call (pf_sim.cuh, MODE 2) when every CTA of the
     // launch is co-resident; otherwise the per-observation launch chain below
     bool persist_ok = false;
-    if (pf->persist_mode != 0 && pf->rs_type != DPOMP_RS_MULTINOMIAL && pf->sim_precision == DPOMP_SIM_F32 && !pf->kernel_timing &&
+    if (pf->persist_mode != 0 && !hist && pf->rs_type != DPOMP_RS_MULTINOMIAL && pf->sim_precision == DPOMP_SIM_F32 && !pf->kernel_timing &&
         make_chunk_perm(pf->scatter_mode, pf->n, pf->ntiles).ncf == 0 && (pf->persist_mode == 2 || ymax > ymin)) {
         if (pf->persist_capacity < 0) pf->persist_capacity = sim_persist_capacity(mh, pf->sim_precision, pf->items);
         persist_ok = (long long)nb * pf->ntiles <= pf->persist_capacity;
@@ -477,7 +487,7 @@ int dpomp_run_partial_enqueue(dpomp_pf* pf, const double* theta, bool theta_on_d
         a.pop = pf->pop[pf->cur];
         a.logw = pf->logw;
         a.wtile = pf->wtile;
-        a.record_logw = pf->record_anc ? 1 : 0;
+        a.record_logw = (pf->record_anc || hist) ? 1 : 0;
         a.theta = pf->theta_dev;
         a.obs_time = pf->obs_time_dev;
         a.obs_ysum = pf->obs_ysum_dev;
@@ -531,6 +541,19 @@ int dpomp_run_partial_enqueue(dpomp_pf* pf, const double* theta, bool theta_on_d
         CK(launch_sim_weight(mh, pf->sim_precision, pf->items, fused ? 1 : 0, a, st));
         if (pf->kernel_timing) CK(kernel_event(pf, -1, st));
         ++launches;
+        int32_t* anc_t = pf->record_anc ? pf->anc : nullptr;  // where the resampling after observation t writes its ancestors
+        if (hist) {  // record observation t: states before resampling, tile partials of the moments
+            HistoryLaunch h{};
+            h.pop = pf->pop[pf->cur]; h.logw = pf->logw;
+            const size_t B = (size_t)pf->n_batch;
+            h.states = (pf->hist_flags & DPOMP_HISTORY_PATHS) ? pf->hist_states + (size_t)t * B * pf->n_comp * pf->n_pad : nullptr;
+            h.part = (pf->hist_flags & DPOMP_HISTORY_MOMENTS)
+                         ? pf->hist_part + (size_t)t * B * pf->ntiles * history_partials_stride(pf->n_comp) : nullptr;
+            h.n = pf->n; h.n_pad = pf->n_pad; h.ntiles = pf->ntiles; h.n_filters = nb; h.n_comp = pf->n_comp; h.has_lik = has_lik;
+            CK(launch_history(pf->items, h, st));
+            ++launches;
+            if (pf->hist_flags & DPOMP_HISTORY_PATHS) anc_t = pf->hist_anc + (size_t)t * B * pf->n_pad;
+        }
         if (fused) {
             // the host mirrors of the device ticket counter / generation advance only once the launch is enqueued: a failed
             // launch leaves the handle consistent (the device counter has not moved either)
@@ -545,7 +568,7 @@ int dpomp_run_partial_enqueue(dpomp_pf* pf, const double* theta, bool theta_on_d
             r.defer_l2 = defer_l2 ? 1 : 0; r.has_lik = has_lik;
             r.grp_m = pf->grp_m; r.grp_s = pf->grp_s; r.grp_f_w = pf->grp_f; r.grp_off_w = pf->grp_off;
             r.filt_s_w = pf->filt_s; r.filt_m_w = pf->filt_m; r.ll_acc = pf->ll_acc;
-            r.anc = pf->record_anc ? pf->anc : nullptr;
+            r.anc = anc_t;
             r.cw = pf->cw;
             r.n = pf->n; r.n_pad = pf->n_pad; r.ntiles = pf->ntiles; r.n_filters = nb; r.n_comp = pf->n_comp;
             r.t = t; r.rs_type = pf->rs_type; r.key = key; r.filter0 = (uint32_t)pf->batch_offset;
@@ -556,6 +579,7 @@ int dpomp_run_partial_enqueue(dpomp_pf* pf, const double* theta, bool theta_on_d
             if (pf->kernel_timing) CK(kernel_event(pf, -1, st));
             launches += (pf->rs_type == DPOMP_RS_MULTINOMIAL) ? 2 : 1;
             pf->cur ^= 1;
+            pf->anc_last = anc_t != pf->anc ? anc_t : nullptr;
         }
         pf->last_resampled = do_rs != 0;
     }
@@ -633,6 +657,8 @@ int dpomp_pf_permute(dpomp_pf* pf, const int64_t* nidx, int32_t n) {
                            (size_t)(pf->n_batch - n) * stride * sizeof(int32_t), cudaMemcpyDeviceToDevice, pf->stream));
     CK(cudaStreamSynchronize(pf->stream));
     pf->cur ^= 1;
+    pf->hist_upto = 0;
+    pf->hist_weights_t = 0;
     return DPOMP_OK;
 }
 
@@ -649,6 +675,8 @@ int dpomp_pf_copy_filters(dpomp_pf* dst, const dpomp_pf* src, const int64_t* dst
     CK(launch_gather_filters(dst->pop[dst->cur], src->pop[src->cur], dst->slots_dev, dst->slots_dev + dst->n_batch, n, stride, dst->stream));
     CK(cudaStreamSynchronize(dst->stream));
     dst->initialised = true;
+    dst->hist_upto = 0;
+    dst->hist_weights_t = 0;
     return DPOMP_OK;
 }
 
@@ -676,6 +704,8 @@ int dpomp_pf_set_pop(dpomp_pf* pf, int32_t b, const int64_t* in) {
     CK(cudaMemcpyAsync(pf->pop[pf->cur] + (size_t)(b - 1) * words, tmp.data(), words * sizeof(int32_t), cudaMemcpyHostToDevice, pf->stream));
     CK(cudaStreamSynchronize(pf->stream));
     pf->initialised = true;
+    pf->hist_upto = 0;
+    pf->hist_weights_t = 0;
     return DPOMP_OK;
 }
 
@@ -695,9 +725,108 @@ int dpomp_pf_get_last_ancestors(dpomp_pf* pf, int32_t b, int64_t* out) {
     if (!pf->record_anc || !pf->anc) return fail(DPOMP_ERR_STATE, "ancestor recording is off");
     CK(cudaSetDevice(pf->device));
     std::vector<int32_t> tmp((size_t)pf->n);
-    CK(cudaMemcpyAsync(tmp.data(), pf->anc + (size_t)(b - 1) * pf->n_pad, (size_t)pf->n * sizeof(int32_t), cudaMemcpyDeviceToHost, pf->stream));
+    const int32_t* src = pf->anc_last ? pf->anc_last : pf->anc;  // with the history on: its slice of the last resampling
+    CK(cudaMemcpyAsync(tmp.data(), src + (size_t)(b - 1) * pf->n_pad, (size_t)pf->n * sizeof(int32_t), cudaMemcpyDeviceToHost, pf->stream));
     CK(cudaStreamSynchronize(pf->stream));
     for (long long p = 0; p < pf->n; ++p) out[p] = (int64_t)tmp[(size_t)p] + 1;
+    return DPOMP_OK;
+}
+
+int dpomp_pf_set_history(dpomp_pf* pf, int32_t flags) {
+    if (!pf) return fail(DPOMP_ERR_ARG, "null handle");
+    if (flags < 0 || flags > (DPOMP_HISTORY_MOMENTS | DPOMP_HISTORY_PATHS)) return fail(DPOMP_ERR_ARG, "unknown history flags");
+    if (flags == pf->hist_flags) return DPOMP_OK;
+    CK(cudaSetDevice(pf->device));
+    CK(cudaStreamSynchronize(pf->stream));
+    cudaFree(pf->hist_states); cudaFree(pf->hist_anc); cudaFree(pf->hist_part); cudaFree(pf->hist_mom); cudaFree(pf->hist_haslik);
+    pf->hist_states = pf->hist_anc = nullptr;
+    pf->hist_part = pf->hist_mom = nullptr;
+    pf->hist_haslik = nullptr;
+    pf->hist_flags = 0;
+    pf->hist_upto = pf->hist_nb = pf->hist_weights_t = 0;
+    pf->anc_last = nullptr;
+    if (flags == 0) return DPOMP_OK;
+    const size_t T = (size_t)pf->n_obs, B = (size_t)pf->n_batch, NP = (size_t)pf->n_pad, C = (size_t)pf->n_comp;
+    cudaError_t e = cudaMalloc((void**)&pf->hist_haslik, T * sizeof(int));
+    if (e == cudaSuccess && (flags & DPOMP_HISTORY_PATHS)) {
+        e = cudaMalloc((void**)&pf->hist_states, T * B * C * NP * sizeof(int32_t));
+        if (e == cudaSuccess) e = cudaMalloc((void**)&pf->hist_anc, T * B * NP * sizeof(int32_t));
+    }
+    if (e == cudaSuccess && (flags & DPOMP_HISTORY_MOMENTS)) {
+        e = cudaMalloc((void**)&pf->hist_part, T * B * pf->ntiles * history_partials_stride(pf->n_comp) * sizeof(double));
+        if (e == cudaSuccess) e = cudaMalloc((void**)&pf->hist_mom, T * B * (2 * C + 1) * sizeof(double));
+    }
+    if (e == cudaSuccess) {
+        std::vector<int> hl(T);
+        for (size_t t = 0; t < T; ++t) hl[t] = pf->model->h.obs_id[t] > 0;
+        e = cudaMemcpy(pf->hist_haslik, hl.data(), T * sizeof(int), cudaMemcpyHostToDevice);
+    }
+    if (e != cudaSuccess) {
+        (void)cudaGetLastError();
+        cudaFree(pf->hist_states); cudaFree(pf->hist_anc); cudaFree(pf->hist_part); cudaFree(pf->hist_mom); cudaFree(pf->hist_haslik);
+        pf->hist_states = pf->hist_anc = nullptr;
+        pf->hist_part = pf->hist_mom = nullptr;
+        pf->hist_haslik = nullptr;
+        return fail(DPOMP_ERR_CUDA, std::string("history buffers: ") + cudaGetErrorString(e));
+    }
+    pf->hist_flags = flags;
+    return DPOMP_OK;
+}
+
+// shared checks of the history getters
+static int history_covers(const dpomp_pf* pf, int flag, int nb, int t_last) {
+    if (nb < 1 || nb > pf->n_batch) return fail(DPOMP_ERR_ARG, "n_batch_used out of range");
+    if (t_last < 1 || t_last > pf->n_obs) return fail(DPOMP_ERR_ARG, "t_last out of range");
+    if (!(pf->hist_flags & flag))
+        return fail(DPOMP_ERR_STATE, flag == DPOMP_HISTORY_PATHS ? "path history is off" : "moment history is off");
+    if (t_last > pf->hist_upto || nb > pf->hist_nb)
+        return fail(DPOMP_ERR_STATE, "the history does not cover observations 1..t_last of these filters");
+    return DPOMP_OK;
+}
+
+int dpomp_pf_get_filtered_moments(dpomp_pf* pf, int32_t nb, int32_t t_last, double* out_mean, double* out_var, double* out_ess) {
+    if (!pf || !out_mean || !out_var || !out_ess) return fail(DPOMP_ERR_ARG, "null argument");
+    int rc = history_covers(pf, DPOMP_HISTORY_MOMENTS, nb, t_last);
+    if (rc) return rc;
+    CK(cudaSetDevice(pf->device));
+    const size_t C = (size_t)pf->n_comp, W = 2 * C + 1, rows = (size_t)nb * t_last;
+    CK(launch_history_moments(pf->hist_part, t_last, pf->n_batch, nb, pf->ntiles, pf->n_comp, pf->hist_mom, pf->stream));
+    std::vector<double> tmp(rows * W);
+    CK(cudaMemcpyAsync(tmp.data(), pf->hist_mom, rows * W * sizeof(double), cudaMemcpyDeviceToHost, pf->stream));
+    CK(cudaStreamSynchronize(pf->stream));
+    for (size_t r = 0; r < rows; ++r) {
+        for (size_t c = 0; c < C; ++c) {
+            out_mean[r * C + c] = tmp[r * W + c];
+            out_var[r * C + c] = tmp[r * W + C + c];
+        }
+        out_ess[r] = tmp[r * W + 2 * C];
+    }
+    return DPOMP_OK;
+}
+
+int dpomp_pf_sample_paths(dpomp_pf* pf, int32_t nb, int32_t n_paths, int32_t t_last, uint64_t key, int64_t* out) {
+    if (!pf || !out) return fail(DPOMP_ERR_ARG, "null argument");
+    if (n_paths < 1) return fail(DPOMP_ERR_ARG, "n_paths must be >= 1");
+    int rc = history_covers(pf, DPOMP_HISTORY_PATHS, nb, t_last);
+    if (rc) return rc;
+    if (t_last != pf->hist_weights_t)
+        return fail(DPOMP_ERR_STATE, "the weights of t_last are no longer on the device (t_last must end the last call)");
+    CK(cudaSetDevice(pf->device));
+    const size_t words = (size_t)nb * n_paths * t_last * pf->n_comp;
+    int64_t* d_out = nullptr;
+    CK(cudaMalloc((void**)&d_out, words * sizeof(int64_t)));
+    PathLaunch a{};
+    a.states = pf->hist_states; a.anc = pf->hist_anc; a.haslik = pf->hist_haslik;
+    a.wtile = pf->wtile; a.tile_f = pf->tile_f; a.tile_off = pf->tile_off; a.grp_f = pf->grp_f; a.grp_off = pf->grp_off;
+    a.filt_s = pf->filt_s; a.out = d_out;
+    a.n = pf->n; a.n_pad = pf->n_pad; a.ntiles = pf->ntiles; a.ngroups = pf->ngroups; a.tile = pf->tile; a.n_batch = pf->n_batch;
+    a.nb = nb; a.n_paths = n_paths; a.n_comp = pf->n_comp; a.t_last = t_last; a.n_obs = pf->n_obs;
+    a.key = key; a.filter0 = (uint32_t)pf->batch_offset; a.filter_ids = pf->use_filter_ids ? pf->filter_ids_dev : nullptr;
+    cudaError_t e = launch_paths(a, pf->stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(out, d_out, words * sizeof(int64_t), cudaMemcpyDeviceToHost, pf->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(pf->stream);
+    cudaFree(d_out);
+    if (e != cudaSuccess) return fail(DPOMP_ERR_CUDA, std::string("sample_paths: ") + cudaGetErrorString(e));
     return DPOMP_OK;
 }
 
@@ -753,6 +882,8 @@ int dpomp_pf_import_filters(dpomp_pf* pf, const int64_t* slots, int32_t n, const
     CK(launch_pack_filters((int32_t*)device_src, pf->pop[pf->cur], pf->slots_dev, n, (long long)pf->n_comp * pf->n_pad, 1, pf->stream));
     CK(cudaStreamSynchronize(pf->stream));
     pf->initialised = true;
+    pf->hist_upto = 0;
+    pf->hist_weights_t = 0;
     return DPOMP_OK;
 }
 

@@ -469,6 +469,8 @@ int dpomp_pf_resample_migrate(dpomp_pf* pf, dpomp_comm* c, const int64_t* nidx, 
     if (n_recv) CCK(launch_pack_filters((int32_t*)c->d_pack_recv, pf->pop[pf->cur], c->d_slots + n_send + n_loc, (int)n_recv, stride, 1, st));
     CCK(cudaStreamSynchronize(st));
     pf->initialised = true;
+    pf->hist_upto = 0;  // the filters have new lineages: their history is gone (include/dpomp.h)
+    pf->hist_weights_t = 0;
     return DPOMP_OK;
 }
 

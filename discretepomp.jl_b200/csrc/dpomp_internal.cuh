@@ -212,6 +212,17 @@ struct dpomp_pf {
     std::vector<int> kev_kind;         // 0 = simulate+weight, 1 = resample
     float kernel_ms[2] = {0.f, 0.f};
     int kernel_launches[2] = {0, 0};
+    // hidden-state history (dpomp_pf_set_history, pf_history.cu)
+    int hist_flags = 0;
+    int32_t* hist_states = nullptr;    // PATHS:   [T][n_batch][C][n_pad] simulated states before resampling
+    int32_t* hist_anc = nullptr;       // PATHS:   [T][n_batch][n_pad] 0-based ancestors of the resampling after observation t
+    double* hist_part = nullptr;       // MOMENTS: [T][n_batch][ntiles][history_partials_stride(C)] tile partials
+    double* hist_mom = nullptr;        // MOMENTS: [n_batch][T][2 C + 1] output of the moments combine
+    int* hist_haslik = nullptr;        // [T] obs_id[t] > 0
+    int hist_upto = 0;                 // observations 1..hist_upto are recorded for the first hist_nb filters
+    int hist_nb = 0;
+    int hist_weights_t = 0;            // observation whose weights are still on the device (last of the last call), 0 = none
+    const int32_t* anc_last = nullptr; // where the last resampling wrote its ancestors when that was not `anc` (history on)
 };
 
 
@@ -263,6 +274,38 @@ cudaError_t launch_pack_filters(int32_t* dst_packed, const int32_t* pop, const i
 cudaError_t launch_search_hook(int rs_type, const double* cw_dev, long long n, const double* u_dev, long long n_out,
                                int64_t* out_dev, cudaStream_t stream);
 int sim_kernel_supported(int n_comp, int n_events);
+
+// ---- hidden-state history (pf_history.cu) -----------------------------------------------------------------------------
+// tile partials of one (observation, filter, tile): m, sum w, sum w^2, then per compartment sum w d_c, sum w d_c^2 and the
+// shift x0_c, with w = exp(logw - m) and d_c = x_c - x0_c (x0 = particle 0 of the filter: no cancellation in the variance)
+__host__ __device__ inline int history_partials_stride(int n_comp) { return 3 + 3 * n_comp; }
+struct HistoryLaunch {
+    const int32_t* pop;      // [B][C][n_pad] simulated states of observation t
+    const double* logw;      // [B][n_pad] their log weights (-inf: padding or event cap)
+    int32_t* states;         // [B][C][n_pad] slice t of the state history, or nullptr
+    double* part;            // [B][ntiles][stride] slice t of the tile partials, or nullptr
+    long long n, n_pad;
+    int ntiles, n_filters, n_comp, has_lik;
+};
+cudaError_t launch_history(int items, const HistoryLaunch& a, cudaStream_t stream);
+// mean, variance and ESS of observations 1..t_last of the first nb filters: out [nb][t_last][2 C + 1]
+cudaError_t launch_history_moments(const double* part, int t_last, int n_batch, int nb, int ntiles, int n_comp, double* out,
+                                   cudaStream_t stream);
+struct PathLaunch {
+    const int32_t* states;   // [T][B][C][n_pad]
+    const int32_t* anc;      // [T][B][n_pad]
+    const int* haslik;       // [T]
+    // the filter's scan tree at observation t_last (as the resample kernel reads it)
+    const double* wtile; const double* tile_f; const double* tile_off; const double* grp_f; const double* grp_off;
+    const double* filt_s;
+    int64_t* out;            // [nb][n_paths][t_last][C]
+    long long n, n_pad;
+    int ntiles, ngroups, tile, n_batch, nb, n_paths, n_comp, t_last, n_obs;
+    uint64_t key;
+    uint32_t filter0;
+    const uint32_t* filter_ids;
+};
+cudaError_t launch_paths(const PathLaunch& a, cudaStream_t stream);
 // count observation law of a model with its device arrays (obs_lgy / obs_lgk uploaded by the caller)
 CountObs count_obs_of(const ModelHost& m, const double* lgy_dev, const double* lgk_dev);
 

@@ -499,6 +499,30 @@ function partial_log_likelihood_batch!(pf::DpompPF, theta::Array{Float64, 2}, ym
     return gx
 end
 
+## hidden states of the filter (dpomp_pf_set_history): filtering mean / variance (C x T x B), ESS (T x B) at every observation
+## and n_paths state paths per filter (C x T x n_paths x B, Int64) traced back through the particle genealogy from the last
+## observation; a theta vector gives B = 1
+function get_filtered_states(model::DPOMPModel, obs_data::Array{Observation, 1}, parameters::Array{Float64};
+                             np::Int64 = C_DF_PF_P, n_paths::Int64 = 0, rs_type::Int64 = 1, seed = rand(UInt64))
+    theta = reshape(parameters, size(parameters, 1), :)
+    B, T = size(theta, 2), length(obs_data)
+    mdl = dpomp_model(get_private_model(model, obs_data))
+    C = length(model.initial_condition)
+    pf = DpompPF(mdl, np, B, rs_type; seed = seed)
+    flags = Int32(1) | (n_paths > 0 ? Int32(2) : Int32(0))   # DPOMP_HISTORY_MOMENTS | DPOMP_HISTORY_PATHS
+    dpomp_check(ccall((:dpomp_pf_set_history, LIBDPOMP), Cint, (Ptr{Cvoid}, Int32), pf.handle, flags))
+    key = rand(UInt64)   # call key of the filter run; the path draws reuse it (their stream block is otherwise unused)
+    dpomp_check(ccall((:dpomp_pf_set_stream_key, LIBDPOMP), Cint, (Ptr{Cvoid}, UInt64), pf.handle, key))
+    loglik = partial_log_likelihood_batch!(pf, theta, 1, T)
+    mean = Array{Float64, 3}(undef, C, T, B); var = similar(mean); ess = Array{Float64, 2}(undef, T, B)
+    GC.@preserve mean var ess dpomp_check(ccall((:dpomp_pf_get_filtered_moments, LIBDPOMP), Cint,
+        (Ptr{Cvoid}, Int32, Int32, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}), pf.handle, B, T, mean, var, ess))
+    paths = Array{Int64, 4}(undef, C, T, n_paths, B)
+    n_paths > 0 && GC.@preserve paths dpomp_check(ccall((:dpomp_pf_sample_paths, LIBDPOMP), Cint,
+        (Ptr{Cvoid}, Int32, Int32, Int32, UInt64, Ptr{Int64}), pf.handle, B, n_paths, T, key, paths))
+    return (time = [o.time for o in obs_data], loglik = loglik, mean = mean, var = var, ess = ess, paths = paths)
+end
+
 ## `pop2[p] .= pop[nidx[p]]` (src/hmm_ibis.jl:74) and `pop[p] .= pop_f` (:108)
 permute_filters!(pf::DpompPF, nidx::Array{Int64, 1}) =
     GC.@preserve nidx dpomp_check(ccall((:dpomp_pf_permute, LIBDPOMP), Cint, (Ptr{Cvoid}, Ptr{Int64}, Int32), pf.handle, nidx, length(nidx)))

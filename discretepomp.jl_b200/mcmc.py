@@ -52,9 +52,14 @@ def gelman_diagnostic_sre(samples: np.ndarray, discard: int) -> np.ndarray:
 
 def run_pmcmc(model: HiddenMarkovModel, theta_init: np.ndarray, steps: int = 50000, adapt_period: int = 10000,
               p: int = 200, seed: int = 1, comm: Optional[Comm] = None, pf_factory: Optional[Callable] = None,
-              verbose: bool = True) -> MCMCSample:
+              verbose: bool = True, state_interval: int = 0) -> MCMCSample:
     """run_pmcmc(model, theta_init, steps = 50000, adapt_period = 10000, p = 200) (src/hmm_mcmc.jl:349-365);
-    theta_init is (n_theta, n_chains).  Returns MCMCSample with samples.theta of shape (n_theta, steps, n_chains)."""
+    theta_init is (n_theta, n_chains).  Returns MCMCSample with samples.theta of shape (n_theta, steps, n_chains).
+
+    state_interval = k > 0 also samples the hidden states (particle marginal Metropolis-Hastings, Andrieu, Doucet &
+    Holenstein 2010): every filter call draws one state path per chain from its particle genealogy, an accepted chain takes
+    its proposal's path, and after the adaptation period the current path of every k-th step is kept in
+    MCMCSample.states, shape (n_chains, n_kept, T, C)."""
     comm = comm or Comm(None)
     start_time = time.time_ns()
     theta_init = np.asarray(theta_init, dtype=np.float64)
@@ -65,6 +70,11 @@ def run_pmcmc(model: HiddenMarkovModel, theta_init: np.ndarray, steps: int = 500
         print(f"Running PMCMC analysis: {n_chains} x {steps} samples")
     make = pf_factory or (lambda nb, sd: ParticleFilter(device_model(model), p, nb, 1, seed=sd))
     pf = make(max(n_loc, 1), seed)
+    if state_interval > 0:
+        pf.set_history(moments=False, paths=True)
+        n_obs, n_comp = pf.n_obs, pf.n_comp
+        paths = np.zeros((n_loc, n_obs, n_comp), dtype=np.int64)  # path of the last evaluation of every chain slot
+        kept = []
     adapt_interval = adapt_period / 10  # ADAPT_INTERVAL = adapt_period / 10 is a Float64 in the reference (:168)
     chains = np.zeros((n_loc, steps, d))
     chol = np.zeros((n_loc, d, d))
@@ -87,16 +97,21 @@ def run_pmcmc(model: HiddenMarkovModel, theta_init: np.ndarray, steps: int = 500
             if last_ids[0] is None or not np.array_equal(last_ids[0], valid):  # filter slot j simulates chain lo + valid[j]
                 pf.set_filter_ids(lo + valid)
                 last_ids[0] = valid
-            pf.set_stream_key(splitmix64((seed & _M64) ^ splitmix64(step + 1)))
+            key = splitmix64((seed & _M64) ^ splitmix64(step + 1))
+            pf.set_stream_key(key)
             t0 = time.perf_counter()
             out[valid] = lp[valid] + pf.loglik(np.ascontiguousarray(thetas[valid].T))
             timers["filter_calls_wall"] += time.perf_counter() - t0
             if hasattr(pf, "last_timing"):
                 timers["filter_device_ms"] += pf.last_timing()[0]
+            if state_interval > 0:  # the lineage ends use a stream block the filter itself never draws from
+                paths[valid] = pf.sample_paths(1, key, nb=len(valid))[:, 0]
         return out
 
     chains[:, 0, :] = t0s
     ll_i = target(chains[:, 0, :], 0)
+    if state_interval > 0:
+        cur_paths = paths.copy()
     # running sums of every chain's samples, SHIFTED by the chain's starting point (no cancellation for tightly
     # concentrated chains): the covariance of the adaptation step without a pass over the history
     shift = chains[:, 0, :].copy()
@@ -115,6 +130,10 @@ def run_pmcmc(model: HiddenMarkovModel, theta_init: np.ndarray, steps: int = 500
         ok = (ll_f != -np.inf) & ((mh > 1) | (mh > u))  # :189-190
         ll_i = np.where(ok, ll_f, ll_i)
         chains[:, i, :] = np.where(ok[:, None], prop, chains[:, i - 1, :])
+        if state_interval > 0:
+            cur_paths[ok] = paths[ok]
+            if i >= adapt_period and (i - adapt_period) % state_interval == 0:
+                kept.append(cur_paths.copy())
         accepted_total += ok
         dx = chains[:, i, :] - shift
         sum_x += dx
@@ -140,17 +159,22 @@ def run_pmcmc(model: HiddenMarkovModel, theta_init: np.ndarray, steps: int = 500
     out.accepted = comm.allgather_f64(accepted_total.astype(np.float64), n_chains).astype(np.int64)
     timers["total_wall"] = (time.time_ns() - start_time) * 1e-9
     out.timers = timers
+    if state_interval > 0:
+        n_kept = len(kept)
+        loc = np.stack(kept, axis=1) if n_kept else np.zeros((n_loc, 0, n_obs, n_comp), dtype=np.int64)
+        flat = comm.allgather_f64(loc.reshape(n_loc, -1).astype(np.float64), n_chains)  # counts < 2^31: exact in f64
+        out.states = flat.reshape(n_chains, n_kept, n_obs, n_comp).astype(np.int64)
     return out
 
 
 def run_pmcmc_analysis(model: DPOMPModel, obs_data, n_chains: int = 3, initial_parameters: Optional[np.ndarray] = None,
                        steps: int = C_DF_MCMC_STEPS, adapt_period: Optional[int] = None, np_: int = 200, seed: int = 1,
-                       comm: Optional[Comm] = None, **kw) -> MCMCSample:
+                       comm: Optional[Comm] = None, state_interval: int = 0, **kw) -> MCMCSample:
     """Public-model wrapper in the style of run_mcmc_analysis (src/DiscretePOMP.jl:185-193): chains start from draws of
-    the prior unless `initial_parameters` (n_theta, n_chains) is given."""
+    the prior unless `initial_parameters` (n_theta, n_chains) is given.  state_interval: see run_pmcmc."""
     mdl = get_private_model(model, obs_data)
     if adapt_period is None:
         adapt_period = int(np.floor(steps * C_DF_MCMC_ADAPT))
     if initial_parameters is None:
         initial_parameters = mdl.prior.rand(n_chains, np.random.default_rng(seed))
-    return run_pmcmc(mdl, initial_parameters, steps, adapt_period, np_, seed=seed, comm=comm, **kw)
+    return run_pmcmc(mdl, initial_parameters, steps, adapt_period, np_, seed=seed, comm=comm, state_interval=state_interval, **kw)

@@ -9,6 +9,7 @@ Here the closure holds a device handle (`ParticleFilter`) and every f(theta) is 
 from __future__ import annotations
 
 import ctypes as C
+from dataclasses import dataclass
 from typing import Callable, List, Optional, Sequence
 
 import numpy as np
@@ -224,6 +225,33 @@ class ParticleFilter:
         _capi.check(_capi.lib().dpomp_pf_get_last_ancestors(self._h, int(b), _capi.ptr(out)))
         return out
 
+    # -- hidden-state history (dpomp_pf_set_history) -------------------------------------------------------------
+    def set_history(self, moments: bool = True, paths: bool = False) -> None:
+        """Record the filtering distributions of every observation: `moments` for filtered_moments(), `paths` (the states
+        and ancestors, T * n_batch * n_pad * (4 C + 4) bytes of device memory) for sample_paths()."""
+        flags = (_capi.HISTORY_MOMENTS if moments else 0) | (_capi.HISTORY_PATHS if paths else 0)
+        _capi.check(_capi.lib().dpomp_pf_set_history(self._h, flags))
+
+    def filtered_moments(self, nb: Optional[int] = None, t_last: Optional[int] = None):
+        """(mean[nb, t_last, C], var[nb, t_last, C], ess[nb, t_last]) of the weighted particles before resampling at
+        observations 1..t_last of the first nb filters."""
+        nb = self.n_batch if nb is None else int(nb)
+        t_last = self.n_obs if t_last is None else int(t_last)
+        mean = np.empty((nb, t_last, self.n_comp)); var = np.empty_like(mean); ess = np.empty((nb, t_last))
+        _capi.check(_capi.lib().dpomp_pf_get_filtered_moments(self._h, nb, t_last, _capi.ptr(mean), _capi.ptr(var),
+                                                              _capi.ptr(ess)))
+        return mean, var, ess
+
+    def sample_paths(self, n_paths: int, key: int, nb: Optional[int] = None, t_last: Optional[int] = None) -> np.ndarray:
+        """n_paths state paths x_1..x_t_last per filter, traced back through the particle genealogy from lineage ends
+        drawn from the weights of t_last (the last observation of the last call): int64 [nb, n_paths, t_last, C]."""
+        nb = self.n_batch if nb is None else int(nb)
+        t_last = self.n_obs if t_last is None else int(t_last)
+        out = np.empty((nb, int(n_paths), t_last, self.n_comp), dtype=np.int64)
+        _capi.check(_capi.lib().dpomp_pf_sample_paths(self._h, nb, int(n_paths), t_last, C.c_uint64(key & 0xFFFFFFFFFFFFFFFF),
+                                                      _capi.ptr(out)))
+        return out
+
     def overflow_count(self) -> int:
         v = C.c_int64()
         _capi.check(_capi.lib().dpomp_pf_overflow_count(self._h, C.byref(v)))
@@ -309,3 +337,40 @@ def get_particle_filter_lpdf(model: DPOMPModel, obs_data: List[Observation], np:
     """get_particle_filter_lpdf(model, obs_data; np, rs_type, essc) (src/hmm_utils.jl:281-284)"""
     mdl = get_private_model(model, obs_data)
     return get_log_pdf_fn(mdl, np, rs_type, essc=essc, **kw)
+
+
+@dataclass
+class FilteredStates:
+    """Hidden states of get_filtered_states: observation times time[T], the log-likelihood estimates loglik[B], the
+    filtering mean / variance mean[B, T, C], var[B, T, C] and effective sample size ess[B, T] at every observation, and
+    paths[B, n_paths, T, C] drawn from the particle genealogy (empty when n_paths = 0).  A 1-D theta drops the B axis."""
+    time: np.ndarray
+    loglik: np.ndarray
+    mean: np.ndarray
+    var: np.ndarray
+    ess: np.ndarray
+    paths: np.ndarray
+
+
+def get_filtered_states(model: DPOMPModel, obs_data: List[Observation], parameters, np: int = C_DF_PF_P, n_paths: int = 0,
+                        rs_type: int = 1, seed: int = 1, **kw) -> FilteredStates:
+    """One bootstrap particle filter per theta (a parameter vector, or an (n_theta, B) matrix) over all observations,
+    recording the filtering moments at every observation and, with n_paths > 0, n_paths state paths per filter traced
+    back through the particle genealogy from the last observation (Kitagawa's filter-smoother)."""
+    import numpy
+
+    th = numpy.asarray(parameters, dtype=numpy.float64)
+    cols = th.reshape(-1, 1) if th.ndim == 1 else th
+    pf = ParticleFilter(device_model(get_private_model(model, obs_data)), np, cols.shape[1], rs_type, seed, **kw)
+    pf.set_history(moments=True, paths=n_paths > 0)
+    key = pf.next_stream_key()
+    ll = pf.loglik(cols)
+    mean, var, ess = pf.filtered_moments()
+    # the lineage ends use block 2 of the resampling tag, which the filter's own draws never use: the call key can be reused
+    paths = (pf.sample_paths(n_paths, key) if n_paths > 0
+             else numpy.zeros((cols.shape[1], 0, pf.n_obs, pf.n_comp), dtype=numpy.int64))
+    time = numpy.array([o.time for o in obs_data], dtype=numpy.float64)
+    if th.ndim == 1:
+        return FilteredStates(time, float(ll[0]), mean[0], var[0], ess[0], paths[0])
+    return FilteredStates(time, ll, mean, var, ess, paths)
+

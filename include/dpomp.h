@@ -224,6 +224,46 @@ int dpomp_pf_set_pop(dpomp_pf* pf, int32_t b /*1-based*/, const int64_t* in);
 int dpomp_pf_get_last_logw(dpomp_pf* pf, int32_t b, double* out_logw);
 int dpomp_pf_get_last_ancestors(dpomp_pf* pf, int32_t b, int64_t* out_anc);
 int dpomp_pf_set_record_ancestors(dpomp_pf* pf, int32_t on);  /* switches the diagnostics (log weights AND ancestors) on/off */
+/*
+ * Hidden-state history of the filters (the filtering distributions that partial_log_likelihood!,
+ * src/hmm_particle_filter.jl:39-76, forms at every observation and then discards).
+ *
+ * dpomp_pf_set_history: flags = 0 (default, off) or an OR of
+ *   DPOMP_HISTORY_MOMENTS  per-observation partial sums of the weighted states, for dpomp_pf_get_filtered_moments
+ *   DPOMP_HISTORY_PATHS    per-observation states and resampling ancestors, for dpomp_pf_sample_paths
+ * The buffers are allocated here, for n_batch filters and all T observations: PATHS needs T * n_batch * n_pad * (4 C + 4)
+ * bytes (n_pad = n_particles rounded up to the tile), MOMENTS T * n_batch * (tiles * (3 + 3 C) + 2 C + 1) * 8 bytes.  On an allocation
+ * failure the call returns DPOMP_ERR_CUDA and the history is off.  Changing the flags discards the recorded history;
+ * setting the current flags again does nothing.  With the history on, partial / loglik run the per-observation launch chain (never the fused or
+ * persistent launch), record the log weights (as dpomp_pf_set_record_ancestors does) and run one more kernel per observation;
+ * log-likelihoods, populations, event counts and the last-call diagnostics are bit-identical to the history off.
+ *
+ * The history belongs to the current lineages of the filters.  It covers observations 1..t when every call since the last
+ * call with ymin == 1 ran with the history on, each call continuing at the observation after the previous one.
+ * dpomp_pf_permute, dpomp_pf_copy_filters (its destination), dpomp_pf_set_pop, dpomp_pf_import_filters and
+ * dpomp_pf_resample_migrate discard it.  Both getters return DPOMP_ERR_STATE when the history is off or does not cover
+ * 1..t_last for the first n_batch_used filters, and DPOMP_ERR_ARG for other arguments out of range.
+ */
+#define DPOMP_HISTORY_MOMENTS 1
+#define DPOMP_HISTORY_PATHS 2
+int dpomp_pf_set_history(dpomp_pf* pf, int32_t flags);
+/* Filtering moments at observations 1..t_last: the particles are the simulated states before resampling, weighted by
+ * exp(log g) normalised (particles at the event cap weigh 0, as in the filter); an observation with obs_id <= 0 has no
+ * likelihood and weighs the n particles equally.  out_mean / out_var [b][t][c] (weighted mean and biased second central
+ * moment), out_ess [b][t] = (sum w)^2 / sum w^2 as compute_ess (src/hmm_particle_filter.jl:4-6).  Needs MOMENTS. */
+int dpomp_pf_get_filtered_moments(dpomp_pf* pf, int32_t n_batch_used, int32_t t_last, double* out_mean, double* out_var,
+                                  double* out_ess);
+/* State paths x_1..x_{t_last} by the genealogy of the particles (Kitagawa's filter-smoother; in particle marginal
+ * Metropolis-Hastings one such path per step gives samples of (theta, x_1..x_T), Andrieu, Doucet & Holenstein 2010).
+ * For each filter, n_paths lineage ends are drawn independently from the weights of observation t_last with the rule of
+ * rs_multinomial (src/hmm_resample.jl:9-16): the first particle q with u S < cw_q, cw the filter's own cumulative weights;
+ * u = u53 of Philox(key; path, global filter id, t_last - 1, resample tag, block 2).  When observation t_last has obs_id <= 0
+ * the end is floor(u n).  Then k_{t-1} = ancestor_{t-1}[k_t] where observation t-1 resampled (k unchanged where it did not)
+ * and x_t = state_t[k_t].  out [b][path][t][c] int64, t = 1..t_last (the Julia array C x t_last x n_paths x n_batch_used).
+ * The weights of t_last must still be on the device: t_last is the last observation of the last call, and no other filter
+ * call may come between (DPOMP_ERR_STATE otherwise).  Needs PATHS. */
+int dpomp_pf_sample_paths(dpomp_pf* pf, int32_t n_batch_used, int32_t n_paths, int32_t t_last, uint64_t key, int64_t* out);
+
 /* number of (filter, particle, interval) simulations that hit the event cap since creation (sticky) */
 int dpomp_pf_overflow_count(dpomp_pf* pf, int64_t* out_count);
 /* total Gillespie events simulated by the last call (all filters) -- for events/s reporting */
